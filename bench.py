@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the three-mlagents hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): env-steps/sec for ball3d at 65 536 envs per GPU, random policy.
 A "step" of this bench is ONE pass of the hot path over the whole batch: one fused 128-step
@@ -17,6 +17,11 @@ rollout of all 65 536 environments (`tmla_rollout_random`, 8 388 608 env-steps, 
              replicas-identical check; `cpu_baseline.ppo` is the CPU restatement of SB3 PPO at the reference defaults
 Multi-GPU: one process per GPU under torchrun; environments shard by global env id, no data-path
 collective for the env-step metric (weak scaling); PPO adds one gradient all-reduce per minibatch.
+
+--dump-outputs DIR writes what the last timed rollout launch returned on rank 0, for a fixed sample of DUMP_ENVS
+environments (seeded choice, sorted env ids) over all T_ROLLOUT steps, as float32 arrays: obs.npy [T, DUMP_ENVS, 6],
+actions.npy, rewards.npy and dones.npy [T, DUMP_ENVS] (37.7 MB in all).  Every launch before the last timed one has a
+fixed count for given --steps / --warmup, so two builds run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -39,6 +44,10 @@ OBS_DIM = 6
 # SURVEY.md §8(d): fused-rollout path writes obs 24 + reward 4 + done 1 + action 4 per env-step,
 # plus the 56 B/env state read+write amortised over the T steps of one launch.
 BYTES_PER_ENV_STEP = 33.0 + 56.0 / T_ROLLOUT
+DUMP_ENVS, DUMP_SEED = 8192, 0
+# untimed launches that load the GPU before the timed ones while nvidia-smi samples clocks: 130 x 50 launches, ~0.4 s on a
+# B200.  A count rather than a time budget, so that the timed launches start from the same environment state in every run.
+PRELOAD_BATCHES = 130
 
 
 NCU_TRAFFIC_CSV = "profiles/r2_rollout_fast_ncu_raw.csv"
@@ -269,9 +278,9 @@ def run_cuda(args):
     # The timed region is only K x ~70 us long; nvidia-smi needs ~100 ms per sample.  The sampler therefore
     # brackets the timed region with the same kernel running back to back (load before, during and after):
     # untimed launches first, then the K timed launches, then untimed launches until >= 5 samples exist.
+    dumped = None
     with ClockSampler(local_rank) as clocks:
-        t_load = time.perf_counter()
-        while time.perf_counter() - t_load < 0.4:
+        for _ in range(PRELOAD_BATCHES):
             for _ in range(50):
                 env.rollout_random(T_ROLLOUT, obs, act, rew, done)
             torch.cuda.synchronize()
@@ -281,11 +290,19 @@ def run_cuda(args):
             env.rollout_random(T_ROLLOUT, obs, act, rew, done)
         e1.record()
         barrier()
+        if args.dump_outputs and rank == 0:      # before the launches below overwrite the buffers
+            idx = torch.from_numpy(np.sort(np.random.default_rng(DUMP_SEED).choice(N_ENVS, DUMP_ENVS, replace=False))).to(dev)
+            dumped = {name: t.index_select(1, idx).float().cpu().numpy()
+                      for name, t in (("obs", obs), ("actions", act), ("rewards", rew), ("dones", done))}
         t_load = time.perf_counter()
         while len(clocks.rows) < 5 and time.perf_counter() - t_load < 3.0:
             for _ in range(50):
                 env.rollout_random(T_ROLLOUT, obs, act, rew, done)
             torch.cuda.synchronize()
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     ms = max_over_ranks(e0.elapsed_time(e1))
     steps_per_launch = N_ENVS * T_ROLLOUT
     value = world * steps_per_launch * K / (ms * 1e-3)
@@ -408,7 +425,13 @@ def main():
     ap.add_argument("--no-config1", action="store_true", help="skip the BASELINE configs[0] wall-clock/eval-reward pair")
     ap.add_argument("--ppo-envs", type=int, default=0, help="envs per GPU for the PPO section (default: 65536 ball3d, 32768 otherwise)")
     ap.add_argument("--quick", action="store_true", help="fused rollout only (for ncu runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed rollout's obs / actions / rewards / dones to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA rollout (--impl cuda)")
     # Exactly ONE line on stdout: libraries that print there on their own (NCCL's version banner under NCCL_DEBUG, a
     # stray warning) are sent to stderr at the file-descriptor level; the JSON line goes to the real stdout.
     sys.stdout.flush()
