@@ -280,6 +280,15 @@ int tmla_ppo_loss(const float *logits, const float *values, const int32_t *actio
                   int64_t global_rows, int n_actions, const double *adv_sums, int normalize_advantage,
                   float clip_range, float ent_coef, float vf_coef, float *dlogits, float *dvalues,
                   float *stats_out, void *stream);
+/* A2C.train's loss head (SB3 2.9.0 a2c.py), the same pass for the whole rollout as ONE batch:
+ *   policy_loss = -(adv * log_prob).mean(), value_loss = mse(returns, values), entropy_loss = -mean(entropy),
+ *   loss = policy_loss + ent_coef * entropy_loss + vf_coef * value_loss; advantages normalised (as tmla_ppo_loss) only when
+ *   normalize_advantage != 0 (A2C's default is off).  Arguments as tmla_ppo_loss without old_logp and clip_range;
+ *   stats_out float[8] in tmla_ppo_loss's layout with approx_kl and clip_fraction left 0. */
+int tmla_a2c_loss(const float *logits, const float *values, const int32_t *actions, const float *advantages, const float *returns,
+                  const int32_t *index, int64_t rows, int64_t global_rows, int n_actions, const double *adv_sums,
+                  int normalize_advantage, float ent_coef, float vf_coef, float *dlogits, float *dvalues, float *stats_out,
+                  void *stream);
 
 /* clip_grad_norm_(max_norm) + Adam.step fused (after the gradient all-reduce).
  *   grad_scale multiplies the gradient first; state m,v float[np]; step is the 1-based Adam step;
@@ -324,6 +333,20 @@ int tmla_adam_clip_allreduce(tmla_comm *c, float *params, float *grads, float *m
                              float max_grad_norm, float lr, float beta1, float beta2, float eps, int64_t step, float *norm_out,
                              int zero_grads, void *wpack, int obs_dim, int hidden, int n_actions, void *stream);
 
+/* clip_grad_norm_(max_norm) + torch.optim.RMSprop.step (A2C's optimizer: alpha 0.99, eps 1e-5, not centred, no momentum, no
+ * weight decay), in ONE launch (csrc/comm.cu):  square_avg = alpha * square_avg + (1 - alpha) * g^2;  p -= lr * g / (sqrt(square_avg) + eps)
+ * (eps after the square root: torch's rule).  alpha is a double because 1 - alpha is formed from it before rounding to float,
+ * as torch does with the Python float it is given (from a float 0.99 the factor would be 8 ulp off).  Arguments as tmla_adam_clip_fused with the one state vector sq_avg float[np]
+ * instead of m, v; the allreduce form as tmla_adam_clip_allreduce (`step` = exchange sequence number).  There is no two-launch
+ * form: a shape the one launch does not cover (more than 262 144 parameters, buffers not 16-byte aligned, a world other than
+ * 1, 2, 4, 8) returns TMLA_EINVAL. */
+int tmla_rmsprop_clip_fused(float *params, float *grads, float *sq_avg, int64_t num_params, float grad_scale, float max_grad_norm, float lr,
+                            double alpha, float eps, float *norm_out, int zero_grads, void *wpack, int obs_dim, int hidden, int n_actions,
+                            void *stream);
+int tmla_rmsprop_clip_allreduce(tmla_comm *c, float *params, float *grads, float *sq_avg, int64_t num_params, float grad_scale,
+                                float max_grad_norm, float lr, double alpha, float eps, int64_t step, float *norm_out, int zero_grads,
+                                void *wpack, int obs_dim, int hidden, int n_actions, void *stream);
+
 /* ---- tensor-core building blocks (csrc/mlp_tc.cu: tcgen05.mma, TMEM accumulators), bf16 row-major device
  * buffers.  Used by the bf16 MLP path; exported so the parity tests can exercise them in isolation.
  *   tmla_tc_linear: out[M,256] = tanh(A . W^T + bias)            (epi 0; layer-2 forward of a tower)
@@ -362,6 +385,14 @@ int tmla_ppo_minibatch_bf16(const float *params, const void *wpack, int obs_dim,
                             const float *advantages, const float *old_logp, const float *returns, const double *adv_sums,
                             int normalize_advantage, float clip_range, float ent_coef, float vf_coef, float *grads,
                             void *scratch, float *stats_out, float *logits_out, float *values_out, int flags, void *stream);
+/* A2C.train (SB3 2.9.0 a2c.py: rollout_buffer.get(batch_size=None), one gradient step per rollout) fused the same way: the
+ * policy tower runs tmla_a2c_loss's loss instead of the clipped surrogate and reads no old log-probabilities.  Arguments as
+ * tmla_ppo_minibatch_bf16 without old_logp and clip_range; index is normally NULL (the whole rollout, row order irrelevant);
+ * the same shapes as tmla_ppo_minibatch_supported; stats_out as tmla_a2c_loss. */
+int tmla_a2c_batch_bf16(const float *params, const void *wpack, int obs_dim, int hidden, int n_actions, const float *obs,
+                        const int32_t *index, int64_t rows, int64_t global_rows, const int32_t *actions, const float *advantages,
+                        const float *returns, const double *adv_sums, int normalize_advantage, float ent_coef, float vf_coef,
+                        float *grads, void *scratch, float *stats_out, float *logits_out, float *values_out, int flags, void *stream);
 
 /* test hooks of csrc/mlp_train.cu:
  *   tmla_tc_wgrad_tiled: G[256,256] (fp32, accumulated) += X^T . Y where X and Y are given as TILE IMAGES — per 128

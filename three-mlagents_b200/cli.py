@@ -21,7 +21,7 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--trainable-only", action="store_true")
     p = sub.add_parser("inspect", help="Print one environment's spaces")
     p.add_argument("task")
-    p = sub.add_parser("train", help="Train one task (PPO on the CUDA backend)")
+    p = sub.add_parser("train", help="Train one task (PPO or A2C on the CUDA backend)")
     p.add_argument("task")
     p.add_argument("--algorithm", "-a")
     p.add_argument("--timesteps", "-t", type=int)

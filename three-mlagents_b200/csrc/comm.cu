@@ -169,6 +169,8 @@ reduce_norm_kernel(CommPtrs cp, int rank, int world_rt, int64_t capacity, float 
 // refresh of the bf16 operand images, with the (summed) gradient held in registers across the barrier: one launch per minibatch
 // instead of gradnorm + adam (single GPU) or reduce_norm + adam (data parallel), and one pass over the gradient instead of two.
 // Arithmetic per element is adam_kernel's (ppo_kernels.cu); the norm is the fixed-order sum of TMLA_NORM_BLOCKS partials.
+// RMS = true is A2C's torch.optim.RMSprop(alpha, eps) step instead (not centred, no momentum, no weight decay): one state
+// vector, square_avg, in `v`, with b2 = alpha and b1 = 1 - alpha (formed in double from the caller's double alpha, then rounded: torch's factors); `m` is unused.
 struct OptStepArgs {
     CommPtrs cp; int rank, world; int64_t capacity; uint32_t seq; uint32_t *ticket; int *err; long long timeout_ns;   // exchange (WORLD > 1)
     float *p, *g, *m, *v; int64_t np;
@@ -209,7 +211,7 @@ __device__ __forceinline__ void opt_grid_barrier(uint32_t *bar, unsigned nblocks
     __syncthreads();
 }
 
-template <int WORLD>
+template <int WORLD, bool RMS>
 __global__ void __launch_bounds__(kReduceThreads)
 opt_step_kernel(const __grid_constant__ OptStepArgs a) {
     __shared__ float sh[kReduceThreads / 32];
@@ -226,7 +228,11 @@ opt_step_kernel(const __grid_constant__ OptStepArgs a) {
 #pragma unroll
     for (int j = 0; j < kOptVecPerThread; ++j) {
         const int64_t i = gtid + j * gsize;
-        if (i < nvec) { p4[j] = reinterpret_cast<const float4 *>(a.p)[i]; m4[j] = reinterpret_cast<const float4 *>(a.m)[i]; v4[j] = reinterpret_cast<const float4 *>(a.v)[i]; }
+        if (i < nvec) {
+            p4[j] = reinterpret_cast<const float4 *>(a.p)[i];
+            if constexpr (!RMS) m4[j] = reinterpret_cast<const float4 *>(a.m)[i];
+            v4[j] = reinterpret_cast<const float4 *>(a.v)[i];
+        }
     }
     // launched as a programmatic dependent of the weight-gradient kernel: everything above ran beside its last CTAs; the
     // gradient is complete once the prerequisite grids have finished (returns at once after an ordinary launch)
@@ -330,11 +336,18 @@ opt_step_kernel(const __grid_constant__ OptStepArgs a) {
     if (gtid == 0) a.norm_out[0] = norm;
     auto step1 = [&](float gi_raw, float &pp, float &mm, float &vv, int64_t idx) {
         const float gi = gi_raw * a.scale * coef;
-        const float mi = a.b1 * mm + (1.0f - a.b1) * gi;
-        const float vi = a.b2 * vv + (1.0f - a.b2) * gi * gi;
-        mm = mi; vv = vi;
-        const float denom = sqrtf(vi) / a.bc2_sqrt + a.eps;
-        const float pn = pp - (a.lr / a.bc1) * (mi / denom);
+        float pn;
+        if constexpr (RMS) {                                // square_avg = alpha sq + (1 - alpha) g^2;  p -= lr g / (sqrt(sq) + eps)
+            const float vi = a.b2 * vv + a.b1 * gi * gi;
+            vv = vi;
+            pn = pp - a.lr * (gi / (sqrtf(vi) + a.eps));
+        } else {
+            const float mi = a.b1 * mm + (1.0f - a.b1) * gi;
+            const float vi = a.b2 * vv + (1.0f - a.b2) * gi * gi;
+            mm = mi; vv = vi;
+            const float denom = sqrtf(vi) / a.bc2_sqrt + a.eps;
+            pn = pp - (a.lr / a.bc1) * (mi / denom);
+        }
         pp = pn;
         if (a.img0) {                                       // hidden-layer weight: refresh its bf16 operand-image entry
             const int64_t e0 = idx - a.w2_off0, e1 = idx - a.w2_off1;
@@ -351,21 +364,25 @@ opt_step_kernel(const __grid_constant__ OptStepArgs a) {
         if (i < nvec) {
             step1(g[j].x, p4[j].x, m4[j].x, v4[j].x, 4 * i + 0); step1(g[j].y, p4[j].y, m4[j].y, v4[j].y, 4 * i + 1);
             step1(g[j].z, p4[j].z, m4[j].z, v4[j].z, 4 * i + 2); step1(g[j].w, p4[j].w, m4[j].w, v4[j].w, 4 * i + 3);
-            reinterpret_cast<float4 *>(a.p)[i] = p4[j]; reinterpret_cast<float4 *>(a.m)[i] = m4[j]; reinterpret_cast<float4 *>(a.v)[i] = v4[j];
+            reinterpret_cast<float4 *>(a.p)[i] = p4[j];
+            if constexpr (!RMS) reinterpret_cast<float4 *>(a.m)[i] = m4[j];
+            reinterpret_cast<float4 *>(a.v)[i] = v4[j];
             reinterpret_cast<float4 *>(a.g)[i] = a.zero_grads ? make_float4(0.0f, 0.0f, 0.0f, 0.0f) : g[j];
         }
     }
     if (tail_owner) {
         const int64_t i = tail0 + threadIdx.x;
-        float pp = a.p[i], mm = a.m[i], vv = a.v[i];
+        float pp = a.p[i], mm = RMS ? 0.0f : a.m[i], vv = a.v[i];
         step1(gt, pp, mm, vv, i);
-        a.p[i] = pp; a.m[i] = mm; a.v[i] = vv;
+        a.p[i] = pp;
+        if (!RMS) a.m[i] = mm;
+        a.v[i] = vv;
         a.g[i] = a.zero_grads ? 0.0f : gt;
     }
 }
 
-// one launch (ordinary or programmatic dependent; own grid barrier); returns TMLA_EINVAL (without an error message) when the shape does not fit so that callers fall back
-template <int WORLD>
+// one launch (ordinary or programmatic dependent; own grid barrier)
+template <int WORLD, bool RMS>
 static int opt_step_launch_t(OptStepArgs &a, cudaStream_t st) {
     static const int mode = [] { const char *e = getenv("TMLA_OPT_PDL"); return e ? atoi(e) : 1; }();   // 0: ordinary launch, 1: programmatic dependent
     cudaLaunchConfig_t cfg;
@@ -375,46 +392,83 @@ static int opt_step_launch_t(OptStepArgs &a, cudaStream_t st) {
     attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr.val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = &attr; cfg.numAttrs = mode ? 1 : 0;
-    TMLA_CUDA(cudaLaunchKernelEx(&cfg, opt_step_kernel<WORLD>, a));
+    TMLA_CUDA(cudaLaunchKernelEx(&cfg, opt_step_kernel<WORLD, RMS>, a));
     return TMLA_OK;
 }
 static bool opt_step_enabled() {      // TMLA_ADAM=split keeps the two-launch path (A/B runs)
     static const bool on = [] { const char *e = getenv("TMLA_ADAM"); return !(e && !strcmp(e, "split")); }();
     return on;
 }
+static bool opt_step_fits(const float *params, const float *grads, const float *m, const float *v, int64_t num_params) {
+    return (num_params >> 2) <= (int64_t)kReduceBlocks * kReduceThreads * kOptVecPerThread && (num_params & 3) < kReduceThreads &&
+           !((reinterpret_cast<uintptr_t>(grads) | reinterpret_cast<uintptr_t>(params) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15u);
+}
+static void opt_step_comm(OptStepArgs &a, const tmla_comm *c, int64_t step) {
+    for (int q = 0; q < kMaxRanks; ++q) a.cp.peer[q] = q < c->world ? c->peer[q] : nullptr;
+    a.rank = c->rank; a.world = c->world; a.capacity = c->capacity; a.ticket = c->ticket; a.err = c->err; a.timeout_ns = c->timeout_ns;
+    a.seq = (uint32_t)(step & 0x7FFFFFFF) | 0x80000000u;
+}
+static int opt_step_images(OptStepArgs &a, void *wpack, int obs_dim, int hidden, int n_actions, int64_t num_params) {
+    if (!wpack) return TMLA_OK;
+    if (hidden != 256) return TMLA_EINVAL;
+    const MlpOffsets o = mlp_offsets(obs_dim, n_actions);
+    if (o.total != num_params) return TMLA_EINVAL;
+    a.img0 = reinterpret_cast<__nv_bfloat16 *>(wpack) + (int64_t)4 * 65536; a.img1 = a.img0 + 65536;
+    a.w2_off0 = o.w2[0]; a.w2_off1 = o.w2[1];
+    return TMLA_OK;
+}
+template <bool RMS>
+static int opt_step_dispatch(const tmla_comm *c, OptStepArgs &a, cudaStream_t st) {
+    switch (c ? c->world : 1) {
+        case 1: return opt_step_launch_t<1, RMS>(a, st);
+        case 2: return opt_step_launch_t<2, RMS>(a, st);
+        case 4: return opt_step_launch_t<4, RMS>(a, st);
+        case 8: return opt_step_launch_t<8, RMS>(a, st);
+        default: return TMLA_EINVAL;
+    }
+}
+
+// returns TMLA_EINVAL (without an error message) when the shape does not fit so that callers fall back
 int opt_step_launch(tmla_comm *c, float *params, float *grads, float *m, float *v, int64_t num_params, float grad_scale, float max_grad_norm,
                     float lr, float beta1, float beta2, float eps, int64_t step, float *norm_out, int zero_grads, void *wpack, int obs_dim,
                     int hidden, int n_actions, void *stream) {
-    if (!opt_step_enabled() || (num_params >> 2) > (int64_t)kReduceBlocks * kReduceThreads * kOptVecPerThread || (num_params & 3) >= kReduceThreads ||
-        (reinterpret_cast<uintptr_t>(grads) | reinterpret_cast<uintptr_t>(params) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15u)
+    if (!opt_step_enabled() || !opt_step_fits(params, grads, m, v, num_params))
         return TMLA_EINVAL;
     OptStepArgs a;
     memset(&a, 0, sizeof(a));
-    if (c) {
-        for (int q = 0; q < kMaxRanks; ++q) a.cp.peer[q] = q < c->world ? c->peer[q] : nullptr;
-        a.rank = c->rank; a.world = c->world; a.capacity = c->capacity; a.ticket = c->ticket; a.err = c->err; a.timeout_ns = c->timeout_ns;
-        a.seq = (uint32_t)(step & 0x7FFFFFFF) | 0x80000000u;
-    }
+    if (c) opt_step_comm(a, c, step);
     a.p = params; a.g = grads; a.m = m; a.v = v; a.np = num_params;
     const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
     a.scale = grad_scale; a.max_norm = max_grad_norm; a.lr = lr; a.b1 = beta1; a.b2 = beta2; a.eps = eps; a.bc1 = (float)bc1; a.bc2_sqrt = (float)sqrt(bc2);
     a.norm_out = norm_out; a.zero_grads = zero_grads;
-    if (wpack) {
-        if (hidden != 256) return TMLA_EINVAL;
-        const MlpOffsets o = mlp_offsets(obs_dim, n_actions);
-        if (o.total != num_params) return TMLA_EINVAL;
-        a.img0 = reinterpret_cast<__nv_bfloat16 *>(wpack) + (int64_t)4 * 65536; a.img1 = a.img0 + 65536;
-        a.w2_off0 = o.w2[0]; a.w2_off1 = o.w2[1];
+    if (opt_step_images(a, wpack, obs_dim, hidden, n_actions, num_params)) return TMLA_EINVAL;
+    return opt_step_dispatch<false>(c, a, (cudaStream_t)stream);
+}
+
+// clip + RMSprop: this one-launch form only (no two-launch fallback, TMLA_ADAM does not apply)
+static int rmsprop_launch(tmla_comm *c, float *params, float *grads, float *sq_avg, int64_t num_params, float grad_scale, float max_grad_norm,
+                          float lr, double alpha, float eps, int64_t step, float *norm_out, int zero_grads, void *wpack, int obs_dim, int hidden,
+                          int n_actions, void *stream) {
+    TMLA_REQUIRE(params && grads && sq_avg && norm_out, "NULL buffer (norm_out doubles as scratch)");
+    TMLA_REQUIRE(num_params > 0, "num_params must be positive");
+    if (!opt_step_fits(params, grads, sq_avg, sq_avg, num_params)) {
+        tmla_set_error("clip + RMSprop runs as one launch only: at most %d parameters in 16-byte aligned buffers (got %lld)",
+                       kReduceBlocks * kReduceThreads * kOptVecPerThread * 4, (long long)num_params);
+        return TMLA_EINVAL;
     }
-    cudaStream_t st = (cudaStream_t)stream;
-    const int world = c ? c->world : 1;
-    switch (world) {
-        case 1: return opt_step_launch_t<1>(a, st);
-        case 2: return opt_step_launch_t<2>(a, st);
-        case 4: return opt_step_launch_t<4>(a, st);
-        case 8: return opt_step_launch_t<8>(a, st);
-        default: return TMLA_EINVAL;
+    OptStepArgs a;
+    memset(&a, 0, sizeof(a));
+    if (c) opt_step_comm(a, c, step);
+    a.p = params; a.g = grads; a.v = sq_avg; a.np = num_params;
+    a.scale = grad_scale; a.max_norm = max_grad_norm; a.lr = lr; a.b2 = (float)alpha; a.b1 = (float)(1.0 - alpha); a.eps = eps;
+    a.norm_out = norm_out; a.zero_grads = zero_grads;
+    if (opt_step_images(a, wpack, obs_dim, hidden, n_actions, num_params)) {
+        tmla_set_error("wpack needs hidden = 256 and num_params matching (obs_dim, n_actions)");
+        return TMLA_EINVAL;
     }
+    const int rc = opt_step_dispatch<true>(c, a, (cudaStream_t)stream);
+    if (rc == TMLA_EINVAL) tmla_set_error("clip + RMSprop with a gradient exchange covers 2, 4 or 8 ranks (got %d)", c ? c->world : 1);
+    return rc;
 }
 
 extern "C" {
@@ -539,6 +593,24 @@ int tmla_adam_clip_allreduce(tmla_comm *c, float *params, float *grads, float *m
     TMLA_LAUNCH_CHECK();
     return adam_clip_launch(params, grads, m, v, num_params, grad_scale, max_grad_norm, lr, beta1, beta2, eps, step, norm_out, zero_grads,
                             wpack, obs_dim, hidden, n_actions, stream, true);
+}
+
+// torch.nn.utils.clip_grad_norm_ + torch.optim.RMSprop.step (A2C), as tmla_adam_clip_fused with one state vector
+int tmla_rmsprop_clip_fused(float *params, float *grads, float *sq_avg, int64_t num_params, float grad_scale, float max_grad_norm, float lr,
+                            double alpha, float eps, float *norm_out, int zero_grads, void *wpack, int obs_dim, int hidden, int n_actions,
+                            void *stream) {
+    return rmsprop_launch(nullptr, params, grads, sq_avg, num_params, grad_scale, max_grad_norm, lr, alpha, eps, 1, norm_out, zero_grads, wpack,
+                          obs_dim, hidden, n_actions, stream);
+}
+
+// grads <- sum over ranks (rank order), then clip + RMSprop in the same launch; `step` is the exchange sequence number
+int tmla_rmsprop_clip_allreduce(tmla_comm *c, float *params, float *grads, float *sq_avg, int64_t num_params, float grad_scale,
+                                float max_grad_norm, float lr, double alpha, float eps, int64_t step, float *norm_out, int zero_grads,
+                                void *wpack, int obs_dim, int hidden, int n_actions, void *stream) {
+    TMLA_REQUIRE(c && c->connected, "comm is NULL or not connected (tmla_comm_connect)");
+    TMLA_REQUIRE(num_params <= c->capacity && step >= 1, "bad arguments (num_params exceeds the comm's capacity?)");
+    return rmsprop_launch(c, params, grads, sq_avg, num_params, grad_scale, max_grad_norm, lr, alpha, eps, step, norm_out, zero_grads, wpack,
+                          obs_dim, hidden, n_actions, stream);
 }
 
 }  // extern "C"

@@ -181,7 +181,11 @@ struct TrainSmem {
 #endif
 };
 
-template <int D, int NOUT>
+// loss of the policy tower (the value tower's mean squared error is the same for both): PPO's clipped surrogate, or A2C's plain
+// policy gradient -(adv * log_prob).mean() (SB3 2.9.0 a2c.py), which has no ratio, no clip and reads no old log-probabilities
+enum { kLossPPO = 0, kLossA2C = 1 };
+
+template <int D, int NOUT, int LOSS = kLossPPO>
 __global__ void __launch_bounds__(kTrainThreads + 32, 1)
 tc_tower_train_kernel(const __grid_constant__ TowerTrainArgs p) {
     using L = TrainSmem<D, NOUT>;
@@ -251,7 +255,7 @@ tc_tower_train_kernel(const __grid_constant__ TowerTrainArgs p) {
             if (PI) {
                 cp_async_ca<4>(dst, p.actions + src, ok ? 4u : 0u);
                 cp_async_ca<4>(dst + 4, p.adv + src, ok ? 4u : 0u);
-                cp_async_ca<4>(dst + 8, p.old_logp + src, ok ? 4u : 0u);
+                if (LOSS == kLossPPO) cp_async_ca<4>(dst + 8, p.old_logp + src, ok ? 4u : 0u);
             } else cp_async_ca<4>(dst, p.returns + src, ok ? 4u : 0u);
         }
     };
@@ -547,20 +551,31 @@ tc_tower_train_kernel(const __grid_constant__ TowerTrainArgs p) {
                 for (int j = 1; j < NOUT; ++j) logp = (a_cur == j) ? lp[j] : logp;
                 float adv = f0_cur;
                 if (p.normalize) adv = (adv - advc[0]) * advc[1];
-                const float lr = logp - f1_cur;
-                const float ratio = __expf(lr);
-                const float lo = 1.0f - p.clip, hi = 1.0f + p.clip;
-                const float s1 = adv * ratio, s2 = adv * fminf(fmaxf(ratio, lo), hi);
-                const bool inside = (ratio >= lo) && (ratio <= hi);
-                const bool active = inside || (s1 < s2);
-                const float dlogp = active ? (-adv * ratio * p.inv_rows) : 0.0f;
+                if constexpr (LOSS == kLossA2C) {
+                    if (valid) {                          // (statistics first: log_prob dies here) approx_kl / clip_fraction stay 0
+                        float *ra = racc + rt * L::RS;
+                        ra[0] += -adv * logp; ra[1] += -ent;
+                    }
+                    const float dlogp = -adv * p.inv_rows;
 #pragma unroll
-                for (int j = 0; j < NOUT; ++j)
-                    dz[j] = valid ? dlogp * ((a_cur == j ? 1.0f : 0.0f) - pr[j]) + p.ent_coef * p.inv_rows * pr[j] * (lp[j] + ent) : 0.0f;
-                if (valid) {
-                    float *ra = racc + rt * L::RS;
-                    ra[0] += -fminf(s1, s2); ra[1] += -ent; ra[2] += (ratio - 1.0f) - lr;
-                    ra[3] += (fabsf(ratio - 1.0f) > p.clip) ? 1.0f : 0.0f;
+                    for (int j = 0; j < NOUT; ++j)
+                        dz[j] = valid ? dlogp * ((a_cur == j ? 1.0f : 0.0f) - pr[j]) + p.ent_coef * p.inv_rows * pr[j] * (lp[j] + ent) : 0.0f;
+                } else {
+                    const float lr = logp - f1_cur;
+                    const float ratio = __expf(lr);
+                    const float lo = 1.0f - p.clip, hi = 1.0f + p.clip;
+                    const float s1 = adv * ratio, s2 = adv * fminf(fmaxf(ratio, lo), hi);
+                    const bool inside = (ratio >= lo) && (ratio <= hi);
+                    const bool active = inside || (s1 < s2);
+                    const float dlogp = active ? (-adv * ratio * p.inv_rows) : 0.0f;
+#pragma unroll
+                    for (int j = 0; j < NOUT; ++j)
+                        dz[j] = valid ? dlogp * ((a_cur == j ? 1.0f : 0.0f) - pr[j]) + p.ent_coef * p.inv_rows * pr[j] * (lp[j] + ent) : 0.0f;
+                    if (valid) {
+                        float *ra = racc + rt * L::RS;
+                        ra[0] += -fminf(s1, s2); ra[1] += -ent; ra[2] += (ratio - 1.0f) - lr;
+                        ra[3] += (fabsf(ratio - 1.0f) > p.clip) ? 1.0f : 0.0f;
+                    }
                 }
             } else {
                 const float dv = z[0] - f0_cur;
@@ -1271,13 +1286,13 @@ static int wgrad_h1_launch_t(const WgradH1Problem &a, const WgradH1Problem &b, c
     return TMLA_OK;
 }
 
-template <int D, int NOUT>
+template <int D, int NOUT, int LOSS = kLossPPO>
 static int tower_train_launch_t(const TowerTrainArgs &a, cudaStream_t st, bool overlap_prev) {
     static int attr_done = 0;
     constexpr uint32_t smem = TrainSmem<D, NOUT>::total;
     static_assert(smem <= 232448, "fused tower training kernel exceeds the 227 KB shared-memory limit");
     if (!attr_done) {
-        TMLA_CUDA(cudaFuncSetAttribute(tc_tower_train_kernel<D, NOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        TMLA_CUDA(cudaFuncSetAttribute(tc_tower_train_kernel<D, NOUT, LOSS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_done = 1;
     }
     const unsigned grid = (unsigned)std::min<int64_t>((a.M + 127) / 128, sm_count_train());
@@ -1292,9 +1307,9 @@ static int tower_train_launch_t(const TowerTrainArgs &a, cudaStream_t st, bool o
         attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr.val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = &attr; cfg.numAttrs = 1;
-        TMLA_CUDA(cudaLaunchKernelEx(&cfg, tc_tower_train_kernel<D, NOUT>, a));
+        TMLA_CUDA(cudaLaunchKernelEx(&cfg, tc_tower_train_kernel<D, NOUT, LOSS>, a));
     } else {
-        tc_tower_train_kernel<D, NOUT><<<grid, kTrainThreads + 32, smem, st>>>(a);
+        tc_tower_train_kernel<D, NOUT, LOSS><<<grid, kTrainThreads + 32, smem, st>>>(a);
     }
     TMLA_LAUNCH_CHECK();
     return TMLA_OK;
@@ -1309,16 +1324,25 @@ int tmla_ppo_minibatch_supported(int obs_dim, int hidden, int n_actions) {
 
 int64_t tmla_ppo_minibatch_scratch(int hidden, int64_t rows) { return 4 * ((rows + 127) / 128 * 128) * (int64_t)hidden; }
 
-int tmla_ppo_minibatch_bf16(const float *params, const void *wpack, int obs_dim, int hidden, int n_actions, const float *obs,
-                            const int32_t *index, int64_t rows, int64_t global_rows, const int32_t *actions,
-                            const float *advantages, const float *old_logp, const float *returns, const double *adv_sums,
-                            int normalize_advantage, float clip_range, float ent_coef, float vf_coef, float *grads,
-                            void *scratch, float *stats_out, float *logits_out, float *values_out, int flags, void *stream) {
-    TMLA_REQUIRE(params && wpack && obs && actions && advantages && old_logp && returns && grads && scratch && stats_out, "NULL buffer");
+}  // extern "C"
+
+template <int D, int A>
+static int policy_tower_launch(const TowerTrainArgs &a, cudaStream_t st, int loss) {
+    return loss == kLossA2C ? tower_train_launch_t<D, A, kLossA2C>(a, st, false) : tower_train_launch_t<D, A>(a, st, false);
+}
+
+// one fused batch of either loss: the policy tower with PPO's or A2C's loss, the shared value tower, the weight-gradient GEMMs
+static int tower_batch_launch(int loss, const char *fn, const float *params, const void *wpack, int obs_dim, int hidden, int n_actions,
+                              const float *obs, const int32_t *index, int64_t rows, int64_t global_rows, const int32_t *actions,
+                              const float *advantages, const float *old_logp, const float *returns, const double *adv_sums,
+                              int normalize_advantage, float clip_range, float ent_coef, float vf_coef, float *grads,
+                              void *scratch, float *stats_out, float *logits_out, float *values_out, int flags, void *stream) {
+    TMLA_REQUIRE(params && wpack && obs && actions && advantages && (old_logp || loss == kLossA2C) && returns && grads && scratch && stats_out,
+                 "NULL buffer");
     TMLA_REQUIRE(rows > 0 && global_rows >= rows, "bad row counts");
     TMLA_REQUIRE(!normalize_advantage || adv_sums, "adv_sums required when normalising");
     if (!tmla_ppo_minibatch_supported(obs_dim, hidden, n_actions)) {
-        tmla_set_error("tmla_ppo_minibatch_bf16: fused path covers hidden=256 with (obs_dim, actions) = (6,5), (4,5), (4,4), (7,3) (got %d/%d/%d)", obs_dim, hidden, n_actions);
+        tmla_set_error("%s: fused path covers hidden=256 with (obs_dim, actions) = (6,5), (4,5), (4,4), (7,3) (got %d/%d/%d)", fn, obs_dim, hidden, n_actions);
         return TMLA_EINVAL;
     }
     cudaStream_t st = (cudaStream_t)stream;
@@ -1354,10 +1378,10 @@ int tmla_ppo_minibatch_bf16(const float *params, const void *wpack, int obs_dim,
         a.gW1 = grads + o.w1[t]; a.gB1 = grads + o.b1[t]; a.gB2 = grads + o.b2[t]; a.gWh = grads + o.wh[t]; a.gBh = grads + o.bh[t];
         a.stats = stats_out;
         int rc;
-        if (obs_dim == 6) rc = t == 0 ? tower_train_launch_t<6, 5>(a, st, false) : tower_train_launch_t<6, 1>(a, st, pdl);
-        else if (obs_dim == 7) rc = t == 0 ? tower_train_launch_t<7, 3>(a, st, false) : tower_train_launch_t<7, 1>(a, st, pdl);
-        else if (n_actions == 5) rc = t == 0 ? tower_train_launch_t<4, 5>(a, st, false) : tower_train_launch_t<4, 1>(a, st, pdl);
-        else rc = t == 0 ? tower_train_launch_t<4, 4>(a, st, false) : tower_train_launch_t<4, 1>(a, st, pdl);
+        if (obs_dim == 6) rc = t == 0 ? policy_tower_launch<6, 5>(a, st, loss) : tower_train_launch_t<6, 1>(a, st, pdl);
+        else if (obs_dim == 7) rc = t == 0 ? policy_tower_launch<7, 3>(a, st, loss) : tower_train_launch_t<7, 1>(a, st, pdl);
+        else if (n_actions == 5) rc = t == 0 ? policy_tower_launch<4, 5>(a, st, loss) : tower_train_launch_t<4, 1>(a, st, pdl);
+        else rc = t == 0 ? policy_tower_launch<4, 4>(a, st, loss) : tower_train_launch_t<4, 1>(a, st, pdl);
         if (rc) return rc;
         if (interleave) { rc = tc_wgrad_tiled_launch(img[t][1], img[t][0], grads + o.w2[t], rows_padded, st); if (rc) return rc; }
     }
@@ -1369,6 +1393,27 @@ int tmla_ppo_minibatch_bf16(const float *params, const void *wpack, int obs_dim,
         return wgrad_h1_launch_t<4>(pa, pb, obs, index, rows, rows_padded, st);
     }
     return tc_wgrad_tiled_launch(img[0][1], img[0][0], grads + o.w2[0], rows_padded, st, img[1][1], img[1][0], grads + o.w2[1], pdl_wgrad);
+}
+
+extern "C" {
+
+int tmla_ppo_minibatch_bf16(const float *params, const void *wpack, int obs_dim, int hidden, int n_actions, const float *obs,
+                            const int32_t *index, int64_t rows, int64_t global_rows, const int32_t *actions,
+                            const float *advantages, const float *old_logp, const float *returns, const double *adv_sums,
+                            int normalize_advantage, float clip_range, float ent_coef, float vf_coef, float *grads,
+                            void *scratch, float *stats_out, float *logits_out, float *values_out, int flags, void *stream) {
+    return tower_batch_launch(kLossPPO, "tmla_ppo_minibatch_bf16", params, wpack, obs_dim, hidden, n_actions, obs, index, rows, global_rows,
+                              actions, advantages, old_logp, returns, adv_sums, normalize_advantage, clip_range, ent_coef, vf_coef, grads,
+                              scratch, stats_out, logits_out, values_out, flags, stream);
+}
+
+int tmla_a2c_batch_bf16(const float *params, const void *wpack, int obs_dim, int hidden, int n_actions, const float *obs,
+                        const int32_t *index, int64_t rows, int64_t global_rows, const int32_t *actions, const float *advantages,
+                        const float *returns, const double *adv_sums, int normalize_advantage, float ent_coef, float vf_coef,
+                        float *grads, void *scratch, float *stats_out, float *logits_out, float *values_out, int flags, void *stream) {
+    return tower_batch_launch(kLossA2C, "tmla_a2c_batch_bf16", params, wpack, obs_dim, hidden, n_actions, obs, index, rows, global_rows,
+                              actions, advantages, nullptr, returns, adv_sums, normalize_advantage, 0.0f, ent_coef, vf_coef, grads,
+                              scratch, stats_out, logits_out, values_out, flags, stream);
 }
 
 int tmla_tc_wgrad_tiled(const void *Xt, const void *Yt, float *G, int64_t rows_padded, void *stream) {

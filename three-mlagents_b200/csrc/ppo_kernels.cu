@@ -2,7 +2,7 @@
 //   K6  gae_kernel            RolloutBuffer.compute_returns_and_advantage   (buffers.py, SB3 2.9.0)
 //   -   permutation_kernel    RolloutBuffer.get  (np.random.permutation + swapaxes flatten)
 //   K7  adv_stats_kernel      advantages.mean()/.std() of PPO.train (warp-shuffle reductions)
-//   K8  ppo_loss_kernel       clipped surrogate + value MSE + entropy, forward AND backward
+//   K8  ppo_loss_kernel       clipped surrogate + value MSE + entropy, forward AND backward (A2C.train: plain policy gradient)
 //   K11 gradnorm/adam kernels clip_grad_norm_ + Adam.step
 //   -   bootstrap_add_kernel  collect_rollouts' `rewards[i] += gamma * V(terminal_obs)`
 // Reached in the reference from backend/mlagents/training.py:150,166 with the hyper-parameters of
@@ -174,8 +174,10 @@ adv_stats_batched_kernel(const float *__restrict__ adv, const int32_t *__restric
 // One thread per sample of the minibatch.  Everything SB3's PPO.train does between evaluate_actions
 // and loss.backward() for Categorical policies, with the analytic gradient of
 //   loss = -mean(min(A r, A clip(r))) + ent_coef * -mean(H) + vf_coef * mean((R - V)^2)
-// written straight into dlogits / dvalues (scaled by 1/global_rows).
-template <int A>
+// written straight into dlogits / dvalues (scaled by 1/global_rows).  A2C (SB3 2.9.0 a2c.py) replaces the surrogate by
+//   -mean(A log pi(a|s))  (no ratio, no clip, no old_logp; approx_kl / clip_fraction stay 0)
+enum { kLossPPO = 0, kLossA2C = 1 };
+template <int A, int LOSS = kLossPPO>
 __global__ void __launch_bounds__(256)
 ppo_loss_kernel(const float *__restrict__ logits, const float *__restrict__ values, const int32_t *__restrict__ actions,
                 const float *__restrict__ advantages, const float *__restrict__ old_logp, const float *__restrict__ returns,
@@ -216,24 +218,37 @@ ppo_loss_kernel(const float *__restrict__ logits, const float *__restrict__ valu
         for (int j = 1; j < A; ++j) logp = (a == j) ? lp[j] : logp;
         float adv = advantages[src];
         if (normalize) adv = (adv - mean) * inv_std;
-        const float lr = logp - old_logp[src];
-        const float ratio = expf(lr);
-        const float lo = 1.0f - clip, hi = 1.0f + clip;
-        const float s1 = adv * ratio, s2 = adv * fminf(fmaxf(ratio, lo), hi);
-        const bool inside = (ratio >= lo) && (ratio <= hi);
-        const bool active = inside || (s1 < s2);
-        const float dlogp = active ? (-adv * ratio * invB) : 0.0f;
-        const float v = values[r], R = returns[src];
-        const float dv = v - R;
-        dvalues[r] = vf_coef * 2.0f * dv * invB;
+        if constexpr (LOSS == kLossA2C) {
+            const float dlogp = -adv * invB;
+            const float v = values[r], R = returns[src];
+            const float dv = v - R;
+            dvalues[r] = vf_coef * 2.0f * dv * invB;
 #pragma unroll
-        for (int j = 0; j < A; ++j)
-            dlogits[r * A + j] = dlogp * ((a == j ? 1.0f : 0.0f) - p[j]) + ent_coef * invB * p[j] * (lp[j] + ent);
-        acc[0] = -fminf(s1, s2);
-        acc[1] = dv * dv;
-        acc[2] = -ent;
-        acc[3] = (ratio - 1.0f) - lr;
-        acc[4] = (fabsf(ratio - 1.0f) > clip) ? 1.0f : 0.0f;
+            for (int j = 0; j < A; ++j)
+                dlogits[r * A + j] = dlogp * ((a == j ? 1.0f : 0.0f) - p[j]) + ent_coef * invB * p[j] * (lp[j] + ent);
+            acc[0] = -adv * logp;
+            acc[1] = dv * dv;
+            acc[2] = -ent;
+        } else {
+            const float lr = logp - old_logp[src];
+            const float ratio = expf(lr);
+            const float lo = 1.0f - clip, hi = 1.0f + clip;
+            const float s1 = adv * ratio, s2 = adv * fminf(fmaxf(ratio, lo), hi);
+            const bool inside = (ratio >= lo) && (ratio <= hi);
+            const bool active = inside || (s1 < s2);
+            const float dlogp = active ? (-adv * ratio * invB) : 0.0f;
+            const float v = values[r], R = returns[src];
+            const float dv = v - R;
+            dvalues[r] = vf_coef * 2.0f * dv * invB;
+#pragma unroll
+            for (int j = 0; j < A; ++j)
+                dlogits[r * A + j] = dlogp * ((a == j ? 1.0f : 0.0f) - p[j]) + ent_coef * invB * p[j] * (lp[j] + ent);
+            acc[0] = -fminf(s1, s2);
+            acc[1] = dv * dv;
+            acc[2] = -ent;
+            acc[3] = (ratio - 1.0f) - lr;
+            acc[4] = (fabsf(ratio - 1.0f) > clip) ? 1.0f : 0.0f;
+        }
     }
     const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
 #pragma unroll
@@ -369,27 +384,49 @@ int tmla_adv_stats_batched(const float *advantages, const int32_t *index, int64_
     return TMLA_OK;
 }
 
-int tmla_ppo_loss(const float *logits, const float *values, const int32_t *actions, const float *advantages,
-                  const float *old_logp, const float *returns, const int32_t *index, int64_t rows, int64_t global_rows,
-                  int n_actions, const double *adv_sums, int normalize_advantage, float clip_range, float ent_coef,
-                  float vf_coef, float *dlogits, float *dvalues, float *stats_out, void *stream) {
-    TMLA_REQUIRE(logits && values && actions && advantages && old_logp && returns && dlogits && dvalues && stats_out, "NULL buffer");
+}  // extern "C"
+
+template <int LOSS>
+static int loss_launch(const char *fn, const float *logits, const float *values, const int32_t *actions, const float *advantages,
+                       const float *old_logp, const float *returns, const int32_t *index, int64_t rows, int64_t global_rows,
+                       int n_actions, const double *adv_sums, int normalize_advantage, float clip_range, float ent_coef,
+                       float vf_coef, float *dlogits, float *dvalues, float *stats_out, void *stream) {
+    TMLA_REQUIRE(logits && values && actions && advantages && (old_logp || LOSS == kLossA2C) && returns && dlogits && dvalues && stats_out,
+                 "NULL buffer");
     TMLA_REQUIRE(rows > 0 && global_rows >= rows, "bad row counts");
     TMLA_REQUIRE(!normalize_advantage || adv_sums, "adv_sums required when normalising");
     cudaStream_t st = (cudaStream_t)stream;
     TMLA_CUDA(cudaMemsetAsync(stats_out, 0, 8 * sizeof(float), st));
     const unsigned grid = (unsigned)ceil_div64(rows, 256);
     const double inv = 1.0 / (double)global_rows;
-#define LOSS_LAUNCH(AA)                                                                                              \
-    ppo_loss_kernel<AA><<<grid, 256, 0, st>>>(logits, values, actions, advantages, old_logp, returns, index, rows, inv, \
-                                              adv_sums, normalize_advantage, clip_range, ent_coef, vf_coef, dlogits, dvalues, stats_out)
+#define LOSS_LAUNCH(AA)                                                                                                    \
+    ppo_loss_kernel<AA, LOSS><<<grid, 256, 0, st>>>(logits, values, actions, advantages, old_logp, returns, index, rows, inv, \
+                                                    adv_sums, normalize_advantage, clip_range, ent_coef, vf_coef, dlogits, dvalues, stats_out)
     if (n_actions == 3) LOSS_LAUNCH(3);
     else if (n_actions == 4) LOSS_LAUNCH(4);
     else if (n_actions == 5) LOSS_LAUNCH(5);
-    else { tmla_set_error("tmla_ppo_loss: n_actions must be 3, 4 or 5 (got %d)", n_actions); return TMLA_EINVAL; }
+    else { tmla_set_error("%s: n_actions must be 3, 4 or 5 (got %d)", fn, n_actions); return TMLA_EINVAL; }
 #undef LOSS_LAUNCH
     TMLA_LAUNCH_CHECK();
     return TMLA_OK;
+}
+
+extern "C" {
+
+int tmla_ppo_loss(const float *logits, const float *values, const int32_t *actions, const float *advantages,
+                  const float *old_logp, const float *returns, const int32_t *index, int64_t rows, int64_t global_rows,
+                  int n_actions, const double *adv_sums, int normalize_advantage, float clip_range, float ent_coef,
+                  float vf_coef, float *dlogits, float *dvalues, float *stats_out, void *stream) {
+    return loss_launch<kLossPPO>("tmla_ppo_loss", logits, values, actions, advantages, old_logp, returns, index, rows, global_rows, n_actions,
+                                 adv_sums, normalize_advantage, clip_range, ent_coef, vf_coef, dlogits, dvalues, stats_out, stream);
+}
+
+int tmla_a2c_loss(const float *logits, const float *values, const int32_t *actions, const float *advantages, const float *returns,
+                  const int32_t *index, int64_t rows, int64_t global_rows, int n_actions, const double *adv_sums,
+                  int normalize_advantage, float ent_coef, float vf_coef, float *dlogits, float *dvalues, float *stats_out,
+                  void *stream) {
+    return loss_launch<kLossA2C>("tmla_a2c_loss", logits, values, actions, advantages, nullptr, returns, index, rows, global_rows, n_actions,
+                                 adv_sums, normalize_advantage, 0.0f, ent_coef, vf_coef, dlogits, dvalues, stats_out, stream);
 }
 
 }  // extern "C"

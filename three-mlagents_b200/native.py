@@ -94,6 +94,7 @@ SIGNATURES = {
     "tmla_adv_stats": (_i, [vp, vp, i64, vp, vp]),
     "tmla_adv_stats_batched": (_i, [vp, vp, i64, i64, vp, vp]),
     "tmla_ppo_loss": (_i, [vp, vp, vp, vp, vp, vp, vp, i64, i64, _i, vp, _i, f32, f32, f32, vp, vp, vp, vp]),
+    "tmla_a2c_loss": (_i, [vp, vp, vp, vp, vp, vp, i64, i64, _i, vp, _i, f32, f32, vp, vp, vp, vp]),
     "tmla_tc_linear": (_i, [_i, vp, vp, vp, vp, vp, i64, vp, vp]),
     "tmla_tc_wgrad": (_i, [vp, vp, vp, i64, vp]),
     "tmla_f32_to_bf16": (_i, [vp, vp, i64, vp]),
@@ -106,10 +107,13 @@ SIGNATURES = {
     "tmla_comm_destroy": (_i, [vp]),
     "tmla_comm_check": (_i, [vp, vp]),
     "tmla_adam_clip_allreduce": (_i, [vp, vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, f32, i64, vp, _i, vp, _i, _i, _i, vp]),
+    "tmla_rmsprop_clip_fused": (_i, [vp, vp, vp, i64, f32, f32, f32, f64, f32, vp, _i, vp, _i, _i, _i, vp]),
+    "tmla_rmsprop_clip_allreduce": (_i, [vp, vp, vp, vp, i64, f32, f32, f32, f64, f32, i64, vp, _i, vp, _i, _i, _i, vp]),
     "tmla_ppo_minibatch_supported": (_i, [_i, _i, _i]),
     "tmla_ppo_minibatch_scratch": (i64, [_i, i64]),
     "tmla_ppo_minibatch_bf16": (_i, [vp, vp, _i, _i, _i, vp, vp, i64, i64, vp, vp, vp, vp, vp, _i, f32, f32, f32, vp, vp, vp,
                                      vp, vp, _i, vp]),
+    "tmla_a2c_batch_bf16": (_i, [vp, vp, _i, _i, _i, vp, vp, i64, i64, vp, vp, vp, vp, _i, f32, f32, vp, vp, vp, vp, vp, _i, vp]),
     "tmla_tc_wgrad_tiled": (_i, [vp, vp, vp, i64, vp]),
     "tmla_tc_probe": (_i, [vp, vp, vp, _i, vp]),
     "tmla_tc_overlap_probe": (_i, [vp, _i, _i, _i, vp]),

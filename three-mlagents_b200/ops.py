@@ -1,4 +1,4 @@
-"""Torch-tensor wrappers over the PPO entry points of libtmla.so (include/tmla.h).
+"""Torch-tensor wrappers over the PPO and A2C entry points of libtmla.so (include/tmla.h).
 
 Each function takes CUDA tensors, checks dtype/contiguity/device, and enqueues the kernel on
 torch's current stream.  torch is plumbing here (memory + streams); the arithmetic is in csrc/.
@@ -157,6 +157,28 @@ def ppo_loss(logits, values, actions, advantages, old_logp, returns, *, index=No
     return dlogits, dvalues, stats
 
 
+def a2c_loss(logits, values, actions, advantages, returns, *, index=None, rows=None, global_rows=None, adv_sums=None,
+             normalize=False, ent_coef=0.0, vf_coef=0.5, dlogits=None, dvalues=None, stats=None):
+    """A2C.train's loss head (tmla_a2c_loss): ppo_loss without old_logp and clip_range; normalisation off by default (SB3's A2C)."""
+    if rows is None:
+        rows = logits.shape[0]
+    n_actions = logits.shape[1]
+    dev = logits.device
+    _chk(actions, torch.int32, "actions"); _chk(index, torch.int32, "index")
+    if dlogits is None:
+        dlogits = torch.empty_like(logits)
+    if dvalues is None:
+        dvalues = torch.empty(rows, dtype=torch.float32, device=dev)
+    if stats is None:
+        stats = torch.empty(8, dtype=torch.float32, device=dev)
+    if normalize and adv_sums is None:
+        adv_sums = adv_stats(advantages, index, rows)
+    check(lib.tmla_a2c_loss(ptr(logits), ptr(values), ptr(actions), ptr(advantages), ptr(returns), ptr(index), int(rows),
+                            int(global_rows or rows), int(n_actions), ptr(adv_sums), 1 if normalize else 0, float(ent_coef),
+                            float(vf_coef), ptr(dlogits), ptr(dvalues), ptr(stats), _s()))
+    return dlogits, dvalues, stats
+
+
 def ppo_minibatch_supported(obs_dim: int, n_actions: int) -> bool:
     return bool(lib.tmla_ppo_minibatch_supported(obs_dim, HIDDEN, n_actions))
 
@@ -191,6 +213,34 @@ def ppo_minibatch(params, wpack, obs, obs_dim, n_actions, actions, advantages, o
     return grads, stats
 
 
+def a2c_batch(params, wpack, obs, obs_dim, n_actions, actions, advantages, returns, *, index=None, rows=None, global_rows=None,
+              adv_sums=None, normalize=False, ent_coef=0.0, vf_coef=0.5, grads=None, scratch=None, stats=None, logits=None,
+              values=None, grads_zeroed=False, accumulate_stats=False):
+    """One A2C.train step's forward + loss + backward over the whole rollout, fused (tmla_a2c_batch_bf16): returns (grads, stats).
+    Flags as ppo_minibatch."""
+    _chk(params, torch.float32, "params"); _chk(wpack, torch.bfloat16, "wpack"); _chk(obs, torch.float32, "obs")
+    _chk(index, torch.int32, "index"); _chk(actions, torch.int32, "actions"); _chk(advantages, torch.float32, "advantages")
+    _chk(returns, torch.float32, "returns")
+    if rows is None:
+        rows = index.numel() if index is not None else obs.shape[0]
+    dev = params.device
+    if grads is None:
+        grads = torch.empty_like(params)
+    if scratch is None:
+        scratch = torch.empty(lib.tmla_ppo_minibatch_scratch(HIDDEN, rows), dtype=torch.bfloat16, device=dev)
+    if stats is None:
+        stats = torch.empty(8, dtype=torch.float32, device=dev)
+    _chk(scratch, torch.bfloat16, "scratch"); _chk(grads, torch.float32, "grads"); _chk(stats, torch.float32, "stats")
+    _chk(logits, torch.float32, "logits"); _chk(values, torch.float32, "values")
+    if normalize and adv_sums is None:
+        adv_sums = adv_stats(advantages, index, rows)
+    check(lib.tmla_a2c_batch_bf16(ptr(params), ptr(wpack), obs_dim, HIDDEN, n_actions, ptr(obs), ptr(index), int(rows),
+                                  int(global_rows or rows), ptr(actions), ptr(advantages), ptr(returns), ptr(adv_sums),
+                                  1 if normalize else 0, float(ent_coef), float(vf_coef), ptr(grads), ptr(scratch), ptr(stats),
+                                  ptr(logits), ptr(values), (1 if grads_zeroed else 0) | (2 if accumulate_stats else 0), _s()))
+    return grads, stats
+
+
 def adam_clip(params, grads, m, v, step, *, grad_scale=1.0, max_grad_norm=0.5, lr=3e-4, beta1=0.9, beta2=0.999,
               eps=1e-5, norm_out=None, zero_grads=False, wpack=None, obs_dim=0, n_actions=0):
     """clip_grad_norm_ + Adam.step.  zero_grads: clear `grads` once consumed.  wpack (+ obs_dim, n_actions): also refresh the bf16
@@ -213,6 +263,30 @@ def adam_clip_allreduce(comm, params, grads, m, v, step, *, grad_scale=1.0, max_
     check(lib.tmla_adam_clip_allreduce(comm.handle, ptr(params), ptr(grads), ptr(m), ptr(v), params.numel(), float(grad_scale),
                                        float(max_grad_norm), float(lr), float(beta1), float(beta2), float(eps), int(step),
                                        ptr(norm_out), 1 if zero_grads else 0, ptr(wpack), int(obs_dim), HIDDEN, int(n_actions), _s()))
+    return norm_out
+
+
+def rmsprop_clip(params, grads, sq_avg, *, grad_scale=1.0, max_grad_norm=0.5, lr=7e-4, alpha=0.99, eps=1e-5, norm_out=None,
+                 zero_grads=False, wpack=None, obs_dim=0, n_actions=0):
+    """clip_grad_norm_ + torch.optim.RMSprop.step in one launch (tmla_rmsprop_clip_fused); flags as adam_clip."""
+    if norm_out is None:
+        norm_out = torch.zeros(132, dtype=torch.float32, device=params.device)
+    _chk(wpack, torch.bfloat16, "wpack"); _chk(grads, torch.float32, "grads"); _chk(sq_avg, torch.float32, "sq_avg")
+    check(lib.tmla_rmsprop_clip_fused(ptr(params), ptr(grads), ptr(sq_avg), params.numel(), float(grad_scale), float(max_grad_norm),
+                                      float(lr), float(alpha), float(eps), ptr(norm_out), 1 if zero_grads else 0, ptr(wpack),
+                                      int(obs_dim), HIDDEN, int(n_actions), _s()))
+    return norm_out
+
+
+def rmsprop_clip_allreduce(comm, params, grads, sq_avg, step, *, grad_scale=1.0, max_grad_norm=0.5, lr=7e-4, alpha=0.99, eps=1e-5,
+                           norm_out=None, zero_grads=False, wpack=None, obs_dim=0, n_actions=0):
+    """grads <- sum over ranks over NVLink peer memory, then rmsprop_clip, in the same launch; `step` = exchange sequence number."""
+    if norm_out is None:
+        norm_out = torch.zeros(132, dtype=torch.float32, device=params.device)
+    _chk(wpack, torch.bfloat16, "wpack"); _chk(grads, torch.float32, "grads"); _chk(sq_avg, torch.float32, "sq_avg")
+    check(lib.tmla_rmsprop_clip_allreduce(comm.handle, ptr(params), ptr(grads), ptr(sq_avg), params.numel(), float(grad_scale),
+                                          float(max_grad_norm), float(lr), float(alpha), float(eps), int(step), ptr(norm_out),
+                                          1 if zero_grads else 0, ptr(wpack), int(obs_dim), HIDDEN, int(n_actions), _s()))
     return norm_out
 
 

@@ -66,6 +66,12 @@ def orthogonal_init(obs_dim: int, n_actions: int, seed: int) -> torch.Tensor:
 
 
 class CudaPPO:
+    algorithm = "ppo"
+    _log_interval = 1                 # learn(): verbose rows every this many iterations
+    _row_every_iteration = True       # learn(): a logger / progress.jsonl row after every iteration (A2C: every log_interval)
+    _HYPER_KEYS = ("learning_rate", "n_steps", "batch_size", "n_epochs", "gamma", "gae_lambda", "clip_range", "ent_coef", "vf_coef",
+                   "max_grad_norm")
+
     def __init__(self, policy: str, env: CudaVecEnv, *, seed: int = 1, learning_rate: float = 3e-4, n_steps: int = 2048,
                  batch_size: int = 64, n_epochs: int = 10, gamma: float = 0.99, gae_lambda: float = 0.95,
                  clip_range: float = 0.2, ent_coef: float = 0.0, vf_coef: float = 0.5, max_grad_norm: float = 0.5,
@@ -93,6 +99,7 @@ class CudaPPO:
         self.device = torch.device("cuda", env.device_index)
         self.num_timesteps = 0
         self.n_updates = 0
+        self._iterations = 0
         self._adam_step = 0
         self._epoch_counter = 0
         self._dist, self.rank, self.world = _dist()
@@ -316,7 +323,7 @@ class CudaPPO:
         var_y = float(self.ret.var())
         ev = float("nan") if var_y == 0 else 1.0 - float((self.ret - self.val).var()) / var_y
         row = {
-            "time/total_timesteps": self.num_timesteps, "time/iterations": len(self.logger_rows) + 1,
+            "time/total_timesteps": self.num_timesteps, "time/iterations": self._iterations,
             "time/time_elapsed": time.time() - t0,
             "time/fps": self.n_steps * self.n_envs * self.world / max(t_roll + t_train, 1e-9),
             "time/rollout_s": t_roll, "time/train_s": t_train,
@@ -331,7 +338,8 @@ class CudaPPO:
         return row
 
     @_on_device
-    def learn(self, total_timesteps: int, callback=None, progress_bar: bool = False, log_interval: int = 1):
+    def learn(self, total_timesteps: int, callback=None, progress_bar: bool = False, log_interval: int | None = None):
+        log_interval = max(1, int(log_interval or self._log_interval))
         t0 = time.time()
         target = self.num_timesteps + int(total_timesteps)
         it = 0
@@ -345,17 +353,19 @@ class CudaPPO:
             n_mb = self.train()
             torch.cuda.synchronize(self.device)
             te = time.time()
-            row = self._log_row(n_mb, tr - ts, te - tr, t0)
-            self.logger_rows.append(row)
             it += 1
-            if self.verbose and self.rank == 0 and it % log_interval == 0:
-                print(json.dumps({k: (round(v, 5) if isinstance(v, float) else v) for k, v in row.items()}), flush=True)
-            if self.tensorboard_log and self.rank == 0:
-                import os
+            self._iterations += 1
+            if self._row_every_iteration or it % log_interval == 0 or self.num_timesteps >= target:
+                row = self._log_row(n_mb, tr - ts, te - tr, t0)
+                self.logger_rows.append(row)
+                if self.verbose and self.rank == 0 and it % log_interval == 0:
+                    print(json.dumps({k: (round(v, 5) if isinstance(v, float) else v) for k, v in row.items()}), flush=True)
+                if self.tensorboard_log and self.rank == 0:
+                    import os
 
-                os.makedirs(self.tensorboard_log, exist_ok=True)
-                with open(os.path.join(self.tensorboard_log, "progress.jsonl"), "a", encoding="utf-8") as f:
-                    f.write(json.dumps(row) + "\n")
+                    os.makedirs(self.tensorboard_log, exist_ok=True)
+                    with open(os.path.join(self.tensorboard_log, "progress.jsonl"), "a", encoding="utf-8") as f:
+                        f.write(json.dumps(row) + "\n")
             if callback is not None:
                 keep = callback(self) if callable(callback) else callback.on_rollout(self)
                 if keep is False:
@@ -437,20 +447,21 @@ class CudaPPO:
             env = CudaVecEnv(task, 1, seed=seed, device=device)
         if (env.obs_dim, env.n_actions) != (z["obs_dim"], z["n_actions"]):
             raise ValueError(f"policy is {z['obs_dim']}->{z['n_actions']} but task '{task}' is {env.obs_dim}->{env.n_actions}")
-        keys = ("learning_rate", "n_steps", "batch_size", "n_epochs", "gamma", "gae_lambda", "clip_range", "ent_coef",
-                "vf_coef", "max_grad_norm")
         hyper = dict(meta.get("hyper", {}))
-        for k in keys:
+        for k in cls._HYPER_KEYS:
             if k not in hyper and isinstance(data.get(k), (int, float)):
                 hyper[k] = data[k]
         model = cls("MlpPolicy", env, seed=seed, _params=z["params"], **hyper)
         model._repack()
-        model.m.copy_(z["adam_m"])
-        model.v.copy_(z["adam_v"])
-        model._adam_step = int(meta.get("adam_step", z["adam_step"]))
+        model._load_optimizer_state(z, meta)
         model.num_timesteps = int(meta.get("num_timesteps", data.get("num_timesteps", 0) or 0))
         model.n_updates = int(meta.get("n_updates", data.get("_n_updates", 0) or 0))
         return model
+
+    def _load_optimizer_state(self, z: dict, meta: dict) -> None:
+        self.m.copy_(z["adam_m"])
+        self.v.copy_(z["adam_v"])
+        self._adam_step = int(meta.get("adam_step", z["adam_step"]))
 
 
 # ---------------------------------------------------------------------------------------- bench / smoke

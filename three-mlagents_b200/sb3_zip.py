@@ -4,7 +4,8 @@ The reference saves `policies/<prefix>_<run_id>.zip` with `model.save` (backend/
 and loads it with `algo_cls.load` (training.py:269).  `write_zip` produces the same archive members SB3 2.9.0
 writes — `data` (JSON), `policy.pth` (state dict with SB3's parameter names), `policy.optimizer.pth` (torch Adam
 state dict), `pytorch_variables.pth`, `_stable_baselines3_version`, `system_info.txt` — plus `tmla.json`, this
-backend's own metadata.  `read_zip` accepts both this backend's zips and zips written by SB3 itself for the
+backend's own metadata.  A2C models (CudaA2C) write the same members with A2C's `data` attributes and a torch RMSprop state dict.
+`read_zip` accepts both this backend's zips and zips written by SB3 itself for the
 same architecture (MlpPolicy, net_arch dict(pi=[256,256], vf=[256,256])), so SB3-trained policies can be
 evaluated on the CUDA backend.
 
@@ -82,6 +83,18 @@ def adam_state_dict(m, v, step: int, hyper: dict, obs_dim: int, n_actions: int) 
     return {"state": state, "param_groups": [group]}
 
 
+def rmsprop_state_dict(sq_avg, step: int, hyper: dict, obs_dim: int, n_actions: int) -> dict:
+    """torch.optim.RMSprop(alpha=0.99, eps=rms_prop_eps, weight_decay=0).state_dict() for the 12 parameter tensors, produced by a
+    real RMSprop instance so that the layout (state keys, param_group entries) is torch's own."""
+    sq = flat_to_state_dict(sq_avg, obs_dim, n_actions)
+    params = [torch.nn.Parameter(torch.zeros(shape)) for _, shape in param_layout(obs_dim, n_actions)]
+    opt = torch.optim.RMSprop(params, lr=hyper["learning_rate"], alpha=0.99, eps=hyper["rms_prop_eps"], weight_decay=0)
+    if step > 0:
+        for p, name in zip(params, sq):
+            opt.state[p] = {"step": torch.tensor(float(step)), "square_avg": sq[name]}
+    return opt.state_dict()
+
+
 # ---- best-effort `data` entries that SB3 stores as base64 cloudpickle -------------------------------------------
 _created_stubs: list[str] = []
 
@@ -150,7 +163,7 @@ def _build_data(model) -> dict:
     pc["__module__"] = "stable_baselines3.common.policies"
     rb = _serialized(buf_cls, "<class 'abc.ABCMeta'>")
     rb["__module__"] = "stable_baselines3.common.buffers"
-    return {
+    data = {
         "policy_class": pc, "verbose": model.verbose, "policy_kwargs": {"net_arch": {"pi": [256, 256], "vf": [256, 256]}},
         "num_timesteps": model.num_timesteps, "_total_timesteps": model.num_timesteps, "_num_timesteps_at_start": 0,
         "seed": model.seed, "action_noise": None, "start_time": 0, "learning_rate": model.lr,
@@ -160,9 +173,18 @@ def _build_data(model) -> dict:
         "observation_space": obs_e, "action_space": act_e, "n_envs": model.n_envs, "n_steps": model.n_steps,
         "gamma": model.gamma, "gae_lambda": model.gae_lambda, "ent_coef": model.ent_coef, "vf_coef": model.vf_coef,
         "max_grad_norm": model.max_grad_norm, "rollout_buffer_class": rb, "rollout_buffer_kwargs": {},
-        "batch_size": model.batch_size, "n_epochs": model.n_epochs, "clip_range": model.clip_range,
-        "clip_range_vf": None, "normalize_advantage": model.normalize_advantage, "target_kl": None,
     }
+    if getattr(model, "algorithm", "ppo") == "a2c":      # A2C.__init__: use_rms_prop puts RMSprop and its kwargs into policy_kwargs
+        kwargs = {"net_arch": {"pi": [256, 256], "vf": [256, 256]}, "optimizer_class": torch.optim.RMSprop,
+                  "optimizer_kwargs": {"alpha": 0.99, "eps": model.rms_prop_eps, "weight_decay": 0}}
+        pk = _serialized(kwargs, "<class 'dict'>")
+        pk.update(net_arch=kwargs["net_arch"], optimizer_class=str(torch.optim.RMSprop), optimizer_kwargs=kwargs["optimizer_kwargs"])
+        data.update(policy_kwargs=pk, normalize_advantage=model.normalize_advantage, rms_prop_eps=model.rms_prop_eps,
+                    use_rms_prop=True)
+    else:
+        data.update(batch_size=model.batch_size, n_epochs=model.n_epochs, clip_range=model.clip_range, clip_range_vf=None,
+                    normalize_advantage=model.normalize_advantage, target_kl=None)
+    return data
 
 
 def _torch_bytes(obj) -> bytes:
@@ -172,17 +194,27 @@ def _torch_bytes(obj) -> bytes:
 
 
 def write_zip(path: str, model) -> None:
-    hyper = {"learning_rate": model.lr, "n_steps": model.n_steps, "batch_size": model.batch_size, "n_epochs": model.n_epochs,
-             "gamma": model.gamma, "gae_lambda": model.gae_lambda, "clip_range": model.clip_range, "ent_coef": model.ent_coef,
-             "vf_coef": model.vf_coef, "max_grad_norm": model.max_grad_norm}
-    meta = {"format": "three-mlagents_b200/2", "algorithm": "ppo", "task_id": model.env.task_id, "obs_dim": model.obs_dim,
+    a2c = getattr(model, "algorithm", "ppo") == "a2c"
+    if a2c:
+        hyper = {"learning_rate": model.lr, "n_steps": model.n_steps, "gamma": model.gamma, "gae_lambda": model.gae_lambda,
+                 "ent_coef": model.ent_coef, "vf_coef": model.vf_coef, "max_grad_norm": model.max_grad_norm,
+                 "rms_prop_eps": model.rms_prop_eps, "normalize_advantage": model.normalize_advantage}
+    else:
+        hyper = {"learning_rate": model.lr, "n_steps": model.n_steps, "batch_size": model.batch_size, "n_epochs": model.n_epochs,
+                 "gamma": model.gamma, "gae_lambda": model.gae_lambda, "clip_range": model.clip_range, "ent_coef": model.ent_coef,
+                 "vf_coef": model.vf_coef, "max_grad_norm": model.max_grad_norm}
+    meta = {"format": "three-mlagents_b200/2", "algorithm": "a2c" if a2c else "ppo", "task_id": model.env.task_id, "obs_dim": model.obs_dim,
             "n_actions": model.n_actions, "net_arch": {"pi": [256, 256], "vf": [256, 256]}, "seed": model.seed,
-            "num_timesteps": model.num_timesteps, "n_updates": model.n_updates, "adam_step": model._adam_step,
-            "mlp_impl": model.mlp_impl, "hyper": hyper}
+            "num_timesteps": model.num_timesteps, "n_updates": model.n_updates,
+            **({"opt_step": model._opt_step} if a2c else {"adam_step": model._adam_step}), "mlp_impl": model.mlp_impl, "hyper": hyper}
+    if a2c:
+        opt_sd = rmsprop_state_dict(model.sq_avg, model._opt_step, hyper, model.obs_dim, model.n_actions)
+    else:
+        opt_sd = adam_state_dict(model.m, model.v, model._adam_step, hyper, model.obs_dim, model.n_actions)
     with zipfile.ZipFile(path, "w") as z:
         z.writestr("data", json.dumps(build_data(model), indent=4))
         z.writestr("policy.pth", _torch_bytes(flat_to_state_dict(model.params, model.obs_dim, model.n_actions)))
-        z.writestr("policy.optimizer.pth", _torch_bytes(adam_state_dict(model.m, model.v, model._adam_step, hyper, model.obs_dim, model.n_actions)))
+        z.writestr("policy.optimizer.pth", _torch_bytes(opt_sd))
         z.writestr("pytorch_variables.pth", _torch_bytes({}))
         z.writestr("_stable_baselines3_version", SB3_VERSION)
         z.writestr("system_info.txt", f"- three-mlagents_b200 CUDA backend (libtmla), torch {torch.__version__}\n")
@@ -190,7 +222,9 @@ def write_zip(path: str, model) -> None:
 
 
 def read_zip(path: str) -> dict:
-    """-> {params, adam_m, adam_v, adam_step, meta (or None), data} for a zip written by this backend or by SB3."""
+    """-> {params, adam_m, adam_v, adam_step, sq_avg, opt_step, optimizer, meta (or None), data} for a zip written by this backend
+    or by SB3.  optimizer: "adam" (exp_avg / exp_avg_sq: PPO), "rmsprop" (square_avg: A2C) or None (no optimizer state);
+    sq_avg / opt_step are RMSprop's state (None / 0 for Adam)."""
     with zipfile.ZipFile(path) as z:
         names = set(z.namelist())
         if "policy.pth" not in names:
@@ -202,17 +236,49 @@ def read_zip(path: str) -> dict:
         n_actions = int(sd["action_net.weight"].shape[0])
         flat = state_dict_to_flat(sd, obs_dim, n_actions)
         m, v, step = torch.zeros_like(flat), torch.zeros_like(flat), 0
+        sq, opt_step, kind = None, 0, None
         if "policy.optimizer.pth" in names:
             opt = torch.load(io.BytesIO(z.read("policy.optimizer.pth")), map_location="cpu", weights_only=True)
             st = opt.get("state", {})
+            kind = _optimizer_kind(opt)
             if len(st) == 12:
                 layout = param_layout(obs_dim, n_actions)
-                m = torch.cat([torch.as_tensor(st[i]["exp_avg"]).float().reshape(-1) for i in range(12)])
-                v = torch.cat([torch.as_tensor(st[i]["exp_avg_sq"]).float().reshape(-1) for i in range(12)])
-                step = int(float(st[0]["step"]))
-                assert m.numel() == sum(int(np.prod(s)) for _, s in layout)
-    return {"params": flat, "adam_m": m, "adam_v": v, "adam_step": step, "meta": meta, "data": data,
-            "obs_dim": obs_dim, "n_actions": n_actions}
+                cat = lambda key: torch.cat([torch.as_tensor(st[i][key]).float().reshape(-1) for i in range(12)])
+                if kind == "rmsprop":
+                    sq, opt_step = cat("square_avg"), int(float(st[0]["step"]))
+                    assert sq.numel() == flat.numel()
+                else:
+                    m, v = cat("exp_avg"), cat("exp_avg_sq")
+                    step = int(float(st[0]["step"]))
+                    assert m.numel() == sum(int(np.prod(s)) for _, s in layout)
+    return {"params": flat, "adam_m": m, "adam_v": v, "adam_step": step, "sq_avg": sq, "opt_step": opt_step, "optimizer": kind,
+            "meta": meta, "data": data, "obs_dim": obs_dim, "n_actions": n_actions}
+
+
+def _optimizer_kind(opt_state_dict: dict) -> str | None:
+    st = opt_state_dict.get("state", {})
+    keys = set(next(iter(st.values()))) if st else set()
+    if "square_avg" in keys:
+        return "rmsprop"
+    if "exp_avg" in keys:
+        return "adam"
+    group = (opt_state_dict.get("param_groups") or [{}])[0]          # no state yet (never stepped): RMSprop groups carry alpha
+    return "rmsprop" if "alpha" in group else ("adam" if "betas" in group else None)
+
+
+def zip_algorithm(path: str) -> str | None:
+    """The algorithm a policy zip was trained with: tmla.json's `algorithm`, else (SB3-written zips) the optimizer state's kind
+    (square_avg: A2C's RMSprop, exp_avg: PPO's Adam), else None."""
+    with zipfile.ZipFile(path) as z:
+        names = set(z.namelist())
+        if "tmla.json" in names:
+            algo = json.loads(z.read("tmla.json")).get("algorithm")
+            if algo:
+                return str(algo).lower()
+        if "policy.optimizer.pth" in names:
+            opt = torch.load(io.BytesIO(z.read("policy.optimizer.pth")), map_location="cpu", weights_only=True)
+            return {"rmsprop": "a2c", "adam": "ppo"}.get(_optimizer_kind(opt))
+    return None
 
 
 TASK_BY_SHAPE = {(21, 3): "basic", (6, 5): "ball3d", (4, 4): "walljump", (45, 3): "brickbreak", (7, 3): "bicycle", (16, 5): "glider"}      # (4,5) is ambiguous (gridworld / push): needs the task id

@@ -5,10 +5,11 @@
 
     DummyVecEnv[Monitor[env]]  ->  CudaVecEnv           (one kernel launch per vec-step)
     stable_baselines3.PPO      ->  CudaPPO              (rollout, GAE, update in libtmla.so)
+    stable_baselines3.A2C      ->  CudaA2C              (the same rollout; one RMSprop step per rollout)
     EvalCallback/evaluate_policy -> CudaPPO.evaluate    (batched deterministic episodes on the device)
 
-Only PPO is on the hot path named by BASELINE.json; asking for dqn/a2c/sac/td3 raises the same
-ValueError the reference raises for an unsupported algorithm (training.py:110-114).
+PPO and A2C have CUDA backends; asking for dqn/sac/td3 raises the same ValueError the reference raises
+for an unsupported algorithm (training.py:110-114).
 """
 from __future__ import annotations
 
@@ -23,6 +24,7 @@ from typing import Any
 
 import numpy as np
 
+from .a2c import CudaA2C
 from .ppo import CudaPPO
 from .registry import TaskSpec, get_task, make_env
 from .vec_env import CudaVecEnv
@@ -30,7 +32,7 @@ from .vec_env import CudaVecEnv
 POLICIES_DIR = Path("policies")
 RUNS_DIR = Path("runs")
 
-ALGORITHMS: dict[str, type] = {"ppo": CudaPPO}
+ALGORITHMS: dict[str, type] = {"ppo": CudaPPO, "a2c": CudaA2C}
 _REFERENCE_ALGORITHMS = ("a2c", "dqn", "ppo", "sac", "td3")      # training.py:31-37
 
 
@@ -88,11 +90,19 @@ def _default_policy(task: TaskSpec) -> str:          # training.py:326-327
 
 def _default_model_kwargs(algorithm_name: str, *, train_env, task: TaskSpec, total_timesteps: int, tensorboard_log: str,
                           verbose: int) -> dict[str, Any]:
-    """PPO branch of training.py:361-391 (hyper-parameters verbatim)."""
-    if algorithm_name != "ppo":
-        raise ValueError(f"Algorithm '{algorithm_name}' has no CUDA backend; use 'ppo'.")
+    """PPO branch of training.py:361-391 (hyper-parameters verbatim).  a2c: SB3 2.9.0 A2C.__init__'s defaults with the PPO
+    branch's net_arch (the reference's own a2c branch is not transcribed here; DESIGN.md §8)."""
+    if algorithm_name not in ALGORITHMS:
+        raise ValueError(f"Algorithm '{algorithm_name}' has no CUDA backend; use one of {sorted(ALGORITHMS)}.")
     if task.observation == "image":
         raise ValueError(f"Task '{task.id}' needs task-specific CNN policy settings.")
+    if algorithm_name == "a2c":
+        return {
+            "tensorboard_log": tensorboard_log, "verbose": verbose,
+            "learning_rate": 7e-4, "n_steps": 5, "gamma": 0.99, "gae_lambda": 1.0, "ent_coef": 0.0, "vf_coef": 0.5,
+            "max_grad_norm": 0.5, "rms_prop_eps": 1e-5, "use_rms_prop": True, "normalize_advantage": False,
+            "policy_kwargs": {"net_arch": {"pi": [256, 256], "vf": [256, 256]}},
+        }
     return {
         "tensorboard_log": tensorboard_log, "verbose": verbose,
         "learning_rate": 3e-4,
@@ -220,7 +230,7 @@ def evaluate_model(task_id: str, model_filename_or_path: str, *, episodes: int |
 def load_model(task: TaskSpec, model_filename_or_path: str | None = None):
     """training.py:261-269."""
     model_path = _resolve_model_path(task, model_filename_or_path)
-    algorithm_name = _infer_algorithm_from_metadata(task, model_path) or "ppo"
+    algorithm_name = _infer_algorithm_from_metadata(task, model_path) or _infer_algorithm_from_zip(model_path) or "ppo"
     if algorithm_name not in ALGORITHMS:
         raise ValueError(f"Model '{model_path}' was trained with '{algorithm_name}', which has no CUDA backend.")
     return ALGORITHMS[algorithm_name].load(model_path, task_id=task.id)
@@ -259,6 +269,13 @@ def _resolve_model_path(task: TaskSpec, model_filename_or_path: str | None) -> P
             return candidate
         path = candidate
     raise FileNotFoundError(f"Model not found: {path}")
+
+
+def _infer_algorithm_from_zip(model_path: Path) -> str | None:
+    """The algorithm a policy zip names itself (tmla.json), or, for SB3-written zips, the one its optimizer state implies."""
+    from . import sb3_zip
+
+    return sb3_zip.zip_algorithm(str(model_path))
 
 
 def _infer_algorithm_from_metadata(task: TaskSpec, model_path: Path) -> str | None:       # training.py:308-323
