@@ -5,7 +5,7 @@
 // (envs.cuh).  One thread per environment; state lives in packed structure-of-arrays planes in HBM
 // (128-bit loads/stores for ball3d, one 64-bit word per env for the integer tasks) and is kept in
 // registers for all T steps by the fused rollout kernel.  Observation rows are staged through shared
-// memory and leave the SM as coalesced 128-bit stores.
+// memory and leave the SM as coalesced 128-bit stores (ball3d's fused rollout: straight from each lane).
 //
 // These kernels are HBM-bound integer/byte/float32 work: no tensor cores, no GEMM reshaping.
 #include <stdarg.h>
@@ -219,7 +219,7 @@ step_kernel(EnvPtrs p, int64_t n, uint64_t seed, uint64_t env_base, uint64_t ste
 
 // --------------------------------------------------------------- fused T-step random-policy rollout
 // State stays in registers for all T steps; per step and env the kernel writes obs (D floats, via the
-// double-buffered shared-memory stage -> st.global.cs.v4), action, reward and done: the [T,N] rollout
+// double-buffered shared-memory stage -> st.global.cs.v4; ball3d: st.global.cs.v2 per lane), action, reward and done: the [T,N] rollout
 // buffer is write-once streaming traffic, 33 B/env-step for ball3d (SURVEY.md §8(d)).
 // One warp per CTA: 65 536 envs -> 2048 CTAs = 13.8 per SM (tail imbalance < 2 %); the obs stage is
 // private to the warp, so __syncwarp() replaces the CTA barrier (measured 78.6 -> 73.1 us vs 64-thread CTAs).
@@ -321,18 +321,18 @@ static constexpr int kSpareEvery = TMLA_SPARE_EVERY;
 #define TMLA_ROLLOUT_UNROLL 2
 #endif
 static constexpr int kRollUnroll = TMLA_ROLLOUT_UNROLL;
-// tasks that split a step into an independent "plan" half (Task::Tilt, Task::plan, Task::advance_planned — ball3d) run the
-// fused rollout software-pipelined: the plan of step t+1 is computed beside the integration / reward chain of step t
-template <class T, class = void> struct is_pipelined { static constexpr bool value = false; };
-template <class T> struct is_pipelined<T, std::void_t<typename T::Tilt>> { static constexpr bool value = true; };
 static_assert((kSpareEvery & (kSpareEvery - 1)) == 0, "power of two");
-template <class Task, bool PIPE_ON = false>
+template <class Task>
 __global__ void __launch_bounds__(kRollBlock)
 rollout_fast_kernel(EnvPtrs p, uint32_t n, uint64_t seed, uint64_t env_base, uint64_t step0, int T,
                     float4 *__restrict__ obs4, int32_t *__restrict__ act_buf, float *__restrict__ rew_buf,
                     uint8_t *__restrict__ done_buf) {
     constexpr int D = Task::D, BLOCK = kRollBlock, NVEC = BLOCK * D / 4;
-    constexpr bool STAGED = (D != 4);
+    // ball3d (D = 6): each lane writes its own 24-byte row as three streaming 64-bit stores.  Measured on B200: 57.4 against
+    // 61.5 us per launch when the rows go through the shared-memory stage and leave as 128-bit stores (the __syncwarp and the
+    // LDS round trip sit in every step).  The other tasks keep the stage (not measured).
+    constexpr bool DIRECT = (D == 6);
+    constexpr bool STAGED = (D != 4) && !DIRECT;
     static_assert((BLOCK * D) % 4 == 0, "block rows must be whole float4s");
     __shared__ __align__(16) float s_stage[STAGED ? 2 * BLOCK * D : 4];
     const uint32_t tid = threadIdx.x, i = blockIdx.x * BLOCK + tid;
@@ -347,12 +347,6 @@ rollout_fast_kernel(EnvPtrs p, uint32_t n, uint64_t seed, uint64_t env_base, uin
     uint32_t sb = 0;                                    // stage buffer toggle: 0 / BLOCK*D
     [[maybe_unused]] typename Task::Spare sp;
     [[maybe_unused]] bool have_spare = false;
-    constexpr bool PIPE = PIPE_ON && is_pipelined<Task>::value;
-    [[maybe_unused]] int a_next = 0;
-    [[maybe_unused]] auto tilt = [&] {
-        if constexpr (PIPE) { a_next = as.next(seed, env_id, step0, 0u, Task::A); return Task::template plan<true>(cst, s, a_next); }
-        else return 0;
-    }();
 #pragma unroll kRollUnroll   // round 1: 73.2 us (no unroll) / 70.8 us (2) / 72.1 us (4); end of round 2: 63.6 (1) / 61.5-61.8 (2) / 64.2 (3) / 61.6-62.5 (4)
     for (int t = 0; t < T; ++t) {
         if constexpr (Task::HAS_SPARE) {
@@ -372,24 +366,16 @@ rollout_fast_kernel(EnvPtrs p, uint32_t n, uint64_t seed, uint64_t env_base, uin
 #pragma unroll
                 for (int j = 0; j < D; ++j) s_stage[sb + tid * D + j] = o[j];
             }
+        } else if constexpr (DIRECT) {
+            float2 *d2 = reinterpret_cast<float2 *>(reinterpret_cast<float *>(obs4) + (size_t)off * D);
+#pragma unroll
+            for (int j = 0; j < D / 2; ++j) __stcs(d2 + j, make_float2(o[2 * j], o[2 * j + 1]));
         } else {
             st_stream_f4(obs4 + off, make_float4(o[0], o[1], o[2], o[3]));
         }
-        int a;
+        const int a = as.next(seed, env_id, step0, (uint32_t)t, Task::A);
         float r; bool term, trunc;
-        if constexpr (PIPE) {
-            // step t: apply the tilt planned one iteration ago, integrate; meanwhile plan step t+1 from the rotation just applied
-            // (steps >= 1 here, so the after-reset float32 round trip cannot apply; a reset below re-plans with it)
-            a = a_next;
-            typename Task::Pending pend;
-            Task::advance_planned(cst, s, tilt, pend, term, trunc);
-            a_next = as.next(seed, env_id, step0, (uint32_t)t + 1u, Task::A);      // (one action past the end on the last step: unused)
-            tilt = Task::template plan<false>(cst, s, a_next);
-            r = Task::finish(pend);
-        } else {
-            a = as.next(seed, env_id, step0, (uint32_t)t, Task::A);
-            Task::step(cst, s, a, r, term, trunc);
-        }
+        Task::step(cst, s, a, r, term, trunc);
         s.ep_ret = __fadd_rn(s.ep_ret, r);
         const bool d = term || trunc;
         __stcs(act_buf + off, a);
@@ -404,7 +390,6 @@ rollout_fast_kernel(EnvPtrs p, uint32_t n, uint64_t seed, uint64_t env_base, uin
             } else {
                 Task::reset(s, seed, env_id, step0 + (uint64_t)t + 1, TMLA_TAG_RESET);
             }
-            if constexpr (PIPE) tilt = Task::template plan<true>(cst, s, a_next);  // new episode: plan again from its rotation
         }
         if constexpr (STAGED) {
             if constexpr (BLOCK == 32) __syncwarp(); else __syncthreads();   // one warp per CTA: no CTA barrier needed
@@ -420,109 +405,6 @@ rollout_fast_kernel(EnvPtrs p, uint32_t n, uint64_t seed, uint64_t env_base, uin
         off += n;
     }
     Task::store(p.buf, i, s);
-}
-
-// Two (EPT) environments per thread: the same arithmetic as rollout_fast_kernel, with the per-environment code written once
-// and unrolled over EPT independent states — the compiler interleaves the two dependency chains statically (ILP), at half as
-// many warps.  A/B switch TMLA_ROLLOUT_EPT=2.  Measured on B200 (bit-identical, 124 registers, no spills): 96.3 us per launch
-// against 63.6 us — a warp with two chains issues every 4.8 cycles instead of every 6.3, but there are half as many warps
-// (1.7 per scheduler): this kernel lives on thread-level parallelism, which 65 536 environments cap at 13.8 warps per SM.
-template <class Task, int EPT>
-__global__ void __launch_bounds__(kRollBlock)
-rollout_fast_ept_kernel(EnvPtrs p, uint32_t n, uint64_t seed, uint64_t env_base, uint64_t step0, int T,
-                        float4 *__restrict__ obs4, int32_t *__restrict__ act_buf, float *__restrict__ rew_buf,
-                        uint8_t *__restrict__ done_buf) {
-    constexpr int D = Task::D, BLOCK = kRollBlock, NVEC = BLOCK * D / 4;
-    constexpr bool STAGED = (D != 4);
-    __shared__ __align__(16) float s_stage[STAGED ? 2 * EPT * BLOCK * D : 4];
-    const uint32_t tid = threadIdx.x;
-    const typename Task::Consts cst = Task::load_consts();
-    typename Task::State s[EPT];
-    TmlaActionStream as[EPT];
-    uint32_t off[EPT], voff[EPT];
-    uint64_t env_id[EPT];
-    [[maybe_unused]] typename Task::Spare sp[EPT];
-    [[maybe_unused]] bool have_spare[EPT];
-#pragma unroll
-    for (int e = 0; e < EPT; ++e) {
-        const uint32_t i = (blockIdx.x * EPT + e) * BLOCK + tid;
-        env_id[e] = env_base + (uint64_t)i;
-        s[e] = Task::load(p.buf, i);
-        as[e].seek(seed, env_id[e], step0, Task::A);
-        off[e] = i;
-        voff[e] = (blockIdx.x * EPT + e) * NVEC + tid;
-        have_spare[e] = false;
-    }
-    const uint32_t rowvec = n / 4 * D;
-    uint32_t sb = 0;
-#pragma unroll 1
-    for (int t = 0; t < T; ++t) {
-#pragma unroll
-        for (int e = 0; e < EPT; ++e) {
-            if constexpr (Task::HAS_SPARE) {
-                if ((t & (kSpareEvery - 1)) == 0 && !have_spare[e]) {
-                    sp[e] = Task::draw(seed, env_id[e], Task::next_episode(s[e]), TMLA_TAG_RESET);
-                    have_spare[e] = true;
-                }
-            }
-            float o[D];
-            Task::observe(s[e], o);
-            if constexpr (STAGED) {
-                float *st = s_stage + sb + e * BLOCK * D + tid * D;
-                if constexpr (D % 2 == 0) {
-#pragma unroll
-                    for (int j = 0; j < D / 2; ++j) reinterpret_cast<float2 *>(st)[j] = make_float2(o[2 * j], o[2 * j + 1]);
-                } else {
-#pragma unroll
-                    for (int j = 0; j < D; ++j) st[j] = o[j];
-                }
-            } else {
-                st_stream_f4(obs4 + off[e], make_float4(o[0], o[1], o[2], o[3]));
-            }
-        }
-        int a[EPT]; float r[EPT]; bool d[EPT];
-#pragma unroll
-        for (int e = 0; e < EPT; ++e) {
-            a[e] = as[e].next(seed, env_id[e], step0, (uint32_t)t, Task::A);
-            bool term, trunc;
-            Task::step(cst, s[e], a[e], r[e], term, trunc);
-            s[e].ep_ret = __fadd_rn(s[e].ep_ret, r[e]);
-            d[e] = term || trunc;
-        }
-#pragma unroll
-        for (int e = 0; e < EPT; ++e) {
-            __stcs(act_buf + off[e], a[e]);
-            __stcs(rew_buf + off[e], r[e]);
-            __stcs(done_buf + off[e], (uint8_t)(d[e] ? 1 : 0));
-            if (d[e]) {
-                if constexpr (Task::HAS_SPARE) {
-                    const uint32_t ep = Task::next_episode(s[e]);
-                    if (!have_spare[e]) sp[e] = Task::draw(seed, env_id[e], ep, TMLA_TAG_RESET);
-                    Task::begin_episode(s[e], sp[e], ep);
-                    have_spare[e] = false;
-                } else {
-                    Task::reset(s[e], seed, env_id[e], step0 + (uint64_t)t + 1, TMLA_TAG_RESET);
-                }
-            }
-            off[e] += n;
-        }
-        if constexpr (STAGED) {
-            __syncwarp();
-#pragma unroll
-            for (int e = 0; e < EPT; ++e) {
-                const float4 *s4 = reinterpret_cast<const float4 *>(s_stage + sb + e * BLOCK * D);
-#pragma unroll
-                for (int v = 0; v < (NVEC + BLOCK - 1) / BLOCK; ++v) {
-                    const int q = v * BLOCK + tid;
-                    if ((v + 1) * BLOCK <= NVEC || q < NVEC) st_stream_f4(obs4 + voff[e] + v * BLOCK, s4[q]);
-                }
-                voff[e] += rowvec;
-            }
-            sb ^= EPT * BLOCK * D;
-        }
-    }
-#pragma unroll
-    for (int e = 0; e < EPT; ++e) Task::store(p.buf, (blockIdx.x * EPT + e) * BLOCK + tid, s[e]);
 }
 
 // ------------------------------------------------------------- policy-driven step (PPO rollout row)
@@ -1310,20 +1192,7 @@ int tmla_rollout_random(tmla_env *h, int T, float *obs_buf, int32_t *act_buf, fl
     const bool fast = obs_buf && act_buf && rew_buf && done_buf && (h->n % kRollBlock == 0) &&
                       ((reinterpret_cast<uintptr_t>(obs_buf) & 15u) == 0) && ((int64_t)T * h->n * D / 4 < ((int64_t)1 << 31));
     const unsigned grid = (unsigned)ceil_div64(h->n, kRollBlock);
-    // TMLA_ROLLOUT_PIPE=1: the software-pipelined ball3d loop (plan of step t+1 beside the integration chain of step t).  Measured
-    // on B200 (profiles/r2_rollout_fast_ncu.txt): 63.52 vs 63.54 us per launch — fixed-latency wait stalls drop 38.6 -> 33.0 %
-    // of the samples and issue slots rise 58.7 -> 62.9 %, but the re-plan inside the reset branch costs 4.8 % more
-    // instructions; the plain loop stays the default.
-    static const bool pipe = [] { const char *e = getenv("TMLA_ROLLOUT_PIPE"); return e && !strcmp(e, "1"); }();
-    static const int ept = [] { const char *e = getenv("TMLA_ROLLOUT_EPT"); return e ? atoi(e) : 1; }();     // A/B: environments per thread
-    if (fast && ept == 2 && h->task == TMLA_BALL3D && h->n % (2 * kRollBlock) == 0) {
-        rollout_fast_ept_kernel<Ball3DTask, 2><<<grid / 2, kRollBlock, 0, (cudaStream_t)stream>>>(
-            ptrs_of(h), (uint32_t)h->n, h->seed, h->env_id_base, h->step_count, T, reinterpret_cast<float4 *>(obs_buf), act_buf, rew_buf, done_buf);
-    } else
-    if (fast && pipe && h->task == TMLA_BALL3D) {
-        rollout_fast_kernel<Ball3DTask, true><<<grid, kRollBlock, 0, (cudaStream_t)stream>>>(
-            ptrs_of(h), (uint32_t)h->n, h->seed, h->env_id_base, h->step_count, T, reinterpret_cast<float4 *>(obs_buf), act_buf, rew_buf, done_buf);
-    } else if (fast) {
+    if (fast) {
         TASK_SWITCH(h->task, (rollout_fast_kernel<TaskT><<<grid, kRollBlock, 0, (cudaStream_t)stream>>>(
                                  ptrs_of(h), (uint32_t)h->n, h->seed, h->env_id_base, h->step_count, T,
                                  reinterpret_cast<float4 *>(obs_buf), act_buf, rew_buf, done_buf)));

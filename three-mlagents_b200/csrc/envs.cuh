@@ -184,11 +184,8 @@ struct Ball3DTask {
     }
     struct Pending { float sq; uint32_t flags; };
     // The tilt half of a step (ball3d.py:76-84): the new rotation of the ONE axis action `a` touches, with the products that
-    // depend on it.  It reads only rx/rz (and, right after a reset, `steps == 0`), never pos/vel — so the fused rollout kernel
-    // computes the tilt of step t+1 while the velocity/position/reward chain of step t is still in flight (two independent
-    // dependency chains per thread instead of one; `PIPELINED`).
+    // depend on it.  It reads only rx/rz (and, right after a reset, `steps == 0`), never pos/vel.
     struct Tilt { double rot, adt; float orot; bool x; };
-    static constexpr bool PIPELINED = true;
     template <bool MAYBE_FIRST>
     static __device__ __forceinline__ Tilt plan(const Consts &c, const State &s, int a) {
         // ACTION_DELTAS (ball3d.py:31-37): 0:+x 1:-x 2:+z 3:-z 4:none, each +-np.deg2rad(3.0).  The sign is
