@@ -305,12 +305,18 @@ rollout_random_kernel(EnvPtrs p, int64_t n, uint64_t seed, uint64_t env_base, ui
     if (active) Task::store(p.buf, i, s);
 }
 
-// Fast path of the fused rollout (what bench.py times): every block full (n % 64 == 0), all four buffers
-// present, 16-byte aligned rows, 32-bit element offsets.  Same arithmetic as the generic kernel above (the
-// tests compare them bit for bit) with the loop bookkeeping stripped down: shared memory is indexed directly
-// (no generic pointers), offsets are running 32-bit counters, and for tasks with an episode-indexed reset
-// stream (ball3d) the next initial state is drawn ahead of time every kSpareEvery steps (`Spare`), so the two Philox
-// blocks of a reset no longer sit inside a divergent branch that ~23 % of the warps enter on every step.
+// Fast path of the fused rollout (what bench.py times): every block full (n % 32 == 0), all four buffers present,
+// 16-byte aligned rows, fewer than 2^31 float4 of observations.  Same arithmetic as the generic kernel above (the tests compare them bit
+// for bit) with the loop bookkeeping stripped down, because at 13.8 one-warp CTAs per SM the launch time follows the
+// instructions each warp issues per step:
+//   - The loop runs over the 16-step blocks of the action stream.  Each block's Philox draw is expanded once into 16
+//     packed 4-bit digits, so a step's action is one shift and one mask, with no per-step branch.  A step0 that is not a
+//     multiple of 16 starts with a partial block.
+//   - For tasks with an episode-indexed reset stream (ball3d) the next initial state is drawn ahead of time (`Spare`) at a
+//     block boundary every kSpareEvery steps, so the two Philox blocks of a reset no longer sit inside a divergent branch
+//     that ~23 % of the warps enter on every step.  A second reset inside one window draws out of line (draw_spare), which
+//     keeps the step loop's code short and contiguous.
+//   - Row pointers are bumped once per step and shared memory is indexed directly (no generic pointers).
 // Refill period of the ahead-of-time reset draws.  The draw is indexed by the env's episode counter, not by time, so the
 // period changes no result — only how often a warp pays two Philox blocks for its consumed lanes (TMLA_SPARE_EVERY).
 #ifndef TMLA_SPARE_EVERY
@@ -321,13 +327,21 @@ static constexpr int kSpareEvery = TMLA_SPARE_EVERY;
 #define TMLA_ROLLOUT_UNROLL 2
 #endif
 static constexpr int kRollUnroll = TMLA_ROLLOUT_UNROLL;
-static_assert((kSpareEvery & (kSpareEvery - 1)) == 0, "power of two");
+static_assert(kSpareEvery % 16 == 0 && ((kSpareEvery / 16) & (kSpareEvery / 16 - 1)) == 0, "a power-of-two number of action blocks");
+static_assert(16 % kRollUnroll == 0, "the unrolled step loop covers whole action blocks");
+
+template <class Task>
+__device__ __noinline__ typename Task::Spare draw_spare(uint64_t seed, uint64_t env_id, uint32_t episode) {
+    return Task::draw(seed, env_id, episode, TMLA_TAG_RESET);
+}
+
 template <class Task>
 __global__ void __launch_bounds__(kRollBlock)
 rollout_fast_kernel(EnvPtrs p, uint32_t n, uint64_t seed, uint64_t env_base, uint64_t step0, int T,
                     float4 *__restrict__ obs4, int32_t *__restrict__ act_buf, float *__restrict__ rew_buf,
                     uint8_t *__restrict__ done_buf) {
     constexpr int D = Task::D, BLOCK = kRollBlock, NVEC = BLOCK * D / 4;
+    static_assert(Task::A <= 16, "actions are packed as 4-bit digits");
     // ball3d (D = 6): each lane writes its own 24-byte row as three streaming 64-bit stores.  Measured on B200: 57.4 against
     // 61.5 us per launch when the rows go through the shared-memory stage and leave as 128-bit stores (the __syncwarp and the
     // LDS round trip sit in every step).  The other tasks keep the stage (not measured).
@@ -339,56 +353,53 @@ rollout_fast_kernel(EnvPtrs p, uint32_t n, uint64_t seed, uint64_t env_base, uin
     const uint64_t env_id = env_base + (uint64_t)i;
     const typename Task::Consts cst = Task::load_consts();
     typename Task::State s = Task::load(p.buf, i);
-    TmlaActionStream as;
-    as.seek(seed, env_id, step0, Task::A);
-    uint32_t off = i;                                   // t*n + i, element offset into the [T,n] planes
-    uint32_t voff = blockIdx.x * NVEC + tid;            // float4 offset of this thread's first vector in row t
-    const uint32_t rowvec = n / 4 * D;                  // float4 per row (n % 64 == 0)
+    // Row pointers of step t, bumped once per step: a 64-bit add each.  A 32-bit element offset scaled into four 64-bit
+    // addresses costs more instructions per step (and so does forcing the bumps into IMAD.WIDE, which ptxas splits).
+    float *orow = reinterpret_cast<float *>(obs4) + (size_t)i * D;                       // this env's obs (unstaged tasks)
+    float4 *vrow = obs4 + blockIdx.x * NVEC + tid;      // this thread's first float4 of the block's rows (staged tasks)
+    int32_t *arow = act_buf + i;
+    float *rrow = rew_buf + i;
+    uint8_t *drow = done_buf + i;
+    const uint32_t rowfloats = n * D;                   // floats per obs row (n % 32 == 0)
     uint32_t sb = 0;                                    // stage buffer toggle: 0 / BLOCK*D
     [[maybe_unused]] typename Task::Spare sp;
     [[maybe_unused]] bool have_spare = false;
-#pragma unroll kRollUnroll   // round 1: 73.2 us (no unroll) / 70.8 us (2) / 72.1 us (4); end of round 2: 63.6 (1) / 61.5-61.8 (2) / 64.2 (3) / 61.6-62.5 (4)
-    for (int t = 0; t < T; ++t) {
-        if constexpr (Task::HAS_SPARE) {
-            if ((t & (kSpareEvery - 1)) == 0 && !have_spare) {   // off the critical path: refill consumed spares
-                sp = Task::draw(seed, env_id, Task::next_episode(s), TMLA_TAG_RESET);
-                have_spare = true;
-            }
-        }
+    // one step with digit j of the current action block; kb: absolute index of the block's first step
+    auto step = [&](uint64_t digits, uint32_t j, uint64_t kb) {
         float o[D];
         Task::observe(s, o);                            // observation the action is taken on
         if constexpr (STAGED) {
             if constexpr (D % 2 == 0) {
                 float2 *s2 = reinterpret_cast<float2 *>(s_stage + sb + tid * D);
 #pragma unroll
-                for (int j = 0; j < D / 2; ++j) s2[j] = make_float2(o[2 * j], o[2 * j + 1]);
+                for (int q = 0; q < D / 2; ++q) s2[q] = make_float2(o[2 * q], o[2 * q + 1]);
             } else {
 #pragma unroll
-                for (int j = 0; j < D; ++j) s_stage[sb + tid * D + j] = o[j];
+                for (int q = 0; q < D; ++q) s_stage[sb + tid * D + q] = o[q];
             }
         } else if constexpr (DIRECT) {
-            float2 *d2 = reinterpret_cast<float2 *>(reinterpret_cast<float *>(obs4) + (size_t)off * D);
+            float2 *d2 = reinterpret_cast<float2 *>(orow);
 #pragma unroll
-            for (int j = 0; j < D / 2; ++j) __stcs(d2 + j, make_float2(o[2 * j], o[2 * j + 1]));
+            for (int q = 0; q < D / 2; ++q) __stcs(d2 + q, make_float2(o[2 * q], o[2 * q + 1]));
         } else {
-            st_stream_f4(obs4 + off, make_float4(o[0], o[1], o[2], o[3]));
+            st_stream_f4(reinterpret_cast<float4 *>(orow), make_float4(o[0], o[1], o[2], o[3]));
         }
-        const int a = as.next(seed, env_id, step0, (uint32_t)t, Task::A);
+        const int a = (int)((uint32_t)(digits >> (4 * j)) & 15u);
         float r; bool term, trunc;
         Task::step(cst, s, a, r, term, trunc);
         s.ep_ret = __fadd_rn(s.ep_ret, r);
         const bool d = term || trunc;
-        __stcs(act_buf + off, a);
-        __stcs(rew_buf + off, r);
-        __stcs(done_buf + off, (uint8_t)(d ? 1 : 0));
+        __stcs(arow, a);
+        __stcs(rrow, r);
+        __stcs(drow, (uint8_t)(d ? 1 : 0));
         if (d) {
             if constexpr (Task::HAS_SPARE) {
                 const uint32_t e = Task::next_episode(s);
-                if (!have_spare) sp = Task::draw(seed, env_id, e, TMLA_TAG_RESET);   // second reset inside one window
+                if (!have_spare) sp = draw_spare<Task>(seed, env_id, e);   // second reset inside one window
                 Task::begin_episode(s, sp, e);
                 have_spare = false;
             } else {
-                Task::reset(s, seed, env_id, step0 + (uint64_t)t + 1, TMLA_TAG_RESET);
+                Task::reset(s, seed, env_id, kb + j + 1, TMLA_TAG_RESET);
             }
         }
         if constexpr (STAGED) {
@@ -397,12 +408,36 @@ rollout_fast_kernel(EnvPtrs p, uint32_t n, uint64_t seed, uint64_t env_base, uin
 #pragma unroll
             for (int v = 0; v < (NVEC + BLOCK - 1) / BLOCK; ++v) {
                 const int e = v * BLOCK + tid;
-                if ((v + 1) * BLOCK <= NVEC || e < NVEC) st_stream_f4(obs4 + voff + v * BLOCK, s4[e]);
+                if ((v + 1) * BLOCK <= NVEC || e < NVEC) st_stream_f4(vrow + v * BLOCK, s4[e]);
             }
             sb ^= BLOCK * D;
-            voff += rowvec;
+            vrow += rowfloats / 4;
+        } else {
+            orow += rowfloats;
         }
-        off += n;
+        arow += n; rrow += n; drow += n;
+    };
+    uint64_t kb = step0 & ~(uint64_t)15;                // first step of the current action block
+    uint32_t j = (uint32_t)step0 & 15u;                 // digit of the next step within it
+    uint32_t left = (uint32_t)T;                        // steps still to run
+    for (uint32_t nb = 0; left != 0; ++nb, kb += 16, j = 0) {
+        const uint64_t digits = TmlaActionStream::block_digits(seed, env_id, kb >> 4, Task::A);
+        if constexpr (Task::HAS_SPARE) {
+            if ((nb & (kSpareEvery / 16 - 1)) == 0 && !have_spare) {   // refill consumed spares
+                sp = Task::draw(seed, env_id, Task::next_episode(s), TMLA_TAG_RESET);
+                have_spare = true;
+            }
+        }
+        if (j == 0 && left >= 16) {
+#pragma unroll kRollUnroll   // round 1: 73.2 us (no unroll) / 70.8 us (2) / 72.1 us (4); end of round 2: 63.6 (1) / 61.5-61.8 (2) / 64.2 (3) / 61.6-62.5 (4)
+            for (uint32_t q = 0; q < 16; ++q) step(digits, q, kb);
+            left -= 16;
+        } else {                                        // partial block: step0 % 16 != 0, or the rollout ends inside it
+            const uint32_t je = min(16u, j + left);
+            left -= je - j;
+#pragma unroll 1
+            for (; j < je; ++j) step(digits, j, kb);
+        }
     }
     Task::store(p.buf, i, s);
 }

@@ -77,4 +77,22 @@ struct TmlaActionStream {
         frac = (uint32_t)p;
         return (int)(p >> 32);
     }
+    // The 16 actions of Philox block `blk` (steps 16*blk .. 16*blk+15), expanded by the same multiply-shift sequence as
+    // next() and packed as 4-bit digits: the action of step 16*blk + j is (digits >> 4*j) & 15.  Needs n_actions <= 16.
+    __device__ __forceinline__ static uint64_t block_digits(uint64_t seed, uint64_t env_id, uint64_t blk, uint32_t n_actions) {
+        const uint4 b = tmla_stream_block(seed, env_id, blk, TMLA_TAG_ACTION, 0);
+        const uint32_t w[4] = {b.x, b.y, b.z, b.w};
+        uint32_t half[2] = {0u, 0u};                      // digits 0-7 | digits 8-15
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            uint32_t frac = w[q];
+#pragma unroll
+            for (int d = 0; d < 4; ++d) {
+                const uint64_t p = (uint64_t)frac * n_actions;
+                frac = (uint32_t)p;
+                half[q >> 1] |= (uint32_t)(p >> 32) << (4 * (4 * (q & 1) + d));
+            }
+        }
+        return ((uint64_t)half[1] << 32) | half[0];
+    }
 };
