@@ -183,6 +183,7 @@ int tmla_step_policy(tmla_env *h, const float *logits, int deterministic, int32_
  * Every pointer is DEVICE memory owned by the caller; the struct has no padding (it is compared bytewise to reuse the graph).
  *   params/wpack/act_cache  as tmla_mlp_forward_bf16 (wpack NULL = fp32 CUDA-core path, act_cache then float); act_cache holds
  *                           4 x max(n, trunc_capacity) x hidden elements, NULL allowed where tmla_mlp_forward_bf16 allows it
+ *                           and, with wpack NULL, for hidden 64 and 128
  *   obs [n_steps+1,n,D]     row 0 = current observations (input), rows 1.. written
  *   actions/log_probs/rewards/values/dones/advantages/returns [n_steps,n];  last_values [n];  logits [n,A] scratch
  *   trunc_count int32[1], trunc_index int32[cap], trunc_obs float[cap,D], trunc_values float[cap]: timeout records
@@ -230,20 +231,24 @@ int tmla_permutation(uint64_t seed, uint64_t epoch, int64_t total, int T, int64_
 /* ---- policy / value network: MlpPolicy with net_arch dict(pi=[H,H], vf=[H,H]), tanh ------------
  * Flat fp32 parameter vector in SB3's policy.parameters() order:
  *   pi.W1[H,D] pi.b1[H] pi.W2[H,H] pi.b2[H] vf.W1[H,D] vf.b1[H] vf.W2[H,H] vf.b2[H] Wa[A,H] ba[A] Wv[1,H] bv[1]
+ * hidden H: 256, 64 or 128 for tmla_mlp_num_params / tmla_mlp_forward / tmla_mlp_backward(_scratch) (64 and 128 run the
+ * float32 kernels of csrc/mlp_small.cu); any other width is TMLA_EINVAL.  The bf16 entry points take 256 only.
  */
 int64_t tmla_mlp_num_params(int obs_dim, int hidden, int n_actions);
 
 /* ActorCriticPolicy.forward / evaluate_actions / predict_values.
  *   x float[rows,D] gathered through `index` (int32[rows], may be NULL = identity);
  *   logits float[rows,A] (NULL: value tower only), values float[rows] (NULL: policy tower only);
- *   act_cache: optional float[4,rows,H] (pi.h1, pi.h2, vf.h1, vf.h2) kept for tmla_mlp_backward;
+ *   act_cache: float[4,rows,H] (pi.h1, pi.h2, vf.h1, vf.h2) kept for tmla_mlp_backward (workspace at H = 256; at H = 64 / 128
+ *   NULL = inference, no activations kept);
  *   rows_dev: optional DEVICE int32 row count overriding `rows` as an upper bound (rows<=capacity). */
 int tmla_mlp_forward(const float *params, int obs_dim, int hidden, int n_actions, const float *x,
                      const int32_t *index, int64_t rows, const int32_t *rows_dev, float *logits,
                      float *values, float *act_cache, void *stream);
 
 /* backward of the above: dlogits float[rows,A], dvalues float[rows] -> grads (flat, same order as
- * params; OVERWRITTEN, not accumulated).  scratch: float[tmla_mlp_backward_scratch(...)] */
+ * params; OVERWRITTEN, not accumulated).  scratch: float[tmla_mlp_backward_scratch(...)] (H = 64 / 128: per-chunk partial
+ * gradients, summed in a fixed order, so two calls on the same inputs give bit-identical gradients) */
 int64_t tmla_mlp_backward_scratch(int obs_dim, int hidden, int n_actions, int64_t rows);
 int tmla_mlp_backward(const float *params, int obs_dim, int hidden, int n_actions, const float *x,
                       const int32_t *index, int64_t rows, const float *act_cache, const float *dlogits,
@@ -251,6 +256,7 @@ int tmla_mlp_backward(const float *params, int obs_dim, int hidden, int n_action
 
 /* bf16 / tensor-core variant of the same network (csrc/mlp_tc.cu): identical semantics, the 256x256 hidden
  * layers run on tcgen05 with bf16 operands and fp32 accumulation, activations (act_cache, scratch) are bf16.
+ * hidden must be 256 (other widths: TMLA_EINVAL with a message naming the float32 entry points).
  *   wpack: bf16[TMLA_WPACK_MATRICES][256][256] = {pi.W2, pi.W2^T, vf.W2, vf.W2^T, pi.W2 image, vf.W2 image} (image = the
  *   shared-memory operand layout the fused minibatch kernel loads with one bulk-TMA copy), refreshed by tmla_mlp_pack_bf16 after every
  *   optimizer step.  act_cache: bf16[4,rows,256] (forward: may be NULL when obs_dim <= 6 = inference only, the
@@ -375,7 +381,8 @@ int tmla_tc_debug(int swap_lbo_sbo);
  *   flags: TMLA_MB_GRADS_ZEROED — the caller guarantees grads is all zeros (tmla_adam_clip_zero left it so): no memset;
  *          TMLA_MB_ACCUMULATE_STATS — stats_out is added to instead of overwritten (a running sum over minibatches).
  * tmla_ppo_minibatch_supported: 1 when the fused path covers (obs_dim, hidden, n_actions) — ball3d, gridworld,
- * push, walljump, bicycle; callers use the three-call sequence otherwise (basic: obs_dim 21, 3 actions). */
+ * push, walljump, bicycle at hidden 256; callers use the three-call sequence otherwise (basic: obs_dim 21, 3 actions; every
+ * shape at hidden 64 / 128, where it returns 0). */
 #define TMLA_MB_GRADS_ZEROED 1
 #define TMLA_MB_ACCUMULATE_STATS 2
 int tmla_ppo_minibatch_supported(int obs_dim, int hidden, int n_actions);

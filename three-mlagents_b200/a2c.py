@@ -6,7 +6,8 @@ data-parallel set-up from CudaPPO.  What differs is A2C.train:
   * ONE gradient step per rollout over all n_steps x n_envs rows (rollout_buffer.get(batch_size=None)); the row order does
     not matter for a single batch, so the buffers are read in place (no permutation);
   * the loss is the plain policy gradient -(adv * log_prob).mean() + ent_coef * entropy_loss + vf_coef * value_loss
-    (tmla_a2c_batch_bf16 fused, tmla_a2c_loss on the three-call path), advantages normalised only on request;
+    (tmla_a2c_batch_bf16 fused, tmla_a2c_loss on the three-call path — the path of net_arch widths 64 and 128, which run the
+    float32 kernels of csrc/mlp_small.cu), advantages normalised only on request;
   * the optimizer is torch.optim.RMSprop(alpha=0.99, eps=rms_prop_eps) after clip_grad_norm_, one launch
     (tmla_rmsprop_clip_fused, or tmla_rmsprop_clip_allreduce with the gradient exchange fused in at world_size > 1).
 """
@@ -76,11 +77,11 @@ class CudaA2C(CudaPPO):
                           scratch=self.scratch_mb, stats=self.stats_acc, grads_zeroed=True, **common)
         else:
             ops.mlp_forward(self.params, obs_flat, D, A, rows=total, logits=self.logits_mb, values=self.values_mb,
-                            act_cache=self.cache_mb, wpack=self.wpack)
+                            act_cache=self.cache_mb, wpack=self.wpack, hidden=self.hidden)
             ops.a2c_loss(self.logits_mb, self.values_mb, self.act, self.adv, self.ret, dlogits=self.dlogits, dvalues=self.dvalues,
                          stats=self.stats_acc, **common)
             ops.mlp_backward(self.params, obs_flat, D, A, self.cache_mb, self.dlogits, self.dvalues, rows=total, grads=self.grads,
-                             scratch=self.scratch_mb, wpack=self.wpack)
+                             scratch=self.scratch_mb, wpack=self.wpack, hidden=self.hidden)
         self._opt_step += 1
         opt = dict(max_grad_norm=self.max_grad_norm, lr=self.lr, alpha=RMSPROP_ALPHA, eps=self.rms_prop_eps, norm_out=self.norm_out,
                    zero_grads=True)

@@ -6,18 +6,18 @@ struct MlpOffsets {
     int64_t w1[2], b1[2], w2[2], b2[2], wh[2], bh[2], total;
     int nout[2];
 };
-static inline MlpOffsets mlp_offsets(int D, int A) {
+static inline MlpOffsets mlp_offsets(int D, int A, int64_t H = 256) {      // H: hidden width (256, or 64 / 128: mlp_small.cu)
     MlpOffsets o;
     int64_t p = 0;
     for (int t = 0; t < 2; ++t) {
-        o.w1[t] = p; p += (int64_t)256 * D;
-        o.b1[t] = p; p += 256;
-        o.w2[t] = p; p += (int64_t)256 * 256;
-        o.b2[t] = p; p += 256;
+        o.w1[t] = p; p += H * D;
+        o.b1[t] = p; p += H;
+        o.w2[t] = p; p += H * H;
+        o.b2[t] = p; p += H;
     }
-    o.wh[0] = p; p += (int64_t)A * 256;
+    o.wh[0] = p; p += (int64_t)A * H;
     o.bh[0] = p; p += A;
-    o.wh[1] = p; p += 256;
+    o.wh[1] = p; p += H;
     o.bh[1] = p; p += 1;
     o.total = p;
     o.nout[0] = A; o.nout[1] = 1;

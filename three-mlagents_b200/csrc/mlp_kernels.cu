@@ -37,6 +37,13 @@ int tc_tower_forward_pipe_dual_launch(int D, int n_actions, const float *const *
 int tc_tower_forward_launch(int D, int nout, const float *W1, const float *B1, const void *W2, const float *B2, const float *Wh,
                             const float *Bh, const float *x, const int32_t *index, int64_t M, const int32_t *rows_dev, float *out,
                             void *h1, void *h2, cudaStream_t st);
+// hidden widths 64 and 128 (mlp_small.cu)
+int small_mlp_forward(const float *params, int D, int hidden, int A, const float *x, const int32_t *index, int64_t rows,
+                      const int32_t *rows_dev, float *logits, float *values, float *act_cache, cudaStream_t st);
+int64_t small_mlp_backward_scratch(int D, int hidden, int A, int64_t rows);
+int small_mlp_backward(const float *params, int D, int hidden, int A, const float *x, const int32_t *index, int64_t rows,
+                       const float *act_cache, const float *dlogits, const float *dvalues, float *grads, float *scratch,
+                       cudaStream_t st);
 
 #include "mlp_common.cuh"
 
@@ -780,13 +787,25 @@ static int mlp_backward_impl(const float *params, const void *wpack, int obs_dim
 
 extern "C" {
 
+static bool small_width(int hidden) { return hidden == 64 || hidden == 128; }
+
 int64_t tmla_mlp_num_params(int obs_dim, int hidden, int n_actions) {
-    if (hidden != H || obs_dim <= 0 || n_actions <= 0) return TMLA_EINVAL;
-    return mlp_offsets(obs_dim, n_actions).total;
+    if (!(hidden == H || small_width(hidden))) { tmla_set_error("hidden must be 64, 128 or 256, got %d", hidden); return TMLA_EINVAL; }
+    if (obs_dim <= 0 || n_actions <= 0) return TMLA_EINVAL;
+    return mlp_offsets(obs_dim, n_actions, hidden).total;
 }
 
-static int check_shape(int D, int hidden, int A) {
-    if (hidden != H) { tmla_set_error("hidden must be 256 (net_arch of training.py:363-365), got %d", hidden); return TMLA_EINVAL; }
+// fp32: the float32 entry points (hidden 64, 128 or 256); otherwise the bf16 tensor-core ones (256 only)
+static int check_shape(int D, int hidden, int A, bool fp32 = false) {
+    if (fp32 && !(hidden == H || small_width(hidden))) {
+        tmla_set_error("hidden must be 64, 128 or 256, got %d", hidden);
+        return TMLA_EINVAL;
+    }
+    if (!fp32 && hidden != H) {
+        tmla_set_error("the bf16 tensor-core path covers hidden = 256 only (got %d); widths 64 and 128 run on tmla_mlp_forward / "
+                       "tmla_mlp_backward in float32", hidden);
+        return TMLA_EINVAL;
+    }
     if (!(D == 4 || D == 6 || D == 7 || D == 16 || D == 21 || D == 45)) { tmla_set_error("obs_dim must be 4, 6, 7, 16, 21 or 45, got %d", D); return TMLA_EINVAL; }
     if (!(A >= 3 && A <= 5)) { tmla_set_error("n_actions must be 3, 4 or 5, got %d", A); return TMLA_EINVAL; }
     return TMLA_OK;
@@ -794,11 +813,14 @@ static int check_shape(int D, int hidden, int A) {
 
 int tmla_mlp_forward(const float *params, int obs_dim, int hidden, int n_actions, const float *x, const int32_t *index,
                      int64_t rows, const int32_t *rows_dev, float *logits, float *values, float *act_cache, void *stream) {
-    TMLA_REQUIRE(params && x && act_cache, "params/x/act_cache must be non-NULL (act_cache is the activation workspace)");
+    TMLA_REQUIRE(params && x, "params/x must be non-NULL");
+    TMLA_REQUIRE(act_cache || small_width(hidden), "act_cache (the activation workspace) may be NULL only for hidden 64 and 128");
     TMLA_REQUIRE(rows > 0, "rows must be positive");
     TMLA_REQUIRE(logits || values, "nothing to compute");
-    int rc = check_shape(obs_dim, hidden, n_actions);
+    int rc = check_shape(obs_dim, hidden, n_actions, true);
     if (rc) return rc;
+    if (hidden != H)
+        return small_mlp_forward(params, obs_dim, hidden, n_actions, x, index, rows, rows_dev, logits, values, act_cache, (cudaStream_t)stream);
     return mlp_forward_impl<float>(params, nullptr, obs_dim, n_actions, x, index, rows, rows_dev, logits, values, act_cache, (cudaStream_t)stream);
 }
 
@@ -816,7 +838,7 @@ int tmla_mlp_forward_bf16(const float *params, const void *wpack, int obs_dim, i
 }
 
 int64_t tmla_mlp_backward_scratch(int obs_dim, int hidden, int n_actions, int64_t rows) {
-    (void)obs_dim; (void)n_actions;
+    if (small_width(hidden)) return small_mlp_backward_scratch(obs_dim, hidden, n_actions, rows);    // per-chunk partial gradients
     return 2 * rows * (int64_t)hidden;
 }
 
@@ -825,8 +847,11 @@ int tmla_mlp_backward(const float *params, int obs_dim, int hidden, int n_action
                       float *scratch, void *stream) {
     TMLA_REQUIRE(params && x && act_cache && dlogits && dvalues && grads && scratch, "NULL buffer");
     TMLA_REQUIRE(rows > 0, "rows must be positive");
-    int rc = check_shape(obs_dim, hidden, n_actions);
+    int rc = check_shape(obs_dim, hidden, n_actions, true);
     if (rc) return rc;
+    if (hidden != H)
+        return small_mlp_backward(params, obs_dim, hidden, n_actions, x, index, rows, act_cache, dlogits, dvalues, grads, scratch,
+                                  (cudaStream_t)stream);
     return mlp_backward_impl<float>(params, nullptr, obs_dim, n_actions, x, index, rows, act_cache, dlogits, dvalues, grads, scratch,
                                     (cudaStream_t)stream);
 }

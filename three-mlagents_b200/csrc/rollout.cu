@@ -74,7 +74,8 @@ int tmla_rollout(tmla_env *h, const tmla_rollout_args *args, void *stream) {
     TMLA_REQUIRE(a.trunc_count && a.trunc_index && a.trunc_obs && a.trunc_values && a.trunc_capacity > 0, "truncation list is incomplete");
     TMLA_REQUIRE(a.n_steps > 0 && a.obs_dim == tmla_task_obs_dim(h->task) && a.n_actions == tmla_task_num_actions(h->task),
                  "n_steps / obs_dim / n_actions do not match the handle's task");
-    TMLA_REQUIRE(a.act_cache || (a.wpack && a.obs_dim <= 6), "act_cache may be NULL only on the fused-tower shapes (bf16, obs_dim <= 6)");
+    TMLA_REQUIRE(a.act_cache || (a.wpack ? a.obs_dim <= 6 : (a.hidden == 64 || a.hidden == 128)),
+                 "act_cache may be NULL only on the fused-tower shapes (bf16, obs_dim <= 6) and for the fp32 widths 64 and 128");
     DeviceGuard guard(h->device);
     cudaStream_t st = (cudaStream_t)stream;
     // the device-side step counter the graph's kernels read: (re)synchronised with the handle on every call (8 bytes)

@@ -10,7 +10,7 @@ import torch
 from . import native
 from .native import lib, check, ptr
 
-HIDDEN = 256
+HIDDEN = 256          # default width; 64 and 128 run on the float32 kernels of csrc/mlp_small.cu (wpack=None only)
 
 
 def _chk(t, dtype, name):
@@ -28,10 +28,10 @@ def _s():
     return native.current_stream()
 
 
-def num_params(obs_dim: int, n_actions: int) -> int:
-    n = lib.tmla_mlp_num_params(obs_dim, HIDDEN, n_actions)
+def num_params(obs_dim: int, n_actions: int, hidden: int = HIDDEN) -> int:
+    n = lib.tmla_mlp_num_params(obs_dim, hidden, n_actions)
     if n < 0:
-        raise ValueError("unsupported MLP shape")
+        raise ValueError(f"unsupported MLP shape (obs_dim {obs_dim}, hidden {hidden}, n_actions {n_actions}): hidden is 64, 128 or 256")
     return int(n)
 
 
@@ -69,9 +69,11 @@ def mlp_pack(params, obs_dim, n_actions, wpack=None):
 
 
 def mlp_forward(params, x, obs_dim, n_actions, *, index=None, rows=None, rows_dev=None, logits=None, values=None,
-                want_logits=True, want_values=True, act_cache=None, wpack=None, keep_act=True):
+                want_logits=True, want_values=True, act_cache=None, wpack=None, keep_act=True, hidden=HIDDEN):
     """ActorCriticPolicy.forward.  wpack=None: float32 CUDA-core path; wpack=bf16 pack: tcgen05 path
-    (act_cache is then bf16 [4,rows,256])."""
+    (act_cache is then bf16 [4,rows,256]).  hidden 64 / 128: float32 only; keep_act=False keeps no activations."""
+    if wpack is not None and hidden != HIDDEN:
+        raise ValueError(f"the bf16 tensor-core path covers hidden = {HIDDEN} only (got {hidden})")
     _chk(params, torch.float32, "params"); _chk(x, torch.float32, "x"); _chk(index, torch.int32, "index")
     if rows is None:
         rows = index.numel() if index is not None else x.shape[0]
@@ -81,14 +83,14 @@ def mlp_forward(params, x, obs_dim, n_actions, *, index=None, rows=None, rows_de
         logits = torch.empty((rows, n_actions), dtype=torch.float32, device=dev)
     if want_values and values is None:
         values = torch.empty(rows, dtype=torch.float32, device=dev)
-    if wpack is not None and not keep_act and obs_dim <= 6:
-        act_cache = None            # fused tower kernel, inference only: no activation workspace
+    if not keep_act and ((wpack is not None and obs_dim <= 6) or hidden != HIDDEN):
+        act_cache = None            # fused tower kernel / small widths, inference only: no activation workspace
     elif act_cache is None:
-        act_cache = torch.empty((4, rows, HIDDEN), dtype=act_dtype, device=dev)
+        act_cache = torch.empty((4, rows, hidden), dtype=act_dtype, device=dev)
     _chk(act_cache, act_dtype, "act_cache")
     lg, vl = (ptr(logits) if want_logits else None), (ptr(values) if want_values else None)
     if wpack is None:
-        check(lib.tmla_mlp_forward(ptr(params), obs_dim, HIDDEN, n_actions, ptr(x), ptr(index), int(rows), ptr(rows_dev),
+        check(lib.tmla_mlp_forward(ptr(params), obs_dim, hidden, n_actions, ptr(x), ptr(index), int(rows), ptr(rows_dev),
                                    lg, vl, ptr(act_cache), _s()))
     else:
         check(lib.tmla_mlp_forward_bf16(ptr(params), ptr(wpack), obs_dim, HIDDEN, n_actions, ptr(x), ptr(index), int(rows),
@@ -97,7 +99,11 @@ def mlp_forward(params, x, obs_dim, n_actions, *, index=None, rows=None, rows_de
 
 
 def mlp_backward(params, x, obs_dim, n_actions, act_cache, dlogits, dvalues, *, index=None, rows=None, grads=None,
-                 scratch=None, wpack=None):
+                 scratch=None, wpack=None, hidden=HIDDEN):
+    """Gradient of ActorCriticPolicy.forward (flat, overwritten).  hidden 64 / 128: scratch holds per-chunk partial gradients,
+    summed in a fixed order (bit-identical across calls)."""
+    if wpack is not None and hidden != HIDDEN:
+        raise ValueError(f"the bf16 tensor-core path covers hidden = {HIDDEN} only (got {hidden})")
     if rows is None:
         rows = index.numel() if index is not None else x.shape[0]
     dev = params.device
@@ -105,11 +111,14 @@ def mlp_backward(params, x, obs_dim, n_actions, act_cache, dlogits, dvalues, *, 
     if grads is None:
         grads = torch.empty_like(params)
     if scratch is None:
-        scratch = torch.empty(lib.tmla_mlp_backward_scratch(obs_dim, HIDDEN, n_actions, rows), dtype=act_dtype, device=dev)
+        size = lib.tmla_mlp_backward_scratch(obs_dim, hidden, n_actions, rows)
+        if size < 0:
+            raise ValueError(native.last_error())
+        scratch = torch.empty(size, dtype=act_dtype, device=dev)
     _chk(dlogits, torch.float32, "dlogits"); _chk(dvalues, torch.float32, "dvalues")
     _chk(act_cache, act_dtype, "act_cache"); _chk(scratch, act_dtype, "scratch")
     if wpack is None:
-        check(lib.tmla_mlp_backward(ptr(params), obs_dim, HIDDEN, n_actions, ptr(x), ptr(index), int(rows), ptr(act_cache),
+        check(lib.tmla_mlp_backward(ptr(params), obs_dim, hidden, n_actions, ptr(x), ptr(index), int(rows), ptr(act_cache),
                                     ptr(dlogits), ptr(dvalues), ptr(grads), ptr(scratch), _s()))
     else:
         check(lib.tmla_mlp_backward_bf16(ptr(params), ptr(wpack), obs_dim, HIDDEN, n_actions, ptr(x), ptr(index), int(rows),
@@ -179,8 +188,8 @@ def a2c_loss(logits, values, actions, advantages, returns, *, index=None, rows=N
     return dlogits, dvalues, stats
 
 
-def ppo_minibatch_supported(obs_dim: int, n_actions: int) -> bool:
-    return bool(lib.tmla_ppo_minibatch_supported(obs_dim, HIDDEN, n_actions))
+def ppo_minibatch_supported(obs_dim: int, n_actions: int, hidden: int = HIDDEN) -> bool:
+    return bool(lib.tmla_ppo_minibatch_supported(obs_dim, hidden, n_actions))
 
 
 def ppo_minibatch(params, wpack, obs, obs_dim, n_actions, actions, advantages, old_logp, returns, *, index=None, rows=None,
@@ -242,7 +251,7 @@ def a2c_batch(params, wpack, obs, obs_dim, n_actions, actions, advantages, retur
 
 
 def adam_clip(params, grads, m, v, step, *, grad_scale=1.0, max_grad_norm=0.5, lr=3e-4, beta1=0.9, beta2=0.999,
-              eps=1e-5, norm_out=None, zero_grads=False, wpack=None, obs_dim=0, n_actions=0):
+              eps=1e-5, norm_out=None, zero_grads=False, wpack=None, obs_dim=0, n_actions=0, hidden=HIDDEN):
     """clip_grad_norm_ + Adam.step.  zero_grads: clear `grads` once consumed.  wpack (+ obs_dim, n_actions): also refresh the bf16
     operand images of the hidden-layer weights inside `wpack` (what the fused minibatch kernel reads)."""
     if norm_out is None:
@@ -250,43 +259,43 @@ def adam_clip(params, grads, m, v, step, *, grad_scale=1.0, max_grad_norm=0.5, l
     _chk(wpack, torch.bfloat16, "wpack")
     check(lib.tmla_adam_clip_fused(ptr(params), ptr(grads), ptr(m), ptr(v), params.numel(), float(grad_scale),
                                    float(max_grad_norm), float(lr), float(beta1), float(beta2), float(eps), int(step),
-                                   ptr(norm_out), 1 if zero_grads else 0, ptr(wpack), int(obs_dim), HIDDEN, int(n_actions), _s()))
+                                   ptr(norm_out), 1 if zero_grads else 0, ptr(wpack), int(obs_dim), int(hidden), int(n_actions), _s()))
     return norm_out
 
 
 def adam_clip_allreduce(comm, params, grads, m, v, step, *, grad_scale=1.0, max_grad_norm=0.5, lr=3e-4, beta1=0.9, beta2=0.999,
-                        eps=1e-5, norm_out=None, zero_grads=False, wpack=None, obs_dim=0, n_actions=0):
+                        eps=1e-5, norm_out=None, zero_grads=False, wpack=None, obs_dim=0, n_actions=0, hidden=HIDDEN):
     """grads <- sum over ranks (one-shot all-reduce over NVLink peer memory, rank order), then adam_clip — two launches, no NCCL."""
     if norm_out is None:
         norm_out = torch.zeros(132, dtype=torch.float32, device=params.device)
     _chk(wpack, torch.bfloat16, "wpack"); _chk(grads, torch.float32, "grads")
     check(lib.tmla_adam_clip_allreduce(comm.handle, ptr(params), ptr(grads), ptr(m), ptr(v), params.numel(), float(grad_scale),
                                        float(max_grad_norm), float(lr), float(beta1), float(beta2), float(eps), int(step),
-                                       ptr(norm_out), 1 if zero_grads else 0, ptr(wpack), int(obs_dim), HIDDEN, int(n_actions), _s()))
+                                       ptr(norm_out), 1 if zero_grads else 0, ptr(wpack), int(obs_dim), int(hidden), int(n_actions), _s()))
     return norm_out
 
 
 def rmsprop_clip(params, grads, sq_avg, *, grad_scale=1.0, max_grad_norm=0.5, lr=7e-4, alpha=0.99, eps=1e-5, norm_out=None,
-                 zero_grads=False, wpack=None, obs_dim=0, n_actions=0):
+                 zero_grads=False, wpack=None, obs_dim=0, n_actions=0, hidden=HIDDEN):
     """clip_grad_norm_ + torch.optim.RMSprop.step in one launch (tmla_rmsprop_clip_fused); flags as adam_clip."""
     if norm_out is None:
         norm_out = torch.zeros(132, dtype=torch.float32, device=params.device)
     _chk(wpack, torch.bfloat16, "wpack"); _chk(grads, torch.float32, "grads"); _chk(sq_avg, torch.float32, "sq_avg")
     check(lib.tmla_rmsprop_clip_fused(ptr(params), ptr(grads), ptr(sq_avg), params.numel(), float(grad_scale), float(max_grad_norm),
                                       float(lr), float(alpha), float(eps), ptr(norm_out), 1 if zero_grads else 0, ptr(wpack),
-                                      int(obs_dim), HIDDEN, int(n_actions), _s()))
+                                      int(obs_dim), int(hidden), int(n_actions), _s()))
     return norm_out
 
 
 def rmsprop_clip_allreduce(comm, params, grads, sq_avg, step, *, grad_scale=1.0, max_grad_norm=0.5, lr=7e-4, alpha=0.99, eps=1e-5,
-                           norm_out=None, zero_grads=False, wpack=None, obs_dim=0, n_actions=0):
+                           norm_out=None, zero_grads=False, wpack=None, obs_dim=0, n_actions=0, hidden=HIDDEN):
     """grads <- sum over ranks over NVLink peer memory, then rmsprop_clip, in the same launch; `step` = exchange sequence number."""
     if norm_out is None:
         norm_out = torch.zeros(132, dtype=torch.float32, device=params.device)
     _chk(wpack, torch.bfloat16, "wpack"); _chk(grads, torch.float32, "grads"); _chk(sq_avg, torch.float32, "sq_avg")
     check(lib.tmla_rmsprop_clip_allreduce(comm.handle, ptr(params), ptr(grads), ptr(sq_avg), params.numel(), float(grad_scale),
                                           float(max_grad_norm), float(lr), float(alpha), float(eps), int(step), ptr(norm_out),
-                                          1 if zero_grads else 0, ptr(wpack), int(obs_dim), HIDDEN, int(n_actions), _s()))
+                                          1 if zero_grads else 0, ptr(wpack), int(obs_dim), int(hidden), int(n_actions), _s()))
     return norm_out
 
 

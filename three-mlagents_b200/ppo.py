@@ -28,7 +28,8 @@ from .native import ptr
 from .distributed import PeerComm, allreduce_sum_, dist_state
 from .vec_env import CudaVecEnv
 
-HIDDEN = 256
+HIDDEN = 256                   # the default net_arch dict(pi=[256, 256], vf=[256, 256]) (training.py:363-365)
+WIDTHS = (64, 128, 256)        # 256: bf16 tcgen05 kernels (default) or fp32; 64, 128: fp32 kernels of csrc/mlp_small.cu
 
 
 _dist = dist_state
@@ -48,14 +49,43 @@ def _on_device(fn):
     return wrapped
 
 
-def orthogonal_init(obs_dim: int, n_actions: int, seed: int) -> torch.Tensor:
+def parse_net_arch(policy_kwargs: dict | None) -> int:
+    """The hidden width H of `policy_kwargs`: net_arch [H, H] or dict(pi=[H, H], vf=[H, H]) with H in 64, 128, 256 (no
+    net_arch: 256).  activation_fn=nn.Tanh and ortho_init=True may be given; any other policy_kwargs entry is rejected."""
+    pk = dict(policy_kwargs or {})
+    supported = ("supported: net_arch [H, H] or dict(pi=[H, H], vf=[H, H]) with H in 64, 128, 256, tanh activations, "
+                 "orthogonal init")
+    act = pk.pop("activation_fn", torch.nn.Tanh)
+    if act is not torch.nn.Tanh:
+        raise ValueError(f"activation_fn {act!r} is not implemented ({supported})")
+    if pk.pop("ortho_init", True) is not True:
+        raise ValueError(f"ortho_init=False is not implemented ({supported})")
+    arch = pk.pop("net_arch", [HIDDEN, HIDDEN])
+    if pk:
+        raise ValueError(f"policy_kwargs {sorted(pk)} are not implemented ({supported})")
+    if isinstance(arch, dict):
+        if set(arch) != {"pi", "vf"}:
+            raise ValueError(f"net_arch {arch!r}: a dict needs exactly the keys 'pi' and 'vf' ({supported})")
+        pi, vf = list(arch["pi"]), list(arch["vf"])
+        if pi != vf:
+            raise ValueError(f"net_arch {arch!r}: pi and vf must be equal ({supported})")
+        arch = pi
+    arch = list(arch) if isinstance(arch, (list, tuple)) else arch
+    if not isinstance(arch, list) or len(arch) != 2 or arch[0] != arch[1] or arch[0] not in WIDTHS \
+            or not all(isinstance(h, int) and not isinstance(h, bool) for h in arch):
+        raise ValueError(f"net_arch {arch!r} is not implemented ({supported})")
+    return int(arch[0])
+
+
+def orthogonal_init(obs_dim: int, n_actions: int, seed: int, hidden: int = HIDDEN) -> torch.Tensor:
     """SB3 ActorCriticPolicy init: orthogonal weights with gain sqrt(2) (towers), 0.01 (action_net),
     1.0 (value_net), zero biases; flat vector in policy.parameters() order (include/tmla.h)."""
     g = torch.Generator().manual_seed(int(seed))
+    H = int(hidden)
     shapes = []
     for _tower in range(2):
-        shapes += [((HIDDEN, obs_dim), math.sqrt(2.0)), ((HIDDEN,), None), ((HIDDEN, HIDDEN), math.sqrt(2.0)), ((HIDDEN,), None)]
-    shapes += [((n_actions, HIDDEN), 0.01), ((n_actions,), None), ((1, HIDDEN), 1.0), ((1,), None)]
+        shapes += [((H, obs_dim), math.sqrt(2.0)), ((H,), None), ((H, H), math.sqrt(2.0)), ((H,), None)]
+    shapes += [((n_actions, H), 0.01), ((n_actions,), None), ((1, H), 1.0), ((1,), None)]
     chunks = []
     for shape, gain in shapes:
         t = torch.zeros(shape, dtype=torch.float32)
@@ -80,9 +110,7 @@ class CudaPPO:
                  _params: torch.Tensor | None = None):
         if policy != "MlpPolicy":
             raise ValueError("CudaPPO supports 'MlpPolicy' (vector observations) only")
-        arch = (policy_kwargs or {}).get("net_arch", {"pi": [256, 256], "vf": [256, 256]})
-        if arch != {"pi": [256, 256], "vf": [256, 256]}:
-            raise ValueError("CudaPPO implements net_arch dict(pi=[256,256], vf=[256,256]) (training.py:363-365)")
+        self.hidden = parse_net_arch(policy_kwargs)
         self.env = env
         self.seed = int(seed)
         self.lr, self.n_steps, self.batch_size, self.n_epochs = float(learning_rate), int(n_steps), int(batch_size), int(n_epochs)
@@ -92,10 +120,13 @@ class CudaPPO:
         self.verbose, self.tensorboard_log = int(verbose), tensorboard_log
         if mlp_impl not in ("auto", "bf16", "fp32"):
             raise ValueError("mlp_impl must be 'auto', 'bf16' (tcgen05 tensor cores) or 'fp32' (CUDA cores)")
-        self.mlp_impl = "bf16" if mlp_impl == "auto" else mlp_impl
+        if mlp_impl == "bf16" and self.hidden != HIDDEN:
+            raise ValueError(f"mlp_impl='bf16' covers net_arch width {HIDDEN} only; width {self.hidden} runs in fp32")
+        self.mlp_impl = ("bf16" if self.hidden == HIDDEN else "fp32") if mlp_impl == "auto" else mlp_impl
         self.obs_dim, self.n_actions, self.n_envs = env.obs_dim, env.n_actions, env.num_envs
         # one fused forward+loss+backward kernel per tower and minibatch (csrc/mlp_train.cu) where the shape allows
-        self.fused_update = bool(fused_update) and self.mlp_impl == "bf16" and ops.ppo_minibatch_supported(self.obs_dim, self.n_actions)
+        self.fused_update = bool(fused_update) and self.mlp_impl == "bf16" and ops.ppo_minibatch_supported(self.obs_dim, self.n_actions,
+                                                                                                          self.hidden)
         self.device = torch.device("cuda", env.device_index)
         self.num_timesteps = 0
         self.n_updates = 0
@@ -104,8 +135,10 @@ class CudaPPO:
         self._epoch_counter = 0
         self._dist, self.rank, self.world = _dist()
         with torch.cuda.device(self.device):
-            p = orthogonal_init(self.obs_dim, self.n_actions, self.seed) if _params is None else _params.detach().float().cpu()
-            assert p.numel() == ops.num_params(self.obs_dim, self.n_actions)
+            p = (orthogonal_init(self.obs_dim, self.n_actions, self.seed, self.hidden) if _params is None
+                 else _params.detach().float().cpu())
+            if p.numel() != ops.num_params(self.obs_dim, self.n_actions, self.hidden):
+                raise ValueError(f"{p.numel()} parameters do not fit net_arch width {self.hidden} for {self.obs_dim} -> {self.n_actions}")
             self.params = p.to(self.device).contiguous()
             self.m = torch.zeros_like(self.params)
             self.v = torch.zeros_like(self.params)
@@ -149,14 +182,17 @@ class CudaPPO:
         self.done = torch.empty((T, N), dtype=torch.uint8, device=dev)
         self.last_values = torch.empty(N, **f32)
         self.logits_roll = torch.empty((N, A), **f32)
-        self.cache_roll = torch.empty((4, N, HIDDEN), dtype=self._act_dtype, device=dev)
+        H = self.hidden
+        small = H != HIDDEN            # widths 64 / 128: the rollout's forwards keep no activations, so no rollout caches
+        self.cache_roll = None if small else torch.empty((4, N, H), dtype=self._act_dtype, device=dev)
         # every env can hit its time limit at most floor(T/limit)+1 times per rollout
         cap = N * (T // self.env.max_episode_steps + 1)
         self.trunc_count = torch.zeros(1, dtype=torch.int32, device=dev)
         self.trunc_index = torch.zeros(cap, dtype=torch.int32, device=dev)
         self.trunc_obs = torch.zeros((cap, D), **f32)
         self.trunc_values = torch.zeros(cap, **f32)
-        self.cache_trunc = torch.empty((4, cap, HIDDEN), dtype=self._act_dtype, device=dev) if cap != N else self.cache_roll
+        self.cache_trunc = (None if small else torch.empty((4, cap, H), dtype=self._act_dtype, device=dev) if cap != N
+                            else self.cache_roll)
         self.ep_stats = torch.zeros(4, **f32)
         total = T * N
         B = min(self.batch_size, total)
@@ -167,9 +203,12 @@ class CudaPPO:
             self.values_mb = torch.empty(B, **f32)
             self.dlogits = torch.empty((B, A), **f32)
             self.dvalues = torch.empty(B, **f32)
-            self.cache_mb = torch.empty((4, B, HIDDEN), dtype=self._act_dtype, device=dev)
-        n_img = 4 if self.fused_update else 2          # fused: H1 and dZ2 tile images of both towers
-        self.scratch_mb = torch.empty(n_img * ((B + 127) // 128 * 128) * HIDDEN, dtype=self._act_dtype, device=dev)
+            self.cache_mb = torch.empty((4, B, H), dtype=self._act_dtype, device=dev)
+        if small:                                      # per-chunk partial gradients of the fixed-order reduction (mlp_small.cu)
+            self.scratch_mb = torch.empty(native.lib.tmla_mlp_backward_scratch(D, H, A, B), dtype=torch.float32, device=dev)
+        else:
+            n_img = 4 if self.fused_update else 2      # fused: H1 and dZ2 tile images of both towers
+            self.scratch_mb = torch.empty(n_img * ((B + 127) // 128 * 128) * HIDDEN, dtype=self._act_dtype, device=dev)
         self.adv_sums = torch.zeros(((total + B - 1) // B, 3), dtype=torch.float64, device=dev)   # one row per minibatch of an epoch
         self.stats = torch.zeros(8, **f32)
         self.stats_acc = torch.zeros(8, **f32)
@@ -194,15 +233,17 @@ class CudaPPO:
             # ONE call: T x {tower forward, sample + env step}, last-value and timeout-bootstrap forwards, GAE — a CUDA graph
             # recorded once per buffer set inside libtmla.so and replayed here (include/tmla.h tmla_rollout)
             if self._rollout_args is None:
-                keep = self.cache_trunc if self.cache_trunc.numel() >= self.cache_roll.numel() else self.cache_roll
-                need_cache = not (self.mlp_impl == "bf16" and D <= 6)
+                need_cache = not ((self.mlp_impl == "bf16" and D <= 6) or self.hidden != HIDDEN)      # inference-only forwards
+                keep = None
+                if need_cache:
+                    keep = self.cache_trunc if self.cache_trunc.numel() >= self.cache_roll.numel() else self.cache_roll
                 self._rollout_args = native.RolloutArgs(
                     params=ptr(self.params), wpack=ptr(self.wpack), act_cache=ptr(keep) if need_cache else None,
                     obs=ptr(self.obs), actions=ptr(self.act), log_probs=ptr(self.logp), rewards=ptr(self.rew), values=ptr(self.val),
                     dones=ptr(self.done), last_values=ptr(self.last_values), advantages=ptr(self.adv), returns=ptr(self.ret),
                     logits=ptr(self.logits_roll), trunc_count=ptr(self.trunc_count), trunc_index=ptr(self.trunc_index),
                     trunc_obs=ptr(self.trunc_obs), trunc_values=ptr(self.trunc_values), ep_stats=ptr(self.ep_stats),
-                    step_counter=ptr(self.step_counter), gamma=self.gamma, gae_lambda=self.gae_lambda, obs_dim=D, hidden=HIDDEN,
+                    step_counter=ptr(self.step_counter), gamma=self.gamma, gae_lambda=self.gae_lambda, obs_dim=D, hidden=self.hidden,
                     n_actions=A, n_steps=T, deterministic=0, trunc_capacity=self.trunc_index.numel())
             native.check(native.lib.tmla_rollout(self.env.handle, self._rollout_args, native.current_stream()))
             nvtx.range_pop()
@@ -212,16 +253,16 @@ class CudaPPO:
         self.ep_stats.zero_()
         for t in range(T):
             ops.mlp_forward(self.params, self.obs[t], D, A, rows=N, logits=self.logits_roll, values=self.val[t],
-                            act_cache=self.cache_roll, wpack=self.wpack, keep_act=False)
+                            act_cache=self.cache_roll, wpack=self.wpack, keep_act=False, hidden=self.hidden)
             ops.step_policy(self.env, self.logits_roll, t, self.obs[t + 1], self.act[t], self.logp[t], self.rew[t],
                             self.done[t], trunc_count=self.trunc_count, trunc_index=self.trunc_index,
                             trunc_obs=self.trunc_obs, ep_stats=self.ep_stats)
         ops.mlp_forward(self.params, self.obs[T], D, A, rows=N, want_logits=False, values=self.last_values,
-                        act_cache=self.cache_roll, wpack=self.wpack, keep_act=False)
+                        act_cache=self.cache_roll, wpack=self.wpack, keep_act=False, hidden=self.hidden)
         # timeout bootstrap: rewards += gamma * V(terminal_obs) for time-limit truncations
         cap = self.trunc_index.numel()
         ops.mlp_forward(self.params, self.trunc_obs, D, A, rows=cap, rows_dev=self.trunc_count, want_logits=False,
-                        values=self.trunc_values, act_cache=self.cache_trunc, wpack=self.wpack, keep_act=False)
+                        values=self.trunc_values, act_cache=self.cache_trunc, wpack=self.wpack, keep_act=False, hidden=self.hidden)
         ops.bootstrap_add(self.rew, self.trunc_count, self.trunc_index, self.trunc_values, self.gamma)
         nvtx.range_pop()
         nvtx.range_push("gae")
@@ -261,13 +302,13 @@ class CudaPPO:
                                       grads_zeroed=True, accumulate_stats=True)
                 else:
                     ops.mlp_forward(self.params, obs_flat, D, A, index=idx, rows=rows, logits=self.logits_mb,
-                                    values=self.values_mb, act_cache=self.cache_mb, wpack=self.wpack)
+                                    values=self.values_mb, act_cache=self.cache_mb, wpack=self.wpack, hidden=self.hidden)
                     ops.ppo_loss(self.logits_mb, self.values_mb, self.act, self.adv, self.logp, self.ret, index=idx,
                                  rows=rows, global_rows=rows * self.world, adv_sums=sums, normalize=sums is not None,
                                  clip_range=self.clip_range, ent_coef=self.ent_coef, vf_coef=self.vf_coef,
                                  dlogits=self.dlogits, dvalues=self.dvalues, stats=self.stats)
                     ops.mlp_backward(self.params, obs_flat, D, A, self.cache_mb, self.dlogits, self.dvalues, index=idx,
-                                     rows=rows, grads=self.grads, scratch=self.scratch_mb, wpack=self.wpack)
+                                     rows=rows, grads=self.grads, scratch=self.scratch_mb, wpack=self.wpack, hidden=self.hidden)
                 self._adam_step += 1
                 if self._comm is not None:                # the one collective on the path, inside the optimizer launches
                     nvtx.range_push("allreduce+adam")
@@ -377,7 +418,7 @@ class CudaPPO:
     def policy_logits(self, obs_dev: torch.Tensor) -> torch.Tensor:
         rows = obs_dev.shape[0]
         logits, _, _ = ops.mlp_forward(self.params, obs_dev.contiguous(), self.obs_dim, self.n_actions, rows=rows,
-                                       want_values=False, wpack=self.wpack, keep_act=False)
+                                       want_values=False, wpack=self.wpack, keep_act=False, hidden=self.hidden)
         return logits
 
     @_on_device
@@ -432,8 +473,9 @@ class CudaPPO:
 
     @classmethod
     def load(cls, path, env: CudaVecEnv | None = None, device: int = 0, task_id: str | None = None):
-        """`PPO.load` (training.py:269): accepts zips written by this backend and SB3-written zips of the same
-        architecture (pass `task_id` for those; it is inferred from the shapes when unambiguous)."""
+        """`PPO.load` (training.py:269): accepts zips written by this backend and SB3-written MlpPolicy zips of hidden width
+        64, 128 or 256 (SB3's default [64, 64] included; pass `task_id` for those, it is inferred from the shapes when
+        unambiguous).  The model is built at the zip's width."""
         from . import sb3_zip
 
         z = sb3_zip.read_zip(str(path))
@@ -451,7 +493,8 @@ class CudaPPO:
         for k in cls._HYPER_KEYS:
             if k not in hyper and isinstance(data.get(k), (int, float)):
                 hyper[k] = data[k]
-        model = cls("MlpPolicy", env, seed=seed, _params=z["params"], **hyper)
+        pk = {} if z["hidden"] == HIDDEN else {"policy_kwargs": {"net_arch": [z["hidden"], z["hidden"]]}}
+        model = cls("MlpPolicy", env, seed=seed, _params=z["params"], **pk, **hyper)
         model._repack()
         model._load_optimizer_state(z, meta)
         model.num_timesteps = int(meta.get("num_timesteps", data.get("num_timesteps", 0) or 0))

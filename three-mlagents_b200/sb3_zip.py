@@ -6,8 +6,8 @@ writes — `data` (JSON), `policy.pth` (state dict with SB3's parameter names), 
 state dict), `pytorch_variables.pth`, `_stable_baselines3_version`, `system_info.txt` — plus `tmla.json`, this
 backend's own metadata.  A2C models (CudaA2C) write the same members with A2C's `data` attributes and a torch RMSprop state dict.
 `read_zip` accepts both this backend's zips and zips written by SB3 itself for the
-same architecture (MlpPolicy, net_arch dict(pi=[256,256], vf=[256,256])), so SB3-trained policies can be
-evaluated on the CUDA backend.
+same architecture (MlpPolicy, net_arch dict(pi=[H,H], vf=[H,H]) with H = 64, 128 or 256; SB3's default is 64), so
+SB3-trained policies can be evaluated on the CUDA backend.  The width is read off the state dict's shapes.
 
 What can be checked here IS checked (tests/test_sb3_zip_cpu.py): parameter names/shapes/order, the round trip
 flat vector <-> state dict, optimizer state layout, archive members, `data` decodability.  Loading the zip
@@ -30,12 +30,14 @@ from collections import OrderedDict
 import numpy as np
 import torch
 
-H = 256
+H = 256                    # default hidden width
+WIDTHS = (64, 128, 256)
 SB3_VERSION = "2.9.0"
 
 
-def param_layout(obs_dim: int, n_actions: int):
+def param_layout(obs_dim: int, n_actions: int, hidden: int = H):
     """(SB3 state-dict key, shape) in policy.parameters() order == order of the flat vector (include/tmla.h)."""
+    H = int(hidden)
     return [
         ("mlp_extractor.policy_net.0.weight", (H, obs_dim)), ("mlp_extractor.policy_net.0.bias", (H,)),
         ("mlp_extractor.policy_net.2.weight", (H, H)), ("mlp_extractor.policy_net.2.bias", (H,)),
@@ -46,10 +48,10 @@ def param_layout(obs_dim: int, n_actions: int):
     ]
 
 
-def flat_to_state_dict(flat: torch.Tensor, obs_dim: int, n_actions: int) -> "OrderedDict[str, torch.Tensor]":
+def flat_to_state_dict(flat: torch.Tensor, obs_dim: int, n_actions: int, hidden: int = H) -> "OrderedDict[str, torch.Tensor]":
     flat = flat.detach().float().cpu().contiguous()
     sd, p = OrderedDict(), 0
-    for name, shape in param_layout(obs_dim, n_actions):
+    for name, shape in param_layout(obs_dim, n_actions, hidden):
         n = int(np.prod(shape))
         sd[name] = flat[p:p + n].clone().view(shape)
         p += n
@@ -58,11 +60,12 @@ def flat_to_state_dict(flat: torch.Tensor, obs_dim: int, n_actions: int) -> "Ord
     return sd
 
 
-def state_dict_to_flat(sd, obs_dim: int, n_actions: int) -> torch.Tensor:
+def state_dict_to_flat(sd, obs_dim: int, n_actions: int, hidden: int = H) -> torch.Tensor:
     chunks = []
-    for name, shape in param_layout(obs_dim, n_actions):
+    for name, shape in param_layout(obs_dim, n_actions, hidden):
         if name not in sd:
-            raise KeyError(f"state dict has no '{name}' (not an MlpPolicy with net_arch dict(pi=[256,256], vf=[256,256])?)")
+            raise KeyError(f"state dict has no '{name}' (not an MlpPolicy with net_arch dict(pi=[{hidden},{hidden}], "
+                           f"vf=[{hidden},{hidden}])?)")
         t = torch.as_tensor(sd[name]).float()
         if tuple(t.shape) != tuple(shape):
             raise ValueError(f"{name}: shape {tuple(t.shape)} != {shape}")
@@ -70,9 +73,21 @@ def state_dict_to_flat(sd, obs_dim: int, n_actions: int) -> torch.Tensor:
     return torch.cat(chunks)
 
 
-def adam_state_dict(m, v, step: int, hyper: dict, obs_dim: int, n_actions: int) -> dict:
+def hidden_width(sd) -> int:
+    """The hidden width of an MlpPolicy state dict: both hidden layers of both towers square and equal, 64, 128 or 256."""
+    try:
+        shapes = [tuple(sd[f"mlp_extractor.{t}.{i}.weight"].shape) for t in ("policy_net", "value_net") for i in (0, 2)]
+    except KeyError as e:
+        raise KeyError(f"state dict has no {e} (not an MlpPolicy with a two-layer net_arch?)") from None
+    h = shapes[0][0]
+    if any(s[0] != h for s in shapes) or shapes[1][1] != h or shapes[3][1] != h or h not in WIDTHS:
+        raise ValueError(f"hidden layers {shapes}: supported are net_arch dict(pi=[H,H], vf=[H,H]) with H in {WIDTHS}")
+    return int(h)
+
+
+def adam_state_dict(m, v, step: int, hyper: dict, obs_dim: int, n_actions: int, hidden: int = H) -> dict:
     """torch.optim.Adam.state_dict() layout for the 12 parameter tensors."""
-    ms, vs = flat_to_state_dict(m, obs_dim, n_actions), flat_to_state_dict(v, obs_dim, n_actions)
+    ms, vs = flat_to_state_dict(m, obs_dim, n_actions, hidden), flat_to_state_dict(v, obs_dim, n_actions, hidden)
     state = {}
     for i, name in enumerate(ms):
         if step > 0:
@@ -83,11 +98,11 @@ def adam_state_dict(m, v, step: int, hyper: dict, obs_dim: int, n_actions: int) 
     return {"state": state, "param_groups": [group]}
 
 
-def rmsprop_state_dict(sq_avg, step: int, hyper: dict, obs_dim: int, n_actions: int) -> dict:
+def rmsprop_state_dict(sq_avg, step: int, hyper: dict, obs_dim: int, n_actions: int, hidden: int = H) -> dict:
     """torch.optim.RMSprop(alpha=0.99, eps=rms_prop_eps, weight_decay=0).state_dict() for the 12 parameter tensors, produced by a
     real RMSprop instance so that the layout (state keys, param_group entries) is torch's own."""
-    sq = flat_to_state_dict(sq_avg, obs_dim, n_actions)
-    params = [torch.nn.Parameter(torch.zeros(shape)) for _, shape in param_layout(obs_dim, n_actions)]
+    sq = flat_to_state_dict(sq_avg, obs_dim, n_actions, hidden)
+    params = [torch.nn.Parameter(torch.zeros(shape)) for _, shape in param_layout(obs_dim, n_actions, hidden)]
     opt = torch.optim.RMSprop(params, lr=hyper["learning_rate"], alpha=0.99, eps=hyper["rms_prop_eps"], weight_decay=0)
     if step > 0:
         for p, name in zip(params, sq):
@@ -163,8 +178,10 @@ def _build_data(model) -> dict:
     pc["__module__"] = "stable_baselines3.common.policies"
     rb = _serialized(buf_cls, "<class 'abc.ABCMeta'>")
     rb["__module__"] = "stable_baselines3.common.buffers"
+    hid = getattr(model, "hidden", H)
+    net_arch = {"pi": [hid, hid], "vf": [hid, hid]}
     data = {
-        "policy_class": pc, "verbose": model.verbose, "policy_kwargs": {"net_arch": {"pi": [256, 256], "vf": [256, 256]}},
+        "policy_class": pc, "verbose": model.verbose, "policy_kwargs": {"net_arch": net_arch},
         "num_timesteps": model.num_timesteps, "_total_timesteps": model.num_timesteps, "_num_timesteps_at_start": 0,
         "seed": model.seed, "action_noise": None, "start_time": 0, "learning_rate": model.lr,
         "tensorboard_log": model.tensorboard_log, "_last_obs": None, "_last_episode_starts": None,
@@ -175,7 +192,7 @@ def _build_data(model) -> dict:
         "max_grad_norm": model.max_grad_norm, "rollout_buffer_class": rb, "rollout_buffer_kwargs": {},
     }
     if getattr(model, "algorithm", "ppo") == "a2c":      # A2C.__init__: use_rms_prop puts RMSprop and its kwargs into policy_kwargs
-        kwargs = {"net_arch": {"pi": [256, 256], "vf": [256, 256]}, "optimizer_class": torch.optim.RMSprop,
+        kwargs = {"net_arch": net_arch, "optimizer_class": torch.optim.RMSprop,
                   "optimizer_kwargs": {"alpha": 0.99, "eps": model.rms_prop_eps, "weight_decay": 0}}
         pk = _serialized(kwargs, "<class 'dict'>")
         pk.update(net_arch=kwargs["net_arch"], optimizer_class=str(torch.optim.RMSprop), optimizer_kwargs=kwargs["optimizer_kwargs"])
@@ -195,6 +212,7 @@ def _torch_bytes(obj) -> bytes:
 
 def write_zip(path: str, model) -> None:
     a2c = getattr(model, "algorithm", "ppo") == "a2c"
+    hid = getattr(model, "hidden", H)
     if a2c:
         hyper = {"learning_rate": model.lr, "n_steps": model.n_steps, "gamma": model.gamma, "gae_lambda": model.gae_lambda,
                  "ent_coef": model.ent_coef, "vf_coef": model.vf_coef, "max_grad_norm": model.max_grad_norm,
@@ -204,16 +222,16 @@ def write_zip(path: str, model) -> None:
                  "gamma": model.gamma, "gae_lambda": model.gae_lambda, "clip_range": model.clip_range, "ent_coef": model.ent_coef,
                  "vf_coef": model.vf_coef, "max_grad_norm": model.max_grad_norm}
     meta = {"format": "three-mlagents_b200/2", "algorithm": "a2c" if a2c else "ppo", "task_id": model.env.task_id, "obs_dim": model.obs_dim,
-            "n_actions": model.n_actions, "net_arch": {"pi": [256, 256], "vf": [256, 256]}, "seed": model.seed,
+            "n_actions": model.n_actions, "net_arch": {"pi": [hid, hid], "vf": [hid, hid]}, "seed": model.seed,
             "num_timesteps": model.num_timesteps, "n_updates": model.n_updates,
             **({"opt_step": model._opt_step} if a2c else {"adam_step": model._adam_step}), "mlp_impl": model.mlp_impl, "hyper": hyper}
     if a2c:
-        opt_sd = rmsprop_state_dict(model.sq_avg, model._opt_step, hyper, model.obs_dim, model.n_actions)
+        opt_sd = rmsprop_state_dict(model.sq_avg, model._opt_step, hyper, model.obs_dim, model.n_actions, hid)
     else:
-        opt_sd = adam_state_dict(model.m, model.v, model._adam_step, hyper, model.obs_dim, model.n_actions)
+        opt_sd = adam_state_dict(model.m, model.v, model._adam_step, hyper, model.obs_dim, model.n_actions, hid)
     with zipfile.ZipFile(path, "w") as z:
         z.writestr("data", json.dumps(build_data(model), indent=4))
-        z.writestr("policy.pth", _torch_bytes(flat_to_state_dict(model.params, model.obs_dim, model.n_actions)))
+        z.writestr("policy.pth", _torch_bytes(flat_to_state_dict(model.params, model.obs_dim, model.n_actions, hid)))
         z.writestr("policy.optimizer.pth", _torch_bytes(opt_sd))
         z.writestr("pytorch_variables.pth", _torch_bytes({}))
         z.writestr("_stable_baselines3_version", SB3_VERSION)
@@ -222,8 +240,8 @@ def write_zip(path: str, model) -> None:
 
 
 def read_zip(path: str) -> dict:
-    """-> {params, adam_m, adam_v, adam_step, sq_avg, opt_step, optimizer, meta (or None), data} for a zip written by this backend
-    or by SB3.  optimizer: "adam" (exp_avg / exp_avg_sq: PPO), "rmsprop" (square_avg: A2C) or None (no optimizer state);
+    """-> {params, adam_m, adam_v, adam_step, sq_avg, opt_step, optimizer, meta (or None), data, obs_dim, n_actions, hidden} for a
+    zip written by this backend or by SB3 (hidden: the width read off the policy's hidden layers).  optimizer: "adam" (exp_avg / exp_avg_sq: PPO), "rmsprop" (square_avg: A2C) or None (no optimizer state);
     sq_avg / opt_step are RMSprop's state (None / 0 for Adam)."""
     with zipfile.ZipFile(path) as z:
         names = set(z.namelist())
@@ -234,7 +252,8 @@ def read_zip(path: str) -> dict:
         data = json.loads(z.read("data")) if "data" in names else {}
         obs_dim = int(sd["mlp_extractor.policy_net.0.weight"].shape[1])
         n_actions = int(sd["action_net.weight"].shape[0])
-        flat = state_dict_to_flat(sd, obs_dim, n_actions)
+        hidden = hidden_width(sd)
+        flat = state_dict_to_flat(sd, obs_dim, n_actions, hidden)
         m, v, step = torch.zeros_like(flat), torch.zeros_like(flat), 0
         sq, opt_step, kind = None, 0, None
         if "policy.optimizer.pth" in names:
@@ -242,7 +261,7 @@ def read_zip(path: str) -> dict:
             st = opt.get("state", {})
             kind = _optimizer_kind(opt)
             if len(st) == 12:
-                layout = param_layout(obs_dim, n_actions)
+                layout = param_layout(obs_dim, n_actions, hidden)
                 cat = lambda key: torch.cat([torch.as_tensor(st[i][key]).float().reshape(-1) for i in range(12)])
                 if kind == "rmsprop":
                     sq, opt_step = cat("square_avg"), int(float(st[0]["step"]))
@@ -252,7 +271,7 @@ def read_zip(path: str) -> dict:
                     step = int(float(st[0]["step"]))
                     assert m.numel() == sum(int(np.prod(s)) for _, s in layout)
     return {"params": flat, "adam_m": m, "adam_v": v, "adam_step": step, "sq_avg": sq, "opt_step": opt_step, "optimizer": kind,
-            "meta": meta, "data": data, "obs_dim": obs_dim, "n_actions": n_actions}
+            "meta": meta, "data": data, "obs_dim": obs_dim, "n_actions": n_actions, "hidden": hidden}
 
 
 def _optimizer_kind(opt_state_dict: dict) -> str | None:
