@@ -379,7 +379,8 @@ int tmla_tc_debug(int swap_lbo_sbo);
  *   grads float[num_params] OVERWRITTEN;  scratch bf16[tmla_ppo_minibatch_scratch(hidden, rows)] (tile images);
  *   stats_out float[8] as tmla_ppo_loss;  logits_out float[rows,A] / values_out float[rows]: optional (NULL);
  *   flags: TMLA_MB_GRADS_ZEROED — the caller guarantees grads is all zeros (tmla_adam_clip_zero left it so): no memset;
- *          TMLA_MB_ACCUMULATE_STATS — stats_out is added to instead of overwritten (a running sum over minibatches).
+ *          TMLA_MB_ACCUMULATE_STATS — stats_out is added to instead of overwritten (a running sum over minibatches);
+ *          TMLA_MB_DETERMINISTIC — bit-reproducible sums (see "deterministic mode" below; needs the larger scratch).
  * tmla_ppo_minibatch_supported: 1 when the fused path covers (obs_dim, hidden, n_actions) — ball3d, gridworld,
  * push, walljump, bicycle at hidden 256; callers use the three-call sequence otherwise (basic: obs_dim 21, 3 actions; every
  * shape at hidden 64 / 128, where it returns 0). */
@@ -414,6 +415,35 @@ int tmla_tc_probe(const void *A, const void *B, float *out, int mode, void *stre
  * [0,n)?  out8 = DEVICE uint64[8] cycle counts {MMAs alone, loads alone, MMAs with loads running, loads under queued MMAs,
  * cycles the issuing lane spent inside the tcgen05.mma instructions, -, -, -}  (profiles/tc_overlap.py) */
 int tmla_tc_overlap_probe(uint64_t *out8, int n, int n_mma, int n_ld, void *stream);
+
+/* ---- deterministic mode ---------------------------------------------------------------------------------------------------
+ * The default update kernels finish their sums over rows with float atomics, so their last bits depend on scheduling.  The
+ * forms below compute the same quantities, but every CTA stores its partial sum in a scratch row of its own and one more launch
+ * adds the rows in CTA order: two calls on the same inputs (same build, same GPU model) give bit-identical results.
+ *   TMLA_MB_DETERMINISTIC (flags of tmla_ppo_minibatch_bf16 / tmla_a2c_batch_bf16): scratch then holds the
+ *       tmla_ppo_minibatch_scratch(hidden, rows) bf16 tile-image elements followed by tmla_det_scratch_bytes(...) bytes of partials;
+ *   tmla_mlp_backward_bf16_det, tmla_ppo_loss_det, tmla_a2c_loss_det: as their default forms plus `partials`, a device buffer of
+ *       tmla_det_scratch_bytes(obs_dim, hidden, n_actions, rows) bytes (one size serves every call of up to `rows` rows: it never
+ *       decreases as rows grow);
+ *   tmla_adv_stats_batched_det: as tmla_adv_stats_batched plus `partials` of tmla_adv_stats_det_scratch_bytes(total, mb_rows)
+ *       bytes (a single batch: mb_rows = total).
+ * Not covered: the float32 256-wide path (tmla_mlp_backward's split-K GEMM) and the gradient exchange between ranks. */
+#define TMLA_MB_DETERMINISTIC 4
+int64_t tmla_det_scratch_bytes(int obs_dim, int hidden, int n_actions, int64_t rows);
+int64_t tmla_adv_stats_det_scratch_bytes(int64_t total, int64_t mb_rows);
+int tmla_mlp_backward_bf16_det(const float *params, const void *wpack, int obs_dim, int hidden, int n_actions, const float *x,
+                               const int32_t *index, int64_t rows, const void *act_cache, const float *dlogits,
+                               const float *dvalues, float *grads, void *scratch, void *partials, void *stream);
+int tmla_adv_stats_batched_det(const float *advantages, const int32_t *index, int64_t total, int64_t mb_rows, double *adv_sums,
+                               void *partials, void *stream);
+int tmla_ppo_loss_det(const float *logits, const float *values, const int32_t *actions, const float *advantages,
+                      const float *old_logp, const float *returns, const int32_t *index, int64_t rows, int64_t global_rows,
+                      int n_actions, const double *adv_sums, int normalize_advantage, float clip_range, float ent_coef,
+                      float vf_coef, float *dlogits, float *dvalues, float *stats_out, void *partials, void *stream);
+int tmla_a2c_loss_det(const float *logits, const float *values, const int32_t *actions, const float *advantages, const float *returns,
+                      const int32_t *index, int64_t rows, int64_t global_rows, int n_actions, const double *adv_sums,
+                      int normalize_advantage, float ent_coef, float vf_coef, float *dlogits, float *dvalues, float *stats_out,
+                      void *partials, void *stream);
 
 #ifdef __cplusplus
 }

@@ -68,20 +68,24 @@ class CudaA2C(CudaPPO):
         nvtx.range_push("update")
         sums = None
         if self.normalize_advantage and total * self.world > 1:
-            sums = ops.adv_stats(self.adv, None, total, self.adv_sums[0])
+            if self.deterministic:         # the whole rollout as one batch of the block-ordered batched statistics
+                sums = ops.adv_stats_batched(self.adv, None, total, total, self.adv_sums, partials=self.adv_partials)[0]
+            else:
+                sums = ops.adv_stats(self.adv, None, total, self.adv_sums[0])
             allreduce_sum_(self.adv_sums)
         common = dict(rows=total, global_rows=total * self.world, adv_sums=sums, normalize=sums is not None, ent_coef=self.ent_coef,
                       vf_coef=self.vf_coef)
         if self.fused_update:              # the optimizer step below leaves the gradient zeroed
             ops.a2c_batch(self.params, self.wpack, obs_flat, D, A, self.act, self.adv, self.ret, grads=self.grads,
-                          scratch=self.scratch_mb, stats=self.stats_acc, grads_zeroed=True, **common)
+                          scratch=self.scratch_mb, stats=self.stats_acc, grads_zeroed=True, deterministic=self.deterministic, **common)
         else:
             ops.mlp_forward(self.params, obs_flat, D, A, rows=total, logits=self.logits_mb, values=self.values_mb,
                             act_cache=self.cache_mb, wpack=self.wpack, hidden=self.hidden)
             ops.a2c_loss(self.logits_mb, self.values_mb, self.act, self.adv, self.ret, dlogits=self.dlogits, dvalues=self.dvalues,
-                         stats=self.stats_acc, **common)
+                         stats=self.stats_acc, partials=self.det_partials, **common)
             ops.mlp_backward(self.params, obs_flat, D, A, self.cache_mb, self.dlogits, self.dvalues, rows=total, grads=self.grads,
-                             scratch=self.scratch_mb, wpack=self.wpack, hidden=self.hidden)
+                             scratch=self.scratch_mb, wpack=self.wpack, hidden=self.hidden,
+                             partials=self.det_partials if self.wpack is not None else None)
         self._opt_step += 1
         opt = dict(max_grad_norm=self.max_grad_norm, lr=self.lr, alpha=RMSPROP_ALPHA, eps=self.rms_prop_eps, norm_out=self.norm_out,
                    zero_grads=True)

@@ -17,7 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIB_DIR, "libtmla.so")
-SOURCES = ["error.cu", "env_kernels.cu", "rollout.cu", "comm.cu", "ppo_kernels.cu", "mlp_kernels.cu", "mlp_small.cu", "mlp_tc.cu", "mlp_fwd_pipe.cu", "mlp_train.cu"]
+SOURCES = ["error.cu", "env_kernels.cu", "rollout.cu", "comm.cu", "ppo_kernels.cu", "mlp_kernels.cu", "mlp_small.cu", "mlp_tc.cu", "mlp_fwd_pipe.cu", "mlp_train.cu", "det_reduce.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",

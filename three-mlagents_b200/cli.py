@@ -1,6 +1,7 @@
 """`three-mlagents` command line — same sub-commands, flags and JSON outputs as
 backend/mlagents/cli.py:13-95 (`list [--trainable-only]`, `inspect <task>`,
-`train <task> [-a ALGO] [-t N] [--seed] [--n-envs] [--eval-episodes] [--eval-freq] [--run-name] [--quiet]`,
+`train <task> [-a ALGO] [-t N] [--seed] [--n-envs] [--eval-episodes] [--eval-freq] [--run-name] [--quiet]`
+(plus `--deterministic`: bit-for-bit repeatable training, torch.use_deterministic_algorithms(True)),
 `evaluate <task> <model> [--episodes] [--seed] [--stochastic]`), running on the CUDA backend.
 
     python -m three_mlagents_b200.cli train basic -a ppo -t 25000 --seed 1
@@ -31,6 +32,8 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--eval-freq", type=int, default=10_000)
     p.add_argument("--run-name")
     p.add_argument("--quiet", action="store_true")
+    p.add_argument("--deterministic", action="store_true",
+                   help="bit-for-bit repeatable training for a fixed seed (torch.use_deterministic_algorithms(True))")
     p = sub.add_parser("evaluate", help="Evaluate a saved policy zip")
     p.add_argument("task")
     p.add_argument("model")
@@ -54,6 +57,10 @@ def main(argv: list[str] | None = None) -> None:
     elif args.command == "train":
         from .training import TrainConfig, train_task
 
+        if args.deterministic:
+            import torch
+
+            torch.use_deterministic_algorithms(True)
         result = train_task(TrainConfig(task_id=args.task, total_timesteps=args.timesteps, algorithm=args.algorithm,
                                         seed=args.seed, n_envs=args.n_envs, eval_episodes=args.eval_episodes,
                                         eval_freq=args.eval_freq, run_name=args.run_name, verbose=0 if args.quiet else 1))

@@ -25,6 +25,22 @@ static inline MlpOffsets mlp_offsets(int D, int A, int64_t H = 256) {      // H:
 }
 
 
+// ---- deterministic mode (TMLA_MB_DETERMINISTIC and the *_det entry points): instead of a float atomic, CTA b of a reducing
+// kernel stores its partial in row b of a partial buffer (rows of a compile-time stride), and det_reduce_launch sums the rows
+// of every segment in row order (det_reduce.cu).  One segment = `len` consecutive values of each of `nrows` rows.
+struct DetSeg {
+    const float *src;             // row 0 of the partials
+    int64_t stride;               // floats between rows
+    int nrows, len;
+    float *dst;                   // dst[i] += sum of rows (or = with `assign`)
+    const float *src2;            // optional second partial set summed after the first (two towers' statistics), else NULL
+    int64_t stride2;
+    int nrows2, assign;
+};
+static constexpr int kDetMaxSegs = 12;
+int det_reduce_launch(const DetSeg *segs, int nseg, cudaStream_t st);
+// partial row of one CTA of the fused tower kernel (mlp_train.cu): W1 | b1 | b2 | Wh | bh | statistics (8)
+__host__ __device__ constexpr int64_t det_tower_row(int D, int NOUT, int H = 256) { return (int64_t)H * D + 2 * H + (int64_t)NOUT * H + NOUT + 8; }
 // squared-norm partials of clip_grad_norm_: one per CTA of the norm pass, summed in a fixed order by every CTA of the Adam kernel
 #define TMLA_NORM_BLOCKS 128
 // ppo_kernels.cu: clip + Adam launch shared with the fused all-reduce (comm.cu)

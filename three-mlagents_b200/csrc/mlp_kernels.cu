@@ -26,6 +26,11 @@ __device__ __forceinline__ void act_store(__nv_bfloat16 *p, int64_t i, float v) 
 int tc_linear_launch(int epi, const void *A, const void *W, const float *bias, const void *aux, void *out, int64_t M,
                      const int32_t *rows_dev, cudaStream_t st);
 int tc_wgrad_launch(const void *X, const void *Y, float *G, int64_t rows, cudaStream_t st);
+int64_t tc_wgrad_det_planes(int64_t rows);
+int tc_wgrad_det_launch(const void *X, const void *Y, float *planes, int64_t rows, cudaStream_t st);
+// deterministic-mode partials of the fused batch (mlp_train.cu) and of the loss statistics (ppo_kernels.cu), in bytes
+int64_t fused_det_scratch_bytes(int obs_dim, int hidden, int n_actions, int64_t rows);
+int64_t loss_det_scratch_bytes(int64_t rows);
 int tc_pack_w2_launch(const float *w2, void *w, void *wt, void *img, cudaStream_t st);
 int tc_tower_forward_dual_launch(int D, int n_actions, const float *const *W1, const float *const *B1, const void *const *W2,
                                  const float *const *B2, const float *const *Wh, const float *const *Bh, const float *x,
@@ -46,6 +51,9 @@ int small_mlp_backward(const float *params, int D, int hidden, int A, const floa
                        cudaStream_t st);
 
 #include "mlp_common.cuh"
+
+// rows per block of the backward's reduction kernels: ~4 blocks per SM, at least 64 rows
+static int backward_rows_per_block(int64_t rows) { return (int)std::max<int64_t>(64, ceil_div64(ceil_div64(rows, 148 * 4), 64) * 64); }
 
 __device__ __forceinline__ int64_t eff_rows(int64_t rows, const int32_t *rows_dev) {
     return rows_dev ? min(rows, (int64_t)*rows_dev) : rows;
@@ -83,7 +91,9 @@ l1_forward_kernel(const float *__restrict__ W1, const float *__restrict__ b1, co
 }
 
 // dW1[j][k] = sum_r dZ1[r][j] x[r][k], db1[j] = sum_r dZ1[r][j]
-template <int D, typename AT>
+// DET (deterministic mode, every kernel below): no atomics — block b stores its sums in row b of the partials (rows of
+// H*D + H floats here: dW1 | db1; dW1 / db1 point into row 0), det_reduce_kernel adds the rows in order
+template <int D, typename AT, bool DET = false>
 __global__ void __launch_bounds__(H)
 l1_backward_kernel(const AT *__restrict__ dz1, const float *__restrict__ x, const int32_t *__restrict__ index,
                    int64_t rows, int rows_per_block, float *__restrict__ dW1, float *__restrict__ db1) {
@@ -109,6 +119,13 @@ l1_backward_kernel(const AT *__restrict__ dz1, const float *__restrict__ x, cons
 #pragma unroll
             for (int k = 0; k < D; ++k) acc[k] = fmaf(g, sx[r][k], acc[k]);
         }
+    }
+    if constexpr (DET) {
+        const int64_t row = (int64_t)blockIdx.x * (H * D + H);
+#pragma unroll
+        for (int k = 0; k < D; ++k) dW1[row + j * D + k] = acc[k];
+        db1[row + j] = accb;
+        return;
     }
 #pragma unroll
     for (int k = 0; k < D; ++k) atomicAdd(dW1 + j * D + k, acc[k]);
@@ -334,7 +351,7 @@ l1_forward_bf16_kernel(const float *__restrict__ W1, const float *__restrict__ b
 
 // dW1[j][k] += sum_r dZ1[r][j] x[r][k],  db1[j] += sum_r dZ1[r][j]
 // dZ1 rows stream through the cp.async pipe; the gathered obs row rides along as the slot's aux floats.
-template <int D>
+template <int D, bool DET = false>
 __global__ void __launch_bounds__(256)
 l1_backward_bf16_kernel(const __nv_bfloat16 *__restrict__ dz1, const float *__restrict__ x, const int32_t *__restrict__ index,
                         int64_t rows, int rows_per_block, float *__restrict__ dW1, float *__restrict__ db1) {
@@ -388,6 +405,13 @@ l1_backward_bf16_kernel(const __nv_bfloat16 *__restrict__ dz1, const float *__re
         for (int c = 0; c < 8; ++c) acc[D][c] += g[c];
     }
     asm volatile("cp.async.wait_group 0;" ::: "memory");
+    if constexpr (DET) {                                   // rows of H*D + H floats: dW1 | db1
+        const int64_t row = (int64_t)blockIdx.x * (H * D + H);
+#pragma unroll
+        for (int k = 0; k < D; ++k) reduce_planes(sh, acc[k], [&](int j, float s) { dW1[row + j * D + k] = s; });
+        reduce_planes(sh, acc[D], [&](int j, float s) { db1[row + j] = s; });
+        return;
+    }
 #pragma unroll
     for (int k = 0; k < D; ++k) reduce_planes(sh, acc[k], [&](int j, float s) { atomicAdd(dW1 + j * D + k, s); });
     reduce_planes(sh, acc[D], [&](int j, float s) { atomicAdd(db1 + j, s); });
@@ -395,7 +419,7 @@ l1_backward_bf16_kernel(const __nv_bfloat16 *__restrict__ dz1, const float *__re
 
 //   dZ2[r][j] = (sum_a dOut[r][a] Wh[a][j]) * (1 - h2[r][j]^2) ; dWh[a][j] += dOut[r][a] h2[r][j] ; db2[j] += dZ2[r][j] ; dbh[a] += dOut[r][a]
 // h2 rows (and the dOut row as aux) stream through the cp.async pipe.
-template <int NOUT>
+template <int NOUT, bool DET = false>
 __global__ void __launch_bounds__(256)
 head_backward_bf16_kernel(const float *__restrict__ Wh, const __nv_bfloat16 *__restrict__ h2, const float *__restrict__ dout,
                           int64_t rows, int rows_per_block, __nv_bfloat16 *__restrict__ dz2, float *__restrict__ dWh,
@@ -445,6 +469,24 @@ head_backward_bf16_kernel(const float *__restrict__ Wh, const __nv_bfloat16 *__r
         reinterpret_cast<uint4 *>(dz2 + (rb + warp + 8 * (int64_t)i) * H)[lane] = pack8(g);
     }
     asm volatile("cp.async.wait_group 0;" ::: "memory");
+    if constexpr (DET) {                                   // rows of NOUT*H + NOUT + H floats: dWh | dbh | db2
+        const int64_t row = (int64_t)blockIdx.x * (NOUT * H + NOUT + H);
+#pragma unroll
+        for (int a = 0; a < NOUT; ++a) reduce_planes(sh, accw[a], [&](int j, float s) { dWh[row + a * H + j] = s; });
+        reduce_planes(sh, accb2, [&](int j, float s) { db2[row + j] = s; });
+        __syncthreads();
+        if (lane == 0)
+#pragma unroll
+            for (int a = 0; a < NOUT; ++a) sh[warp][a] = accbh[a];
+        __syncthreads();
+        if (threadIdx.x < NOUT) {
+            float t = 0.0f;
+#pragma unroll
+            for (int w = 0; w < 8; ++w) t += sh[w][threadIdx.x];
+            dbh[row + threadIdx.x] = t;
+        }
+        return;
+    }
 #pragma unroll
     for (int a = 0; a < NOUT; ++a) reduce_planes(sh, accw[a], [&](int j, float s) { atomicAdd(dWh + a * H + j, s); });
     reduce_planes(sh, accb2, [&](int j, float s) { atomicAdd(db2 + j, s); });
@@ -631,6 +673,9 @@ static int ensure_pipe_attrs() {
     PIPE_ATTR(head_backward_bf16_kernel<1>); PIPE_ATTR(head_backward_bf16_kernel<3>); PIPE_ATTR(head_backward_bf16_kernel<4>);
     PIPE_ATTR(head_backward_bf16_kernel<5>);
     PIPE_ATTR(l1_backward_bf16_kernel<4>); PIPE_ATTR(l1_backward_bf16_kernel<6>);
+    PIPE_ATTR((head_backward_bf16_kernel<1, true>)); PIPE_ATTR((head_backward_bf16_kernel<3, true>));   // deterministic forms
+    PIPE_ATTR((head_backward_bf16_kernel<4, true>)); PIPE_ATTR((head_backward_bf16_kernel<5, true>));
+    PIPE_ATTR((l1_backward_bf16_kernel<4, true>)); PIPE_ATTR((l1_backward_bf16_kernel<6, true>));
 #undef PIPE_ATTR
     done = 1;
     return TMLA_OK;
@@ -732,7 +777,7 @@ static int mlp_backward_impl(const float *params, const void *wpack, int obs_dim
     TMLA_CUDA(cudaMemsetAsync(grads, 0, sizeof(float) * o.total, st));
     AT *dz2 = scratch, *dz1 = scratch + rows * H;
     // chunk rows so that ~4 blocks per SM share the reduction kernels
-    const int rpb = (int)std::max<int64_t>(64, ceil_div64(ceil_div64(rows, 148 * 4), 64) * 64);
+    const int rpb = backward_rows_per_block(rows);
     const unsigned gr = (unsigned)ceil_div64(rows, rpb);
     for (int t = 0; t < 2; ++t) {
         const AT *h1 = act_cache + (int64_t)(2 * t) * rows * H, *h2 = act_cache + (int64_t)(2 * t + 1) * rows * H;
@@ -783,6 +828,76 @@ static int mlp_backward_impl(const float *params, const void *wpack, int obs_dim
         TMLA_LAUNCH_CHECK();
     }
     return TMLA_OK;
+}
+
+// Deterministic form of the bf16 backward: the same kernels and block split, every atomic replaced by a partial row per block
+// (a 256x256 plane per weight-gradient CTA), then one det_reduce launch.  Partials (floats), per tower t:
+//   W2 planes [2][P] | head rows [2][gr][A_t*H + A_t + H] | layer-1 rows [2][gr][H*D + H]     (P = tc_wgrad_det_planes(rows))
+struct BackwardDetLayout {
+    int64_t planes, gr, head[2], l1, w2_off[2], head_off[2], l1_off[2], total;
+};
+static BackwardDetLayout backward_det_layout(int D, int A, int64_t planes, int64_t gr) {
+    BackwardDetLayout L;
+    L.planes = planes; L.gr = gr;
+    L.head[0] = (int64_t)A * H + A + H; L.head[1] = H + 1 + H; L.l1 = (int64_t)H * D + H;
+    int64_t p = 0;
+    for (int t = 0; t < 2; ++t) { L.w2_off[t] = p; p += planes * H * H; }
+    for (int t = 0; t < 2; ++t) { L.head_off[t] = p; p += gr * L.head[t]; }
+    for (int t = 0; t < 2; ++t) { L.l1_off[t] = p; p += gr * L.l1; }
+    L.total = p;
+    return L;
+}
+static int64_t backward_det_bytes(int D, int A, int64_t rows) {     // monotone in rows: upper bounds of the block counts
+    const int64_t gr_max = std::min<int64_t>(ceil_div64(rows, 64), 148 * 4);
+    return 4 * backward_det_layout(D, A, tc_wgrad_det_planes(rows), gr_max).total;
+}
+
+static int mlp_backward_bf16_det(const float *params, const void *wpack, int obs_dim, int n_actions, const float *x, const int32_t *index,
+                                 int64_t rows, const __nv_bfloat16 *act_cache, const float *dlogits, const float *dvalues, float *grads,
+                                 __nv_bfloat16 *scratch, float *part, cudaStream_t st) {
+    int rc = ensure_pipe_attrs();
+    if (rc) return rc;
+    const MlpOffsets o = mlp_offsets(obs_dim, n_actions);
+    TMLA_CUDA(cudaMemsetAsync(grads, 0, sizeof(float) * o.total, st));
+    __nv_bfloat16 *dz2 = scratch, *dz1 = scratch + rows * H;
+    const int rpb = backward_rows_per_block(rows);
+    const unsigned gr = (unsigned)ceil_div64(rows, rpb);
+    const BackwardDetLayout L = backward_det_layout(obs_dim, n_actions, tc_wgrad_det_planes(rows), gr);
+    for (int t = 0; t < 2; ++t) {
+        const __nv_bfloat16 *h1 = act_cache + (int64_t)(2 * t) * rows * H, *h2 = act_cache + (int64_t)(2 * t + 1) * rows * H;
+        const float *dout = t == 0 ? dlogits : dvalues;
+        const int nout = o.nout[t];
+        float *hw = part + L.head_off[t], *hb = hw + nout * H, *hb2 = hb + nout;        // row 0: dWh | dbh | db2
+        const float *wh = params + o.wh[t];
+        if (t == 1) head_backward_bf16_kernel<1, true><<<gr, 256, kPipeSmem, st>>>(wh, h2, dout, rows, rpb, dz2, hw, hb, hb2);
+        else if (n_actions == 3) head_backward_bf16_kernel<3, true><<<gr, 256, kPipeSmem, st>>>(wh, h2, dout, rows, rpb, dz2, hw, hb, hb2);
+        else if (n_actions == 4) head_backward_bf16_kernel<4, true><<<gr, 256, kPipeSmem, st>>>(wh, h2, dout, rows, rpb, dz2, hw, hb, hb2);
+        else head_backward_bf16_kernel<5, true><<<gr, 256, kPipeSmem, st>>>(wh, h2, dout, rows, rpb, dz2, hw, hb, hb2);
+        TMLA_LAUNCH_CHECK();
+        const __nv_bfloat16 *w2t = reinterpret_cast<const __nv_bfloat16 *>(wpack) + (int64_t)(2 * t + 1) * H * H;
+        rc = tc_linear_launch(1, dz2, w2t, nullptr, h1, dz1, rows, nullptr, st);
+        if (rc) return rc;
+        rc = tc_wgrad_det_launch(dz2, h1, part + L.w2_off[t], rows, st);
+        if (rc) return rc;
+        float *lw = part + L.l1_off[t], *lb = lw + H * obs_dim;                       // row 0: dW1 | db1
+#define L1B(DD) l1_backward_kernel<DD, __nv_bfloat16, true><<<gr, H, 0, st>>>(dz1, x, index, rows, rpb, lw, lb)
+        if (obs_dim == 4) l1_backward_bf16_kernel<4, true><<<gr, 256, kPipeSmem, st>>>(dz1, x, index, rows, rpb, lw, lb);
+        else if (obs_dim == 6) l1_backward_bf16_kernel<6, true><<<gr, 256, kPipeSmem, st>>>(dz1, x, index, rows, rpb, lw, lb);
+        else if (obs_dim == 45) L1B(45); else if (obs_dim == 7) L1B(7); else if (obs_dim == 16) L1B(16); else L1B(21);
+#undef L1B
+        TMLA_LAUNCH_CHECK();
+    }
+    DetSeg sg[kDetMaxSegs];
+    int n = 0;
+    const int g = (int)gr;
+    for (int t = 0; t < 2; ++t) {
+        const int nout = o.nout[t];
+        sg[n++] = DetSeg{part + L.w2_off[t], H * H, (int)L.planes, H * H, grads + o.w2[t], nullptr, 0, 0, 0};
+        sg[n++] = DetSeg{part + L.head_off[t], L.head[t], g, nout * H + nout, grads + o.wh[t], nullptr, 0, 0, 0};     // Wh | bh
+        sg[n++] = DetSeg{part + L.head_off[t] + nout * H + nout, L.head[t], g, H, grads + o.b2[t], nullptr, 0, 0, 0};
+        sg[n++] = DetSeg{part + L.l1_off[t], L.l1, g, (int)L.l1, grads + o.w1[t], nullptr, 0, 0, 0};             // W1 | b1
+    }
+    return det_reduce_launch(sg, n, st);
 }
 
 extern "C" {
@@ -865,6 +980,24 @@ int tmla_mlp_backward_bf16(const float *params, const void *wpack, int obs_dim, 
     if (rc) return rc;
     return mlp_backward_impl<__nv_bfloat16>(params, wpack, obs_dim, n_actions, x, index, rows, (const __nv_bfloat16 *)act_cache,
                                             dlogits, dvalues, grads, (__nv_bfloat16 *)scratch, (cudaStream_t)stream);
+}
+
+int tmla_mlp_backward_bf16_det(const float *params, const void *wpack, int obs_dim, int hidden, int n_actions, const float *x,
+                               const int32_t *index, int64_t rows, const void *act_cache, const float *dlogits,
+                               const float *dvalues, float *grads, void *scratch, void *partials, void *stream) {
+    TMLA_REQUIRE(params && wpack && x && act_cache && dlogits && dvalues && grads && scratch && partials, "NULL buffer");
+    TMLA_REQUIRE(rows > 0, "rows must be positive");
+    int rc = check_shape(obs_dim, hidden, n_actions);
+    if (rc) return rc;
+    return mlp_backward_bf16_det(params, wpack, obs_dim, n_actions, x, index, rows, (const __nv_bfloat16 *)act_cache, dlogits, dvalues,
+                                 grads, (__nv_bfloat16 *)scratch, (float *)partials, (cudaStream_t)stream);
+}
+
+int64_t tmla_det_scratch_bytes(int obs_dim, int hidden, int n_actions, int64_t rows) {
+    if (rows <= 0) { tmla_set_error("rows must be positive"); return TMLA_EINVAL; }
+    int64_t b = loss_det_scratch_bytes(rows);
+    if (hidden == H && check_shape(obs_dim, hidden, n_actions) == TMLA_OK) b = std::max(b, backward_det_bytes(obs_dim, n_actions, rows));
+    return std::max(b, fused_det_scratch_bytes(obs_dim, hidden, n_actions, rows));
 }
 
 // bf16 copies of the two hidden-layer weights per tower: wpack = [pi.W2, pi.W2^T, vf.W2, vf.W2^T, pi.W2 image, vf.W2 image],

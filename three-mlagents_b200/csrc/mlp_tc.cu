@@ -196,6 +196,8 @@ __device__ __forceinline__ void store_block_transposed(uint8_t *dst, const uint4
     }
 }
 
+// DET: G is an array of 256x256 partial planes, CTA b stores its split-K share in plane b (summed in order by det_reduce_kernel)
+template <bool DET = false>
 __global__ void __launch_bounds__(256, 1)
 tc_wgrad_kernel(const __nv_bfloat16 *__restrict__ X, const __nv_bfloat16 *__restrict__ Y, float *__restrict__ G, int64_t rows) {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -280,11 +282,13 @@ tc_wgrad_kernel(const __nv_bfloat16 *__restrict__ X, const __nv_bfloat16 *__rest
         for (int i = 0; i < 16; ++i) {
             const int r = warp + 8 * i;
             float *grow = G + (int64_t)(mh * 128 + r) * H;
+            if constexpr (DET) grow += (int64_t)blockIdx.x * (H * H);
 #pragma unroll
             for (int hseg = 0; hseg < 2; ++hseg) {
                 const int ch = hseg * 32 + lane;
                 const float4 v = *reinterpret_cast<const float4 *>(smem + r * 1024 + ((ch ^ (r & 7)) << 4));
-                asm volatile("red.global.add.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(grow + ch * 4), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+                if constexpr (DET) *reinterpret_cast<float4 *>(grow + ch * 4) = v;
+                else asm volatile("red.global.add.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(grow + ch * 4), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
             }
         }
     }
@@ -545,7 +549,8 @@ static int ensure_attrs() {
     if (g_attr_done) return TMLA_OK;
     TMLA_CUDA(cudaFuncSetAttribute(tc_linear_kernel<EPI_BIAS_TANH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLinearSmem));
     TMLA_CUDA(cudaFuncSetAttribute(tc_linear_kernel<EPI_DTANH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLinearSmem));
-    TMLA_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgradSmem));
+    TMLA_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgradSmem));
+    TMLA_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgradSmem));
     g_attr_done = 1;
     return TMLA_OK;
 }
@@ -574,7 +579,16 @@ int tc_wgrad_launch(const void *X, const void *Y, float *G, int64_t rows, cudaSt
     int rc = ensure_attrs();
     if (rc) return rc;
     const unsigned grid = (unsigned)std::min<int64_t>((rows + kgRows - 1) / kgRows, sm_count());
-    tc_wgrad_kernel<<<grid, 256, kWgradSmem, st>>>((const __nv_bfloat16 *)X, (const __nv_bfloat16 *)Y, G, rows);
+    tc_wgrad_kernel<false><<<grid, 256, kWgradSmem, st>>>((const __nv_bfloat16 *)X, (const __nv_bfloat16 *)Y, G, rows);
+    TMLA_LAUNCH_CHECK();
+    return TMLA_OK;
+}
+// deterministic form: one partial plane per CTA into `planes` (tc_wgrad_det_planes(rows) of them, all written)
+int64_t tc_wgrad_det_planes(int64_t rows) { return std::min<int64_t>((rows + kgRows - 1) / kgRows, sm_count()); }
+int tc_wgrad_det_launch(const void *X, const void *Y, float *planes, int64_t rows, cudaStream_t st) {
+    int rc = ensure_attrs();
+    if (rc) return rc;
+    tc_wgrad_kernel<true><<<(unsigned)tc_wgrad_det_planes(rows), 256, kWgradSmem, st>>>((const __nv_bfloat16 *)X, (const __nv_bfloat16 *)Y, planes, rows);
     TMLA_LAUNCH_CHECK();
     return TMLA_OK;
 }

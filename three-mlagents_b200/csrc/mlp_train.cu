@@ -151,8 +151,8 @@ struct TowerTrainArgs {
     // outputs
     __nv_bfloat16 *h1_out, *dz2_out;    // ceil(M/128) tile images of 64 KB each (shared-memory operand layout), for the dW2 GEMM
     float *out;                          // optional [M][NOUT] head outputs (logits / values)
-    float *gW1, *gB1, *gB2, *gWh, *gBh;  // gradient slices (accumulated with atomics; caller zeroes)
-    float *stats;                        // float[8] (tmla_ppo_loss layout), accumulated
+    float *gW1, *gB1, *gB2, *gWh, *gBh;  // gradient slices (accumulated with atomics; caller zeroes) — DET: row 0 of the partials
+    float *stats;                        // float[8] (tmla_ppo_loss layout), accumulated — DET: row 0 of the partials
 };
 
 // small [rows][16] bf16 operand tiles: chunk (r, cb) at (r/8)*256 + cb*128 + (r%8)*16
@@ -185,7 +185,7 @@ struct TrainSmem {
 // policy gradient -(adv * log_prob).mean() (SB3 2.9.0 a2c.py), which has no ratio, no clip and reads no old log-probabilities
 enum { kLossPPO = 0, kLossA2C = 1 };
 
-template <int D, int NOUT, int LOSS = kLossPPO>
+template <int D, int NOUT, int LOSS = kLossPPO, bool DET = false>
 __global__ void __launch_bounds__(kTrainThreads + 32, 1)
 tc_tower_train_kernel(const __grid_constant__ TowerTrainArgs p) {
     using L = TrainSmem<D, NOUT>;
@@ -687,6 +687,49 @@ tc_tower_train_kernel(const __grid_constant__ TowerTrainArgs p) {
     // ---- flush: TMEM gradient accumulators (lane = hidden unit) -> one atomic per value; scalar sums
     // (rotating the order of the accumulator groups with the CTA index, so that 148 CTAs do not queue on one cache line, was
     // measured: no gain — 402.2 vs 401.3 us per minibatch — and, inlined, it raised the tile loop's spills: +15 us)
+    // DET: the gradient and statistics pointers address row 0 of the partial buffer; this CTA stores its sums in its own row
+    // (every value is owned by one thread, so plain stores), det_reduce_kernel adds the rows in order.
+    if constexpr (DET) {
+        if (warp < 4) {
+            const int64_t row = (int64_t)blockIdx.x * det_tower_row(D, NOUT);
+#pragma unroll
+            for (int mh = 0; mh < 2; ++mh) {
+                const int j = mh * 128 + rt;
+                uint32_t g[16];
+                tmem_ld16(lane_base + C_GWH + mh * 16, g);
+#pragma unroll
+                for (int a = 0; a < NOUT; ++a) p.gWh[row + a * H + j] = __uint_as_float(g[a]) + __uint_as_float(g[NOUT + a]);
+                tmem_ld16(lane_base + C_GB2 + mh * 16, g);
+                p.gB2[row + j] = __uint_as_float(g[2 * D]);
+                tmem_ld16(lane_base + C_GW1 + mh * 16, g);
+#pragma unroll
+                for (int k = 0; k < D; ++k) p.gW1[row + j * D + k] = __uint_as_float(g[k]) + __uint_as_float(g[D + k]);
+                p.gB1[row + j] = __uint_as_float(g[2 * D]);
+            }
+            if (warp == 0) {                               // the CTA's 128 per-row sums, rows l, l+32, l+64, l+96 per lane
+                float st_acc[4], dbh_acc[NOUT];
+                auto rows_sum = [&](int q) {
+                    return warp_sum_f(((racc[lane * L::RS + q] + racc[(lane + 32) * L::RS + q]) + racc[(lane + 64) * L::RS + q]) +
+                                      racc[(lane + 96) * L::RS + q]);
+                };
+#pragma unroll
+                for (int q = 0; q < 4; ++q) st_acc[q] = rows_sum(q) * p.inv_rows;
+#pragma unroll
+                for (int a = 0; a < NOUT; ++a) dbh_acc[a] = rows_sum(4 + a);
+                if (lane == 0) {
+#pragma unroll
+                    for (int a = 0; a < NOUT; ++a) p.gBh[row + a] = dbh_acc[a];
+                    float *st = p.stats + row;             // slots 0..5 of tmla_ppo_loss's layout; 6, 7 (row 0) as below
+                    if (PI) {
+                        st[0] = st_acc[0]; st[1] = 0.0f; st[2] = st_acc[1]; st[3] = st_acc[2]; st[4] = st_acc[3];
+                        st[5] = st_acc[0] + p.ent_coef * st_acc[1];
+                    } else {
+                        st[0] = 0.0f; st[1] = st_acc[0]; st[2] = 0.0f; st[3] = 0.0f; st[4] = 0.0f; st[5] = p.vf_coef * st_acc[0];
+                    }
+                }
+            }
+        }
+    } else
     if (warp < 4) {
 #pragma unroll
         for (int mh = 0; mh < 2; ++mh) {
@@ -757,6 +800,7 @@ static constexpr uint32_t kwStage = 2 * kwChunk;              // X and Y
 static constexpr int kwStages = 3;
 static constexpr uint32_t kWgradTiledSmem = kwStages * kwStage + 128;   // 196736 (>= the 128 KB epilogue stage)
 
+template <bool DET = false>
 __global__ void __launch_bounds__(256, 1)
 tc_wgrad_tiled_kernel(const __nv_bfloat16 *__restrict__ Xt0, const __nv_bfloat16 *__restrict__ Yt0, float *__restrict__ G0,
                       const __nv_bfloat16 *__restrict__ Xt1, const __nv_bfloat16 *__restrict__ Yt1, float *__restrict__ G1, int64_t nchunks,
@@ -782,6 +826,8 @@ tc_wgrad_tiled_kernel(const __nv_bfloat16 *__restrict__ Xt0, const __nv_bfloat16
     float *G = second ? G1 : G0;
     const int64_t first = dual ? (second ? before1 : (int64_t)blockIdx.x - before1) : blockIdx.x, stride = dual ? (second ? n1 : n0) : gridDim.x;
     if (first >= nchunks) return;
+    // DET: G0 / G1 are arrays of 256x256 partial planes, one per CTA of the problem (plane `first`), summed by det_reduce_kernel
+    if constexpr (DET) G += first * (H * H);
 
     if (warp == 0) tmem_alloc<512>(tmem_holder);
     if (tid == 32) {
@@ -868,7 +914,8 @@ tc_wgrad_tiled_kernel(const __nv_bfloat16 *__restrict__ Xt0, const __nv_bfloat16
             for (int hseg = 0; hseg < 2; ++hseg) {
                 const int ch = hseg * 32 + lane;
                 const float4 v = *reinterpret_cast<const float4 *>(smem + r * 1024 + ((ch ^ (r & 7)) << 4));
-                asm volatile("red.global.add.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(grow + ch * 4), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+                if constexpr (DET) *reinterpret_cast<float4 *>(grow + ch * 4) = v;
+                else asm volatile("red.global.add.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(grow + ch * 4), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
             }
         }
     }
@@ -1237,20 +1284,30 @@ static int wgrad_reverse() {      // TMLA_WGRAD_REV=0 restores front-to-back rea
     static const int r = [] { const char *e = getenv("TMLA_WGRAD_REV"); return (e && !strcmp(e, "0")) ? 0 : 1; }();
     return r;
 }
+// grid of the weight-gradient launch and the number n1 of its CTAs that work on problem 1 (0 for a single problem)
+static void wgrad_tiled_split(int64_t rows_padded, bool dual, unsigned *grid_out, int *n1_out) {
+    const int64_t nchunks = rows_padded / 64;
+    unsigned grid = (unsigned)std::min<int64_t>(dual ? 2 * nchunks : nchunks, sm_count_train());
+    if (dual) grid &= ~1u;
+    // share of the CTAs given to problem 1 (the tower that ran LAST: its image tail is L2-resident): TMLA_WGRAD_N1 per 148 CTAs
+    static const int n1_of_148 = [] { const char *e = getenv("TMLA_WGRAD_N1"); return e ? atoi(e) : 74; }();
+    *grid_out = grid;
+    *n1_out = dual ? std::max(1, std::min((int)grid - 1, (int)((int64_t)grid * n1_of_148 / 148))) : 0;
+}
+// DET: G and G1 receive one 256x256 partial plane per CTA of their problem (det_reduce_kernel sums them)
+template <bool DET = false>
 static int tc_wgrad_tiled_launch(const void *Xt, const void *Yt, float *G, int64_t rows_padded, cudaStream_t st,
                                  const void *Xt1 = nullptr, const void *Yt1 = nullptr, float *G1 = nullptr, bool overlap_prev = false) {
     static int attr_done = 0;
     if (!attr_done) {
-        TMLA_CUDA(cudaFuncSetAttribute(tc_wgrad_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgradTiledSmem));
+        TMLA_CUDA(cudaFuncSetAttribute(tc_wgrad_tiled_kernel<DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgradTiledSmem));
         attr_done = 1;
     }
     const int64_t nchunks = rows_padded / 64;
-    unsigned grid = (unsigned)std::min<int64_t>(Xt1 ? 2 * nchunks : nchunks, sm_count_train());
-    if (Xt1) grid &= ~1u;
-    // share of the CTAs given to problem 1 (the tower that ran LAST: its image tail is L2-resident): TMLA_WGRAD_N1 per 148 CTAs
-    static const int n1_of_148 = [] { const char *e = getenv("TMLA_WGRAD_N1"); return e ? atoi(e) : 74; }();
+    unsigned grid;
+    int n1;
+    wgrad_tiled_split(rows_padded, Xt1 != nullptr, &grid, &n1);
     static const int wgrad_hint = [] { const char *e = getenv("TMLA_WGRAD_HINT"); return e ? atoi(e) : 1; }();
-    int n1 = Xt1 ? std::max(1, std::min((int)grid - 1, (int)((int64_t)grid * n1_of_148 / 148))) : 0;
     if (overlap_prev) {                                    // programmatic dependent of the tower kernel before it (see tower_train_launch_t)
         cudaLaunchConfig_t cfg;
         memset(&cfg, 0, sizeof(cfg));
@@ -1259,10 +1316,10 @@ static int tc_wgrad_tiled_launch(const void *Xt, const void *Yt, float *G, int64
         attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr.val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = &attr; cfg.numAttrs = 1;
-        TMLA_CUDA(cudaLaunchKernelEx(&cfg, tc_wgrad_tiled_kernel, (const __nv_bfloat16 *)Xt, (const __nv_bfloat16 *)Yt, G, (const __nv_bfloat16 *)Xt1,
+        TMLA_CUDA(cudaLaunchKernelEx(&cfg, tc_wgrad_tiled_kernel<DET>, (const __nv_bfloat16 *)Xt, (const __nv_bfloat16 *)Yt, G, (const __nv_bfloat16 *)Xt1,
                                      (const __nv_bfloat16 *)Yt1, G1, nchunks, wgrad_reverse(), n1, wgrad_hint));
     } else {
-        tc_wgrad_tiled_kernel<<<grid, 256, kWgradTiledSmem, st>>>((const __nv_bfloat16 *)Xt, (const __nv_bfloat16 *)Yt, G,
+        tc_wgrad_tiled_kernel<DET><<<grid, 256, kWgradTiledSmem, st>>>((const __nv_bfloat16 *)Xt, (const __nv_bfloat16 *)Yt, G,
                                                                   (const __nv_bfloat16 *)Xt1, (const __nv_bfloat16 *)Yt1, G1, nchunks, wgrad_reverse(), n1, wgrad_hint);
     }
     TMLA_LAUNCH_CHECK();
@@ -1286,13 +1343,13 @@ static int wgrad_h1_launch_t(const WgradH1Problem &a, const WgradH1Problem &b, c
     return TMLA_OK;
 }
 
-template <int D, int NOUT, int LOSS = kLossPPO>
+template <int D, int NOUT, int LOSS = kLossPPO, bool DET = false>
 static int tower_train_launch_t(const TowerTrainArgs &a, cudaStream_t st, bool overlap_prev) {
     static int attr_done = 0;
     constexpr uint32_t smem = TrainSmem<D, NOUT>::total;
     static_assert(smem <= 232448, "fused tower training kernel exceeds the 227 KB shared-memory limit");
     if (!attr_done) {
-        TMLA_CUDA(cudaFuncSetAttribute(tc_tower_train_kernel<D, NOUT, LOSS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        TMLA_CUDA(cudaFuncSetAttribute(tc_tower_train_kernel<D, NOUT, LOSS, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_done = 1;
     }
     const unsigned grid = (unsigned)std::min<int64_t>((a.M + 127) / 128, sm_count_train());
@@ -1307,9 +1364,9 @@ static int tower_train_launch_t(const TowerTrainArgs &a, cudaStream_t st, bool o
         attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr.val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = &attr; cfg.numAttrs = 1;
-        TMLA_CUDA(cudaLaunchKernelEx(&cfg, tc_tower_train_kernel<D, NOUT, LOSS>, a));
+        TMLA_CUDA(cudaLaunchKernelEx(&cfg, tc_tower_train_kernel<D, NOUT, LOSS, DET>, a));
     } else {
-        tc_tower_train_kernel<D, NOUT, LOSS><<<grid, kTrainThreads + 32, smem, st>>>(a);
+        tc_tower_train_kernel<D, NOUT, LOSS, DET><<<grid, kTrainThreads + 32, smem, st>>>(a);
     }
     TMLA_LAUNCH_CHECK();
     return TMLA_OK;
@@ -1326,9 +1383,93 @@ int64_t tmla_ppo_minibatch_scratch(int hidden, int64_t rows) { return 4 * ((rows
 
 }  // extern "C"
 
+// TMLA_MB_DETERMINISTIC: partials (floats) after the tile images — one 256x256 weight-gradient plane per CTA of the
+// weight-gradient launch (at most one CTA per SM, over both towers), then one row per tower-kernel CTA and tower
+static int64_t fused_det_partials(int obs_dim, int n_actions, int64_t rows) {
+    const int64_t ctas = std::min<int64_t>((rows + 127) / 128, sm_count_train());
+    return (int64_t)sm_count_train() * H * H + ctas * (det_tower_row(obs_dim, n_actions) + det_tower_row(obs_dim, 1));
+}
+int64_t fused_det_scratch_bytes(int obs_dim, int hidden, int n_actions, int64_t rows) {
+    if (!tmla_ppo_minibatch_supported(obs_dim, hidden, n_actions) || rows <= 0) return 0;
+    return 4 * fused_det_partials(obs_dim, n_actions, rows);
+}
+
 template <int D, int A>
-static int policy_tower_launch(const TowerTrainArgs &a, cudaStream_t st, int loss) {
+static int policy_tower_launch(const TowerTrainArgs &a, cudaStream_t st, int loss, bool det) {
+    if (det) return loss == kLossA2C ? tower_train_launch_t<D, A, kLossA2C, true>(a, st, false) : tower_train_launch_t<D, A, kLossPPO, true>(a, st, false);
     return loss == kLossA2C ? tower_train_launch_t<D, A, kLossA2C>(a, st, false) : tower_train_launch_t<D, A>(a, st, false);
+}
+template <int D>
+static int value_tower_launch(const TowerTrainArgs &a, cudaStream_t st, bool pdl, bool det) {
+    return det ? tower_train_launch_t<D, 1, kLossPPO, true>(a, st, pdl) : tower_train_launch_t<D, 1>(a, st, pdl);
+}
+
+static int tower_launch(const TowerTrainArgs &a, int t, int obs_dim, int n_actions, int loss, cudaStream_t st, bool pdl, bool det) {
+    if (obs_dim == 6) return t == 0 ? policy_tower_launch<6, 5>(a, st, loss, det) : value_tower_launch<6>(a, st, pdl, det);
+    if (obs_dim == 7) return t == 0 ? policy_tower_launch<7, 3>(a, st, loss, det) : value_tower_launch<7>(a, st, pdl, det);
+    if (n_actions == 5) return t == 0 ? policy_tower_launch<4, 5>(a, st, loss, det) : value_tower_launch<4>(a, st, pdl, det);
+    return t == 0 ? policy_tower_launch<4, 4>(a, st, loss, det) : value_tower_launch<4>(a, st, pdl, det);
+}
+
+static void tower_args(TowerTrainArgs &a, int t, const MlpOffsets &o, const float *params, const void *wpack, const float *obs, const int32_t *index,
+                       int64_t rows, int64_t global_rows, const int32_t *actions, const float *advantages, const float *old_logp,
+                       const float *returns, const double *adv_sums, int normalize_advantage, float clip_range, float ent_coef, float vf_coef) {
+    a.W1 = params + o.w1[t]; a.B1 = params + o.b1[t];
+    a.W2 = reinterpret_cast<const __nv_bfloat16 *>(wpack) + (int64_t)(4 + t) * H * H;
+    a.B2 = params + o.b2[t]; a.Wh = params + o.wh[t]; a.Bh = params + o.bh[t];
+    a.x = obs; a.index = index; a.M = rows;
+    a.actions = actions; a.adv = advantages; a.old_logp = old_logp; a.returns = returns;
+    a.adv_sums = adv_sums; a.normalize = normalize_advantage;
+    a.clip = clip_range; a.ent_coef = ent_coef; a.vf_coef = vf_coef; a.inv_rows = (float)(1.0 / (double)global_rows);
+}
+
+// TMLA_MB_DETERMINISTIC: the same kernels and schedule with every atomic replaced by a per-CTA partial (the tower kernels' rows,
+// the weight-gradient planes), then one det_reduce launch that adds them into `grads` and `stats_out` in CTA order.  The
+// experiment switches (TMLA_WGRAD, TMLA_WGRAD_H1) do not apply.
+static int tower_batch_det(int loss, const MlpOffsets &o, const float *params, const void *wpack, int obs_dim, int n_actions, const float *obs,
+                           const int32_t *index, int64_t rows, int64_t global_rows, const int32_t *actions, const float *advantages,
+                           const float *old_logp, const float *returns, const double *adv_sums, int normalize_advantage, float clip_range,
+                           float ent_coef, float vf_coef, float *grads, __nv_bfloat16 *const (*img)[2], float *stats_out, float *logits_out,
+                           float *values_out, cudaStream_t st) {
+    const int64_t rows_padded = (rows + 127) / 128 * 128;
+    float *planes = reinterpret_cast<float *>(img[1][1] + rows_padded * H);    // partials follow the four tile images
+    unsigned wgrid;
+    int n1;
+    wgrad_tiled_split(rows_padded, true, &wgrid, &n1);
+    const int n0 = (int)wgrid - n1;
+    const int64_t nchunks = rows_padded / 64;
+    float *planes1 = planes + (int64_t)n0 * H * H;
+    float *trow[2] = {planes + (int64_t)wgrid * H * H, nullptr};
+    const int ctas = (int)std::min<int64_t>(rows_padded / 128, sm_count_train());
+    const int64_t rlen[2] = {det_tower_row(obs_dim, n_actions), det_tower_row(obs_dim, 1)};
+    trow[1] = trow[0] + ctas * rlen[0];
+    static const bool pdl_on = [] { const char *e = getenv("TMLA_PDL"); return !(e && !strcmp(e, "0")); }();
+    for (int t = 0; t < 2; ++t) {
+        TowerTrainArgs a;
+        tower_args(a, t, o, params, wpack, obs, index, rows, global_rows, actions, advantages, old_logp, returns, adv_sums, normalize_advantage,
+                   clip_range, ent_coef, vf_coef);
+        a.h1_out = img[t][0]; a.dz2_out = img[t][1]; a.out = t == 0 ? logits_out : values_out;
+        float *r = trow[t];                               // row layout: W1 | b1 | b2 | Wh | bh | statistics (det_tower_row)
+        a.gW1 = r; a.gB1 = r + H * obs_dim; a.gB2 = a.gB1 + H; a.gWh = a.gB2 + H; a.gBh = a.gWh + o.nout[t] * H; a.stats = a.gBh + o.nout[t];
+        const int rc = tower_launch(a, t, obs_dim, n_actions, loss, st, pdl_on, true);
+        if (rc) return rc;
+    }
+    int rc = tc_wgrad_tiled_launch<true>(img[0][1], img[0][0], planes, rows_padded, st, img[1][1], img[1][0], planes1, false);
+    if (rc) return rc;
+    DetSeg sg[kDetMaxSegs];
+    int n = 0;
+    sg[n++] = DetSeg{planes, H * H, (int)std::min<int64_t>(n0, nchunks), H * H, grads + o.w2[0], nullptr, 0, 0, 0};
+    sg[n++] = DetSeg{planes1, H * H, (int)std::min<int64_t>(n1, nchunks), H * H, grads + o.w2[1], nullptr, 0, 0, 0};
+    for (int t = 0; t < 2; ++t) {
+        const int D = obs_dim, nout = o.nout[t];
+        sg[n++] = DetSeg{trow[t], rlen[t], ctas, H * D + H, grads + o.w1[t], nullptr, 0, 0, 0};                 // W1 | b1
+        sg[n++] = DetSeg{trow[t] + H * D + H, rlen[t], ctas, H, grads + o.b2[t], nullptr, 0, 0, 0};             // b2
+        sg[n++] = DetSeg{trow[t] + H * D + 2 * H, rlen[t], ctas, nout * H + nout, grads + o.wh[t], nullptr, 0, 0, 0};   // Wh | bh
+    }
+    const int64_t st_off[2] = {rlen[0] - 8, rlen[1] - 8};
+    sg[n++] = DetSeg{trow[0] + st_off[0], rlen[0], ctas, 6, stats_out, trow[1] + st_off[1], rlen[1], ctas, 0};
+    if (normalize_advantage) sg[n++] = DetSeg{trow[0] + st_off[0] + 6, rlen[0], 1, 2, stats_out + 6, nullptr, 0, 0, 1};   // CTA 0: mean, std
+    return det_reduce_launch(sg, n, st);
 }
 
 // one fused batch of either loss: the policy tower with PPO's or A2C's loss, the shared value tower, the weight-gradient GEMMs
@@ -1353,6 +1494,9 @@ static int tower_batch_launch(int loss, const char *fn, const float *params, con
     // scratch: H1 and dZ2 tile images of both towers (one weight-gradient launch covers the two towers)
     __nv_bfloat16 *img[2][2];
     for (int t = 0; t < 2; ++t) for (int q = 0; q < 2; ++q) img[t][q] = reinterpret_cast<__nv_bfloat16 *>(scratch) + (int64_t)(2 * t + q) * rows_padded * H;
+    if (flags & TMLA_MB_DETERMINISTIC) return tower_batch_det(loss, o, params, wpack, obs_dim, n_actions, obs, index, rows, global_rows, actions,
+                                                              advantages, old_logp, returns, adv_sums, normalize_advantage, clip_range, ent_coef,
+                                                              vf_coef, grads, img, stats_out, logits_out, values_out, st);
     static const bool interleave = [] { const char *e = getenv("TMLA_WGRAD"); return e && !strcmp(e, "interleave"); }();   // A/B: wgrad right after each tower
     // TMLA_WGRAD_H1=recompute: the weight-gradient kernel recomputes H1 from the observations, so that no H1 image is written
     // or read (tc_wgrad_h1_kernel).  Measured on B200, one 262 144-row ball3d minibatch (2 towers + wgrad): 413.5 us with 8
@@ -1367,21 +1511,13 @@ static int tower_batch_launch(int loss, const char *fn, const float *params, con
     for (int t = 0; t < 2; ++t) {
         __nv_bfloat16 *h1 = img[t][0], *dz2 = img[t][1];
         TowerTrainArgs a;
-        a.W1 = params + o.w1[t]; a.B1 = params + o.b1[t];
-        a.W2 = reinterpret_cast<const __nv_bfloat16 *>(wpack) + (int64_t)(4 + t) * H * H;
-        a.B2 = params + o.b2[t]; a.Wh = params + o.wh[t]; a.Bh = params + o.bh[t];
-        a.x = obs; a.index = index; a.M = rows;
-        a.actions = actions; a.adv = advantages; a.old_logp = old_logp; a.returns = returns;
-        a.adv_sums = adv_sums; a.normalize = normalize_advantage;
-        a.clip = clip_range; a.ent_coef = ent_coef; a.vf_coef = vf_coef; a.inv_rows = (float)(1.0 / (double)global_rows);
+        tower_args(a, t, o, params, wpack, obs, index, rows, global_rows, actions, advantages, old_logp, returns, adv_sums, normalize_advantage,
+                   clip_range, ent_coef, vf_coef);
         a.h1_out = recompute ? nullptr : h1; a.dz2_out = dz2; a.out = t == 0 ? logits_out : values_out;
         a.gW1 = grads + o.w1[t]; a.gB1 = grads + o.b1[t]; a.gB2 = grads + o.b2[t]; a.gWh = grads + o.wh[t]; a.gBh = grads + o.bh[t];
         a.stats = stats_out;
         int rc;
-        if (obs_dim == 6) rc = t == 0 ? policy_tower_launch<6, 5>(a, st, loss) : tower_train_launch_t<6, 1>(a, st, pdl);
-        else if (obs_dim == 7) rc = t == 0 ? policy_tower_launch<7, 3>(a, st, loss) : tower_train_launch_t<7, 1>(a, st, pdl);
-        else if (n_actions == 5) rc = t == 0 ? policy_tower_launch<4, 5>(a, st, loss) : tower_train_launch_t<4, 1>(a, st, pdl);
-        else rc = t == 0 ? policy_tower_launch<4, 4>(a, st, loss) : tower_train_launch_t<4, 1>(a, st, pdl);
+        rc = tower_launch(a, t, obs_dim, n_actions, loss, st, pdl, false);
         if (rc) return rc;
         if (interleave) { rc = tc_wgrad_tiled_launch(img[t][1], img[t][0], grads + o.w2[t], rows_padded, st); if (rc) return rc; }
     }

@@ -146,6 +146,8 @@ adv_stats_kernel(const float *__restrict__ adv, const int32_t *__restrict__ inde
 }
 
 // all minibatches of an epoch in one launch: blockIdx.y = minibatch, rows [mb*mb_rows, min(total, (mb+1)*mb_rows))
+// DET: `sums` is double[n_mb][gridDim.x][2]: each block stores its (sum, sum of squares); adv_stats_det_reduce_kernel adds them
+template <bool DET = false>
 __global__ void __launch_bounds__(256)
 adv_stats_batched_kernel(const float *__restrict__ adv, const int32_t *__restrict__ index, int64_t total, int64_t mb_rows, double *sums) {
     __shared__ double sh[2][8];
@@ -163,10 +165,29 @@ adv_stats_batched_kernel(const float *__restrict__ adv, const int32_t *__restric
         s = l < 8 ? sh[0][l] : 0.0; ss = l < 8 ? sh[1][l] : 0.0;
         s = warp_sum(s); ss = warp_sum(ss);
         if (l == 0) {
+            if constexpr (DET) {
+                double *o = sums + 2 * ((int64_t)blockIdx.y * gridDim.x + blockIdx.x);
+                o[0] = s; o[1] = ss;
+                return;
+            }
             double *o = sums + 3 * blockIdx.y;
             atomicAdd(o + 0, s); atomicAdd(o + 1, ss);
             if (blockIdx.x == 0) atomicAdd(o + 2, (double)(hi - lo));
         }
+    }
+}
+// one warp per minibatch: lane l adds the partials of blocks l, l+32, ... in order, then a fixed butterfly
+__global__ void __launch_bounds__(32)
+adv_stats_det_reduce_kernel(const double *__restrict__ part, int gx, int64_t total, int64_t mb_rows, double *__restrict__ sums) {
+    const int l = threadIdx.x;
+    const double *p = part + 2 * (int64_t)blockIdx.x * gx;
+    double s = 0.0, ss = 0.0;
+    for (int b = l; b < gx; b += 32) { s += p[2 * b]; ss += p[2 * b + 1]; }
+    s = warp_sum(s); ss = warp_sum(ss);
+    if (l == 0) {
+        const int64_t lo = (int64_t)blockIdx.x * mb_rows, hi = min(total, lo + mb_rows);
+        double *o = sums + 3 * blockIdx.x;
+        o[0] = s; o[1] = ss; o[2] = (double)(hi - lo);
     }
 }
 
@@ -176,8 +197,10 @@ adv_stats_batched_kernel(const float *__restrict__ adv, const int32_t *__restric
 //   loss = -mean(min(A r, A clip(r))) + ent_coef * -mean(H) + vf_coef * mean((R - V)^2)
 // written straight into dlogits / dvalues (scaled by 1/global_rows).  A2C (SB3 2.9.0 a2c.py) replaces the surrogate by
 //   -mean(A log pi(a|s))  (no ratio, no clip, no old_logp; approx_kl / clip_fraction stay 0)
+// DET: `stats` is float[gridDim.x][8]: block b stores its six sums in row b (block 0 also mean / std in slots 6, 7), summed in
+// block order by det_reduce_kernel
 enum { kLossPPO = 0, kLossA2C = 1 };
-template <int A, int LOSS = kLossPPO>
+template <int A, int LOSS = kLossPPO, bool DET = false>
 __global__ void __launch_bounds__(256)
 ppo_loss_kernel(const float *__restrict__ logits, const float *__restrict__ values, const int32_t *__restrict__ actions,
                 const float *__restrict__ advantages, const float *__restrict__ old_logp, const float *__restrict__ returns,
@@ -262,6 +285,13 @@ ppo_loss_kernel(const float *__restrict__ logits, const float *__restrict__ valu
             acc[q] = x * invB;
         }
         if (l == 0) {
+            if constexpr (DET) {
+                float *row = stats + 8 * (int64_t)blockIdx.x;
+#pragma unroll
+                for (int q = 0; q < 5; ++q) row[q] = acc[q];
+                row[5] = acc[0] + ent_coef * acc[2] + vf_coef * acc[1];
+                return;
+            }
 #pragma unroll
             for (int q = 0; q < 5; ++q) atomicAdd(stats + q, acc[q]);
             atomicAdd(stats + 5, acc[0] + ent_coef * acc[2] + vf_coef * acc[1]);
@@ -333,6 +363,8 @@ __global__ void bootstrap_add_kernel(float *rew, const int32_t *count, const int
     if (i < c) rew[idx[i]] = __fadd_rn(rew[idx[i]], __fmul_rn(g, vals[i]));
 }
 
+static unsigned adv_stats_batched_gx(int64_t mb_rows) { return (unsigned)std::min<int64_t>(ceil_div64(mb_rows, 256 * 8), 148 * 2); }
+
 extern "C" {
 
 int tmla_gae(const float *rewards, const float *values, const uint8_t *dones, const float *last_values, double gamma,
@@ -378,19 +410,41 @@ int tmla_adv_stats_batched(const float *advantages, const int32_t *index, int64_
     const int64_t n_mb = ceil_div64(total, mb_rows);
     TMLA_REQUIRE(n_mb <= 65535, "too many minibatches");
     TMLA_CUDA(cudaMemsetAsync(adv_sums, 0, 3 * sizeof(double) * n_mb, (cudaStream_t)stream));
-    const unsigned gx = (unsigned)std::min<int64_t>(ceil_div64(mb_rows, 256 * 8), 148 * 2);
-    adv_stats_batched_kernel<<<dim3(gx, (unsigned)n_mb), 256, 0, (cudaStream_t)stream>>>(advantages, index, total, mb_rows, adv_sums);
+    const unsigned gx = adv_stats_batched_gx(mb_rows);
+    adv_stats_batched_kernel<false><<<dim3(gx, (unsigned)n_mb), 256, 0, (cudaStream_t)stream>>>(advantages, index, total, mb_rows, adv_sums);
+    TMLA_LAUNCH_CHECK();
+    return TMLA_OK;
+}
+
+int64_t tmla_adv_stats_det_scratch_bytes(int64_t total, int64_t mb_rows) {
+    if (total <= 0 || mb_rows <= 0) { tmla_set_error("total and mb_rows must be positive"); return TMLA_EINVAL; }
+    return 16 * ceil_div64(total, mb_rows) * (int64_t)adv_stats_batched_gx(mb_rows);
+}
+
+int tmla_adv_stats_batched_det(const float *advantages, const int32_t *index, int64_t total, int64_t mb_rows, double *adv_sums,
+                               void *partials, void *stream) {
+    TMLA_REQUIRE(advantages && adv_sums && partials && total > 0 && mb_rows > 0, "bad arguments");
+    const int64_t n_mb = ceil_div64(total, mb_rows);
+    TMLA_REQUIRE(n_mb <= 65535, "too many minibatches");
+    const unsigned gx = adv_stats_batched_gx(mb_rows);
+    cudaStream_t st = (cudaStream_t)stream;
+    adv_stats_batched_kernel<true><<<dim3(gx, (unsigned)n_mb), 256, 0, st>>>(advantages, index, total, mb_rows, (double *)partials);
+    TMLA_LAUNCH_CHECK();
+    adv_stats_det_reduce_kernel<<<(unsigned)n_mb, 32, 0, st>>>((const double *)partials, (int)gx, total, mb_rows, adv_sums);
     TMLA_LAUNCH_CHECK();
     return TMLA_OK;
 }
 
 }  // extern "C"
 
+int64_t loss_det_scratch_bytes(int64_t rows) { return 4 * 8 * ceil_div64(rows, 256); }
+
+// det_part != NULL: the deterministic form (per-block statistics rows in det_part, then det_reduce)
 template <int LOSS>
 static int loss_launch(const char *fn, const float *logits, const float *values, const int32_t *actions, const float *advantages,
                        const float *old_logp, const float *returns, const int32_t *index, int64_t rows, int64_t global_rows,
                        int n_actions, const double *adv_sums, int normalize_advantage, float clip_range, float ent_coef,
-                       float vf_coef, float *dlogits, float *dvalues, float *stats_out, void *stream) {
+                       float vf_coef, float *dlogits, float *dvalues, float *stats_out, void *stream, float *det_part = nullptr) {
     TMLA_REQUIRE(logits && values && actions && advantages && (old_logp || LOSS == kLossA2C) && returns && dlogits && dvalues && stats_out,
                  "NULL buffer");
     TMLA_REQUIRE(rows > 0 && global_rows >= rows, "bad row counts");
@@ -399,16 +453,25 @@ static int loss_launch(const char *fn, const float *logits, const float *values,
     TMLA_CUDA(cudaMemsetAsync(stats_out, 0, 8 * sizeof(float), st));
     const unsigned grid = (unsigned)ceil_div64(rows, 256);
     const double inv = 1.0 / (double)global_rows;
-#define LOSS_LAUNCH(AA)                                                                                                    \
-    ppo_loss_kernel<AA, LOSS><<<grid, 256, 0, st>>>(logits, values, actions, advantages, old_logp, returns, index, rows, inv, \
-                                                    adv_sums, normalize_advantage, clip_range, ent_coef, vf_coef, dlogits, dvalues, stats_out)
-    if (n_actions == 3) LOSS_LAUNCH(3);
-    else if (n_actions == 4) LOSS_LAUNCH(4);
-    else if (n_actions == 5) LOSS_LAUNCH(5);
-    else { tmla_set_error("%s: n_actions must be 3, 4 or 5 (got %d)", fn, n_actions); return TMLA_EINVAL; }
+#define LOSS_LAUNCH(AA, DET, OUT)                                                                                              \
+    ppo_loss_kernel<AA, LOSS, DET><<<grid, 256, 0, st>>>(logits, values, actions, advantages, old_logp, returns, index, rows, inv, \
+                                                         adv_sums, normalize_advantage, clip_range, ent_coef, vf_coef, dlogits, dvalues, OUT)
+    if (n_actions < 3 || n_actions > 5) { tmla_set_error("%s: n_actions must be 3, 4 or 5 (got %d)", fn, n_actions); return TMLA_EINVAL; }
+    if (det_part) {
+        if (n_actions == 3) LOSS_LAUNCH(3, true, det_part);
+        else if (n_actions == 4) LOSS_LAUNCH(4, true, det_part);
+        else LOSS_LAUNCH(5, true, det_part);
+    } else {
+        if (n_actions == 3) LOSS_LAUNCH(3, false, stats_out);
+        else if (n_actions == 4) LOSS_LAUNCH(4, false, stats_out);
+        else LOSS_LAUNCH(5, false, stats_out);
+    }
 #undef LOSS_LAUNCH
     TMLA_LAUNCH_CHECK();
-    return TMLA_OK;
+    if (!det_part) return TMLA_OK;
+    DetSeg sg[2] = {DetSeg{det_part, 8, (int)grid, 6, stats_out, nullptr, 0, 0, 0},
+                    DetSeg{det_part + 6, 8, 1, 2, stats_out + 6, nullptr, 0, 0, 1}};     // block 0's mean / std
+    return det_reduce_launch(sg, normalize_advantage ? 2 : 1, st);
 }
 
 extern "C" {
@@ -427,6 +490,26 @@ int tmla_a2c_loss(const float *logits, const float *values, const int32_t *actio
                   void *stream) {
     return loss_launch<kLossA2C>("tmla_a2c_loss", logits, values, actions, advantages, nullptr, returns, index, rows, global_rows, n_actions,
                                  adv_sums, normalize_advantage, 0.0f, ent_coef, vf_coef, dlogits, dvalues, stats_out, stream);
+}
+
+int tmla_ppo_loss_det(const float *logits, const float *values, const int32_t *actions, const float *advantages,
+                      const float *old_logp, const float *returns, const int32_t *index, int64_t rows, int64_t global_rows,
+                      int n_actions, const double *adv_sums, int normalize_advantage, float clip_range, float ent_coef,
+                      float vf_coef, float *dlogits, float *dvalues, float *stats_out, void *partials, void *stream) {
+    TMLA_REQUIRE(partials, "NULL partials");
+    return loss_launch<kLossPPO>("tmla_ppo_loss_det", logits, values, actions, advantages, old_logp, returns, index, rows, global_rows,
+                                 n_actions, adv_sums, normalize_advantage, clip_range, ent_coef, vf_coef, dlogits, dvalues, stats_out, stream,
+                                 (float *)partials);
+}
+
+int tmla_a2c_loss_det(const float *logits, const float *values, const int32_t *actions, const float *advantages, const float *returns,
+                      const int32_t *index, int64_t rows, int64_t global_rows, int n_actions, const double *adv_sums,
+                      int normalize_advantage, float ent_coef, float vf_coef, float *dlogits, float *dvalues, float *stats_out,
+                      void *partials, void *stream) {
+    TMLA_REQUIRE(partials, "NULL partials");
+    return loss_launch<kLossA2C>("tmla_a2c_loss_det", logits, values, actions, advantages, nullptr, returns, index, rows, global_rows,
+                                 n_actions, adv_sums, normalize_advantage, 0.0f, ent_coef, vf_coef, dlogits, dvalues, stats_out, stream,
+                                 (float *)partials);
 }
 
 }  // extern "C"

@@ -117,6 +117,12 @@ SIGNATURES = {
     "tmla_tc_wgrad_tiled": (_i, [vp, vp, vp, i64, vp]),
     "tmla_tc_probe": (_i, [vp, vp, vp, _i, vp]),
     "tmla_tc_overlap_probe": (_i, [vp, _i, _i, _i, vp]),
+    "tmla_det_scratch_bytes": (i64, [_i, _i, _i, i64]),
+    "tmla_adv_stats_det_scratch_bytes": (i64, [i64, i64]),
+    "tmla_mlp_backward_bf16_det": (_i, [vp, vp, _i, _i, _i, vp, vp, i64, vp, vp, vp, vp, vp, vp, vp]),
+    "tmla_adv_stats_batched_det": (_i, [vp, vp, i64, i64, vp, vp, vp]),
+    "tmla_ppo_loss_det": (_i, [vp, vp, vp, vp, vp, vp, vp, i64, i64, _i, vp, _i, f32, f32, f32, vp, vp, vp, vp, vp]),
+    "tmla_a2c_loss_det": (_i, [vp, vp, vp, vp, vp, vp, i64, i64, _i, vp, _i, f32, f32, vp, vp, vp, vp, vp]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -98,10 +98,31 @@ def mlp_forward(params, x, obs_dim, n_actions, *, index=None, rows=None, rows_de
     return logits, values, act_cache
 
 
+def det_scratch_bytes(obs_dim: int, n_actions: int, rows: int, hidden: int = HIDDEN) -> int:
+    """Bytes of the deterministic-mode partials (tmla_det_scratch_bytes) for calls of up to `rows` rows: the `partials` of
+    mlp_backward / ppo_loss / a2c_loss, and what ppo_minibatch / a2c_batch(deterministic=True) add to their scratch."""
+    n = lib.tmla_det_scratch_bytes(obs_dim, hidden, n_actions, int(rows))
+    if n < 0:
+        raise ValueError(native.last_error())
+    return int(n)
+
+
+def fused_scratch_elems(obs_dim: int, n_actions: int, rows: int, deterministic: bool = False) -> int:
+    """bf16 elements of the scratch of ppo_minibatch / a2c_batch: the tile images, plus the partials when deterministic."""
+    n = lib.tmla_ppo_minibatch_scratch(HIDDEN, int(rows))
+    return n + ((det_scratch_bytes(obs_dim, n_actions, rows) + 1) // 2 if deterministic else 0)
+
+
+def _partials(partials, name="partials"):
+    if partials is not None and (not partials.is_cuda or not partials.is_contiguous()):
+        raise ValueError(f"{name} must be a contiguous CUDA tensor")
+
+
 def mlp_backward(params, x, obs_dim, n_actions, act_cache, dlogits, dvalues, *, index=None, rows=None, grads=None,
-                 scratch=None, wpack=None, hidden=HIDDEN):
+                 scratch=None, wpack=None, hidden=HIDDEN, partials=None):
     """Gradient of ActorCriticPolicy.forward (flat, overwritten).  hidden 64 / 128: scratch holds per-chunk partial gradients,
-    summed in a fixed order (bit-identical across calls)."""
+    summed in a fixed order (bit-identical across calls).  partials (bf16 path, det_scratch_bytes bytes): the deterministic
+    form, tmla_mlp_backward_bf16_det."""
     if wpack is not None and hidden != HIDDEN:
         raise ValueError(f"the bf16 tensor-core path covers hidden = {HIDDEN} only (got {hidden})")
     if rows is None:
@@ -117,9 +138,13 @@ def mlp_backward(params, x, obs_dim, n_actions, act_cache, dlogits, dvalues, *, 
         scratch = torch.empty(size, dtype=act_dtype, device=dev)
     _chk(dlogits, torch.float32, "dlogits"); _chk(dvalues, torch.float32, "dvalues")
     _chk(act_cache, act_dtype, "act_cache"); _chk(scratch, act_dtype, "scratch")
+    _partials(partials)
     if wpack is None:
         check(lib.tmla_mlp_backward(ptr(params), obs_dim, hidden, n_actions, ptr(x), ptr(index), int(rows), ptr(act_cache),
                                     ptr(dlogits), ptr(dvalues), ptr(grads), ptr(scratch), _s()))
+    elif partials is not None:
+        check(lib.tmla_mlp_backward_bf16_det(ptr(params), ptr(wpack), obs_dim, HIDDEN, n_actions, ptr(x), ptr(index), int(rows),
+                                             ptr(act_cache), ptr(dlogits), ptr(dvalues), ptr(grads), ptr(scratch), ptr(partials), _s()))
     else:
         check(lib.tmla_mlp_backward_bf16(ptr(params), ptr(wpack), obs_dim, HIDDEN, n_actions, ptr(x), ptr(index), int(rows),
                                          ptr(act_cache), ptr(dlogits), ptr(dvalues), ptr(grads), ptr(scratch), _s()))
@@ -133,19 +158,32 @@ def adv_stats(advantages, index, rows, sums=None):
     return sums
 
 
-def adv_stats_batched(advantages, index, total, mb_rows, sums=None):
-    """(sum, sum of squares, count) of the advantages of every minibatch of an epoch: double[n_mb, 3]."""
+def adv_stats_batched(advantages, index, total, mb_rows, sums=None, partials=None):
+    """(sum, sum of squares, count) of the advantages of every minibatch of an epoch: double[n_mb, 3].  partials
+    (adv_det_scratch_bytes bytes): the deterministic form, per-block sums added in block order."""
     n_mb = (total + mb_rows - 1) // mb_rows
     if sums is None:
         sums = torch.empty((n_mb, 3), dtype=torch.float64, device=advantages.device)
     _chk(sums, torch.float64, "sums")
-    check(lib.tmla_adv_stats_batched(ptr(advantages), ptr(index), int(total), int(mb_rows), ptr(sums), _s()))
+    _partials(partials)
+    if partials is not None:
+        check(lib.tmla_adv_stats_batched_det(ptr(advantages), ptr(index), int(total), int(mb_rows), ptr(sums), ptr(partials), _s()))
+    else:
+        check(lib.tmla_adv_stats_batched(ptr(advantages), ptr(index), int(total), int(mb_rows), ptr(sums), _s()))
     return sums
+
+
+def adv_det_scratch_bytes(total: int, mb_rows: int) -> int:
+    n = lib.tmla_adv_stats_det_scratch_bytes(int(total), int(mb_rows))
+    if n < 0:
+        raise ValueError(native.last_error())
+    return int(n)
 
 
 def ppo_loss(logits, values, actions, advantages, old_logp, returns, *, index=None, rows=None, global_rows=None,
              adv_sums=None, normalize=True, clip_range=0.2, ent_coef=0.01, vf_coef=0.5, dlogits=None, dvalues=None,
-             stats=None):
+             stats=None, partials=None):
+    """PPO's loss head (tmla_ppo_loss); partials (det_scratch_bytes bytes): statistics summed in block order (tmla_ppo_loss_det)."""
     if rows is None:
         rows = logits.shape[0]
     n_actions = logits.shape[1]
@@ -159,16 +197,21 @@ def ppo_loss(logits, values, actions, advantages, old_logp, returns, *, index=No
         stats = torch.empty(8, dtype=torch.float32, device=dev)
     if normalize and adv_sums is None:
         adv_sums = adv_stats(advantages, index, rows)
-    check(lib.tmla_ppo_loss(ptr(logits), ptr(values), ptr(actions), ptr(advantages), ptr(old_logp), ptr(returns),
-                            ptr(index), int(rows), int(global_rows or rows), int(n_actions), ptr(adv_sums),
-                            1 if normalize else 0, float(clip_range), float(ent_coef), float(vf_coef), ptr(dlogits),
-                            ptr(dvalues), ptr(stats), _s()))
+    _partials(partials)
+    args = (ptr(logits), ptr(values), ptr(actions), ptr(advantages), ptr(old_logp), ptr(returns), ptr(index), int(rows),
+            int(global_rows or rows), int(n_actions), ptr(adv_sums), 1 if normalize else 0, float(clip_range), float(ent_coef),
+            float(vf_coef), ptr(dlogits), ptr(dvalues), ptr(stats))
+    if partials is not None:
+        check(lib.tmla_ppo_loss_det(*args, ptr(partials), _s()))
+    else:
+        check(lib.tmla_ppo_loss(*args, _s()))
     return dlogits, dvalues, stats
 
 
 def a2c_loss(logits, values, actions, advantages, returns, *, index=None, rows=None, global_rows=None, adv_sums=None,
-             normalize=False, ent_coef=0.0, vf_coef=0.5, dlogits=None, dvalues=None, stats=None):
-    """A2C.train's loss head (tmla_a2c_loss): ppo_loss without old_logp and clip_range; normalisation off by default (SB3's A2C)."""
+             normalize=False, ent_coef=0.0, vf_coef=0.5, dlogits=None, dvalues=None, stats=None, partials=None):
+    """A2C.train's loss head (tmla_a2c_loss): ppo_loss without old_logp and clip_range; normalisation off by default (SB3's A2C).
+    partials: as ppo_loss (tmla_a2c_loss_det)."""
     if rows is None:
         rows = logits.shape[0]
     n_actions = logits.shape[1]
@@ -182,10 +225,22 @@ def a2c_loss(logits, values, actions, advantages, returns, *, index=None, rows=N
         stats = torch.empty(8, dtype=torch.float32, device=dev)
     if normalize and adv_sums is None:
         adv_sums = adv_stats(advantages, index, rows)
-    check(lib.tmla_a2c_loss(ptr(logits), ptr(values), ptr(actions), ptr(advantages), ptr(returns), ptr(index), int(rows),
-                            int(global_rows or rows), int(n_actions), ptr(adv_sums), 1 if normalize else 0, float(ent_coef),
-                            float(vf_coef), ptr(dlogits), ptr(dvalues), ptr(stats), _s()))
+    _partials(partials)
+    args = (ptr(logits), ptr(values), ptr(actions), ptr(advantages), ptr(returns), ptr(index), int(rows), int(global_rows or rows),
+            int(n_actions), ptr(adv_sums), 1 if normalize else 0, float(ent_coef), float(vf_coef), ptr(dlogits), ptr(dvalues), ptr(stats))
+    if partials is not None:
+        check(lib.tmla_a2c_loss_det(*args, ptr(partials), _s()))
+    else:
+        check(lib.tmla_a2c_loss(*args, _s()))
     return dlogits, dvalues, stats
+
+
+TMLA_MB_GRADS_ZEROED, TMLA_MB_ACCUMULATE_STATS, TMLA_MB_DETERMINISTIC = 1, 2, 4      # include/tmla.h
+
+
+def _mb_flags(grads_zeroed: bool, accumulate_stats: bool, deterministic: bool) -> int:
+    return ((TMLA_MB_GRADS_ZEROED if grads_zeroed else 0) | (TMLA_MB_ACCUMULATE_STATS if accumulate_stats else 0)
+            | (TMLA_MB_DETERMINISTIC if deterministic else 0))
 
 
 def ppo_minibatch_supported(obs_dim: int, n_actions: int, hidden: int = HIDDEN) -> bool:
@@ -194,10 +249,11 @@ def ppo_minibatch_supported(obs_dim: int, n_actions: int, hidden: int = HIDDEN) 
 
 def ppo_minibatch(params, wpack, obs, obs_dim, n_actions, actions, advantages, old_logp, returns, *, index=None, rows=None,
                   global_rows=None, adv_sums=None, normalize=True, clip_range=0.2, ent_coef=0.01, vf_coef=0.5, grads=None,
-                  scratch=None, stats=None, logits=None, values=None, grads_zeroed=False, accumulate_stats=False):
+                  scratch=None, stats=None, logits=None, values=None, grads_zeroed=False, accumulate_stats=False, deterministic=False):
     """One PPO.train minibatch, forward + loss + backward fused (tmla_ppo_minibatch_bf16): returns (grads, stats).
     grads_zeroed: `grads` is known to be all zeros (adam_clip(zero_grads=True) left it so) — skips the memset launch;
-    accumulate_stats: add to `stats` instead of overwriting it."""
+    accumulate_stats: add to `stats` instead of overwriting it; deterministic: TMLA_MB_DETERMINISTIC (bit-reproducible sums,
+    scratch of fused_scratch_elems(..., deterministic=True))."""
     _chk(params, torch.float32, "params"); _chk(wpack, torch.bfloat16, "wpack"); _chk(obs, torch.float32, "obs")
     _chk(index, torch.int32, "index"); _chk(actions, torch.int32, "actions"); _chk(advantages, torch.float32, "advantages")
     _chk(old_logp, torch.float32, "old_logp"); _chk(returns, torch.float32, "returns")
@@ -207,7 +263,7 @@ def ppo_minibatch(params, wpack, obs, obs_dim, n_actions, actions, advantages, o
     if grads is None:
         grads = torch.empty_like(params)
     if scratch is None:
-        scratch = torch.empty(lib.tmla_ppo_minibatch_scratch(HIDDEN, rows), dtype=torch.bfloat16, device=dev)
+        scratch = torch.empty(fused_scratch_elems(obs_dim, n_actions, rows, deterministic), dtype=torch.bfloat16, device=dev)
     if stats is None:
         stats = torch.empty(8, dtype=torch.float32, device=dev)
     _chk(scratch, torch.bfloat16, "scratch"); _chk(grads, torch.float32, "grads"); _chk(stats, torch.float32, "stats")
@@ -218,13 +274,13 @@ def ppo_minibatch(params, wpack, obs, obs_dim, n_actions, actions, advantages, o
                                       int(global_rows or rows), ptr(actions), ptr(advantages), ptr(old_logp), ptr(returns),
                                       ptr(adv_sums), 1 if normalize else 0, float(clip_range), float(ent_coef),
                                       float(vf_coef), ptr(grads), ptr(scratch), ptr(stats), ptr(logits), ptr(values),
-                                      (1 if grads_zeroed else 0) | (2 if accumulate_stats else 0), _s()))
+                                      _mb_flags(grads_zeroed, accumulate_stats, deterministic), _s()))
     return grads, stats
 
 
 def a2c_batch(params, wpack, obs, obs_dim, n_actions, actions, advantages, returns, *, index=None, rows=None, global_rows=None,
               adv_sums=None, normalize=False, ent_coef=0.0, vf_coef=0.5, grads=None, scratch=None, stats=None, logits=None,
-              values=None, grads_zeroed=False, accumulate_stats=False):
+              values=None, grads_zeroed=False, accumulate_stats=False, deterministic=False):
     """One A2C.train step's forward + loss + backward over the whole rollout, fused (tmla_a2c_batch_bf16): returns (grads, stats).
     Flags as ppo_minibatch."""
     _chk(params, torch.float32, "params"); _chk(wpack, torch.bfloat16, "wpack"); _chk(obs, torch.float32, "obs")
@@ -236,7 +292,7 @@ def a2c_batch(params, wpack, obs, obs_dim, n_actions, actions, advantages, retur
     if grads is None:
         grads = torch.empty_like(params)
     if scratch is None:
-        scratch = torch.empty(lib.tmla_ppo_minibatch_scratch(HIDDEN, rows), dtype=torch.bfloat16, device=dev)
+        scratch = torch.empty(fused_scratch_elems(obs_dim, n_actions, rows, deterministic), dtype=torch.bfloat16, device=dev)
     if stats is None:
         stats = torch.empty(8, dtype=torch.float32, device=dev)
     _chk(scratch, torch.bfloat16, "scratch"); _chk(grads, torch.float32, "grads"); _chk(stats, torch.float32, "stats")
@@ -246,7 +302,7 @@ def a2c_batch(params, wpack, obs, obs_dim, n_actions, actions, advantages, retur
     check(lib.tmla_a2c_batch_bf16(ptr(params), ptr(wpack), obs_dim, HIDDEN, n_actions, ptr(obs), ptr(index), int(rows),
                                   int(global_rows or rows), ptr(actions), ptr(advantages), ptr(returns), ptr(adv_sums),
                                   1 if normalize else 0, float(ent_coef), float(vf_coef), ptr(grads), ptr(scratch), ptr(stats),
-                                  ptr(logits), ptr(values), (1 if grads_zeroed else 0) | (2 if accumulate_stats else 0), _s()))
+                                  ptr(logits), ptr(values), _mb_flags(grads_zeroed, accumulate_stats, deterministic), _s()))
     return grads, stats
 
 

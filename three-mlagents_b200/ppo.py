@@ -134,6 +134,15 @@ class CudaPPO:
         self._adam_step = 0
         self._epoch_counter = 0
         self._dist, self.rank, self.world = _dist()
+        # torch.use_deterministic_algorithms(True): every sum of the update in a fixed order, so that a run is bit-for-bit
+        # repeatable for a fixed seed, task, n_envs, hyper-parameters, build and GPU model (DESIGN.md §8)
+        self.deterministic = torch.are_deterministic_algorithms_enabled()
+        if self.deterministic and self.mlp_impl == "fp32" and self.hidden == HIDDEN:
+            raise ValueError("torch.use_deterministic_algorithms(True): mlp_impl='fp32' at width 256 has no deterministic form (its "
+                             "weight-gradient GEMM splits K over CTAs with float atomics); use mlp_impl='bf16' or 'auto'")
+        if self.deterministic and self.world > 1:
+            raise ValueError("torch.use_deterministic_algorithms(True): data-parallel training (world_size > 1) has no deterministic "
+                             "form (the advantage statistics are all-reduced through NCCL, whose summation order is not fixed)")
         with torch.cuda.device(self.device):
             p = (orthogonal_init(self.obs_dim, self.n_actions, self.seed, self.hidden) if _params is None
                  else _params.detach().float().cpu())
@@ -204,11 +213,17 @@ class CudaPPO:
             self.dlogits = torch.empty((B, A), **f32)
             self.dvalues = torch.empty(B, **f32)
             self.cache_mb = torch.empty((4, B, H), dtype=self._act_dtype, device=dev)
+        det = self.deterministic
         if small:                                      # per-chunk partial gradients of the fixed-order reduction (mlp_small.cu)
             self.scratch_mb = torch.empty(native.lib.tmla_mlp_backward_scratch(D, H, A, B), dtype=torch.float32, device=dev)
+        elif self.fused_update:                        # H1 and dZ2 tile images of both towers (+ deterministic mode's partials)
+            self.scratch_mb = torch.empty(ops.fused_scratch_elems(D, A, B, det), dtype=self._act_dtype, device=dev)
         else:
-            n_img = 4 if self.fused_update else 2      # fused: H1 and dZ2 tile images of both towers
-            self.scratch_mb = torch.empty(n_img * ((B + 127) // 128 * 128) * HIDDEN, dtype=self._act_dtype, device=dev)
+            self.scratch_mb = torch.empty(2 * ((B + 127) // 128 * 128) * HIDDEN, dtype=self._act_dtype, device=dev)
+        # deterministic mode: per-CTA partials of the three-call path's loss statistics and backward, of the advantage statistics
+        self.det_partials = (torch.empty(ops.det_scratch_bytes(D, A, B, H), dtype=torch.uint8, device=dev)
+                             if det and not self.fused_update else None)
+        self.adv_partials = torch.empty(ops.adv_det_scratch_bytes(total, B), dtype=torch.uint8, device=dev) if det else None
         self.adv_sums = torch.zeros(((total + B - 1) // B, 3), dtype=torch.float64, device=dev)   # one row per minibatch of an epoch
         self.stats = torch.zeros(8, **f32)
         self.stats_acc = torch.zeros(8, **f32)
@@ -288,7 +303,7 @@ class CudaPPO:
             ops.permutation(self.seed + 7919 * self.rank, self._epoch_counter, T, N, out=self.perm)
             self._epoch_counter += 1
             if self.normalize_advantage:                  # advantage statistics of all minibatches: one launch, one all-reduce
-                ops.adv_stats_batched(self.adv, self.perm, total, B, self.adv_sums)
+                ops.adv_stats_batched(self.adv, self.perm, total, B, self.adv_sums, partials=self.adv_partials)
                 allreduce_sum_(self.adv_sums)
             for mb, start in enumerate(range(0, total, B)):
                 rows = min(B, total - start)
@@ -299,16 +314,17 @@ class CudaPPO:
                                       index=idx, rows=rows, global_rows=rows * self.world, adv_sums=sums,
                                       normalize=sums is not None, clip_range=self.clip_range, ent_coef=self.ent_coef,
                                       vf_coef=self.vf_coef, grads=self.grads, scratch=self.scratch_mb, stats=self.stats_acc,
-                                      grads_zeroed=True, accumulate_stats=True)
+                                      grads_zeroed=True, accumulate_stats=True, deterministic=self.deterministic)
                 else:
                     ops.mlp_forward(self.params, obs_flat, D, A, index=idx, rows=rows, logits=self.logits_mb,
                                     values=self.values_mb, act_cache=self.cache_mb, wpack=self.wpack, hidden=self.hidden)
                     ops.ppo_loss(self.logits_mb, self.values_mb, self.act, self.adv, self.logp, self.ret, index=idx,
                                  rows=rows, global_rows=rows * self.world, adv_sums=sums, normalize=sums is not None,
                                  clip_range=self.clip_range, ent_coef=self.ent_coef, vf_coef=self.vf_coef,
-                                 dlogits=self.dlogits, dvalues=self.dvalues, stats=self.stats)
+                                 dlogits=self.dlogits, dvalues=self.dvalues, stats=self.stats, partials=self.det_partials)
                     ops.mlp_backward(self.params, obs_flat, D, A, self.cache_mb, self.dlogits, self.dvalues, index=idx,
-                                     rows=rows, grads=self.grads, scratch=self.scratch_mb, wpack=self.wpack, hidden=self.hidden)
+                                     rows=rows, grads=self.grads, scratch=self.scratch_mb, wpack=self.wpack, hidden=self.hidden,
+                                     partials=self.det_partials if self.wpack is not None else None)
                 self._adam_step += 1
                 if self._comm is not None:                # the one collective on the path, inside the optimizer launches
                     nvtx.range_push("allreduce+adam")

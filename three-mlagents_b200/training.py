@@ -192,6 +192,7 @@ def train_task(config: TrainConfig, *, callback=None, model_kwargs: dict[str, An
         metadata = {
             "task": task.card(), "config": asdict(config), "algorithm": algorithm_name, "run_id": run_id,
             "model_filename": model_filename, "model_path": str(model_path),
+            "deterministic": bool(model.deterministic),
             "mean_reward": mean_reward, "std_reward": std_reward,
             "episode_rewards": [float(r) for r in episode_rewards],
             "episode_lengths": [int(n) for n in episode_lengths],
